@@ -2,6 +2,7 @@
 """bench.py - FASTQ->uQ encode throughput of the B200 path (BASELINE.json metric).
 
     python bench.py [--gpus N] [--steps K] [--warmup W]            # ours
+    python bench.py ... --dump-outputs DIR                          # also: outputs of the last timed step as DIR/*.npy
     python bench.py --impl reference [--steps K] [--warmup W]      # the reference algorithm on host cores
 
 Workload (BASELINE.json configs[1]): 100 M reads x 150 bp Illumina-style synthetic FASTQ,
@@ -118,10 +119,27 @@ def emit(line):
         os.write(_REAL_STDOUT, data)
 
 
+def dump_outputs(path, arrays, budget=60_000_000):
+    """arrays (name -> ndarray, the members encode hands its caller) -> path/<name>.npy, so that two builds can be compared
+    value for value.  Values are float32 for 1- and 2-byte integers and float64 otherwise (exact below 2**53).  An array
+    larger than its equal share of `budget` bytes is replaced by the elements at a fixed, seeded set of flat (C-order)
+    indices, the same for every array of that size."""
+    import numpy as np
+    os.makedirs(path, exist_ok=True)
+    per = budget // (8 * max(len(arrays), 1))
+    for name, a in sorted(arrays.items()):
+        if a.size > per:
+            idx = np.sort(np.random.default_rng(SEED).choice(a.size, per, replace=False))
+            a = a[np.unravel_index(idx, a.shape)]
+        np.save(os.path.join(path, name + ".npy"), a.astype(np.float32 if a.dtype.itemsize <= 2 else np.float64))
+
+
 def run_ours(args):
     quiet_stdout()
     from uq_b200 import shard
     rank, local_rank, world = shard.world()
+    if args.dump_outputs and world > 1:
+        sys.exit("--dump-outputs: single-process runs only")
     dist = None
     if world > 1:
         import torch
@@ -199,7 +217,9 @@ def run_ours(args):
             dist.destroy_process_group()
             sys.exit(3)
 
-    def one_step():
+    kept = []
+
+    def one_step(keep=False):
         fq = ctx.adopt_fastq(dev)
         if global_mode:
             # ONE container from all ranks: global statistics, sample-sort unique (NCCL all-to-all), global order
@@ -209,7 +229,10 @@ def run_ours(args):
         else:
             members, cfg = host.encode_device(ctx, fq, **opts)
             out_bytes = members.nbytes()
-            members.free()
+            if keep:
+                kept.append(members)
+            else:
+                members.free()
         fq.free()
         return out_bytes, cfg
 
@@ -225,8 +248,8 @@ def run_ours(args):
     launches0 = ctx.launches
     hc0 = list(comm.host_collectives) if global_mode else None
     ctx.span_begin()
-    for _ in range(args.steps):
-        out_bytes, cfg = one_step()
+    for i in range(args.steps):
+        out_bytes, cfg = one_step(keep=bool(args.dump_outputs) and i == args.steps - 1)
     ms = ctx.span_end()
     barrier()
     clocks = sampler.stop() if sampler else None
@@ -238,6 +261,10 @@ def run_ours(args):
                      "transport": "shared-memory board (one node)" if comm.board is not None else "gloo all_gather_object"}
     report = ctx.timing_report()
     ctx.timing(False)
+    if kept:
+        # before the decode and e2e legs, which need the HBM these members hold
+        dump_outputs(args.dump_outputs, kept[0].download())
+        kept[0].free()
     ms = max_over_ranks(ms)
     total_reads = sum_over_ranks(float(n))
     total_fbytes = sum_over_ranks(float(fbytes))
@@ -602,6 +629,8 @@ def main():
     ap.add_argument("--e2e-serial", action="store_true", help="e2e without copy/compute overlap (diagnostics)")
     ap.add_argument("--no-cpu", action="store_true")
     ap.add_argument("--no-parity", action="store_true", help="N>1: skip the sharded-vs-single parity check before the timed loop")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the output arrays of the last timed step as DIR/<name>.npy "
+                                                          "(float32 / float64, a seeded sample of each large array, < 64 MB)")
     args = ap.parse_args()
     if args.impl == "reference":
         run_reference(args)
