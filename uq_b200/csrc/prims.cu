@@ -187,23 +187,57 @@ __global__ void __launch_bounds__(256) k_bits_reduce(const uint64_t* __restrict_
     }
 }
 
-template <bool AUXDIGIT>
+// Bucket of the MSD sort below: items [start, start + size) of the array; its tiles are t0 .. t0 + nt - 1 of the pass and
+// the counters of its tile t are ghist[t0 * 256 + digit * nt + t] (digit-major inside the bucket, so that one exclusive scan
+// of all counters yields every bucket's digit runs in order).
+struct msd_bucket { uint32_t start, size, t0, nt; };
+
+// SEG = false: tile blockIdx.x of [0, n), counters ghist[digit * nblk + tile].  SEG = true: the tile belongs to bucket
+// tile_bucket[blockIdx.x] (see msd_bucket).
+template <bool SEG>
+struct radix_tile {
+    uint64_t tile0, end;        // items [tile0, min(end, tile0 + PR_TILE))
+    uint64_t hbase, hstride;    // counter of digit d: hbase + d * hstride
+    uint32_t bstart, hfirst;    // SEG: first item and first counter of the bucket
+    __device__ __forceinline__ radix_tile(uint64_t n, uint32_t nblk, const uint32_t* tile_bucket, const msd_bucket* buckets) {
+        if (SEG) {
+            const msd_bucket b = buckets[tile_bucket[blockIdx.x]];
+            const uint32_t t = blockIdx.x - b.t0;
+            tile0 = (uint64_t)b.start + (uint64_t)t * PR_TILE;
+            end = (uint64_t)b.start + b.size;
+            hbase = (uint64_t)b.t0 * 256 + t;
+            hstride = b.nt;
+            bstart = b.start;
+            hfirst = b.t0 * 256;
+        } else {
+            tile0 = (uint64_t)blockIdx.x * PR_TILE;
+            end = n;
+            hbase = blockIdx.x;
+            hstride = nblk;
+            bstart = hfirst = 0;
+        }
+    }
+};
+
+template <bool AUXDIGIT, bool SEG = false>
 __global__ void __launch_bounds__(PR_THREADS) k_radix_hist(const uint64_t* __restrict__ key, const uint32_t* __restrict__ aux, uint64_t n,
-                                                          int shift, uint32_t* __restrict__ ghist, uint32_t nblk) {
+                                                          int shift, uint32_t* __restrict__ ghist, uint32_t nblk,
+                                                          const uint32_t* __restrict__ tile_bucket = nullptr,
+                                                          const msd_bucket* __restrict__ buckets = nullptr) {
     __shared__ uint32_t hist[256];
     hist[threadIdx.x] = 0;
+    const radix_tile<SEG> T(n, nblk, tile_bucket, buckets);
     __syncthreads();
-    uint64_t tile0 = (uint64_t)blockIdx.x * PR_TILE;
 #pragma unroll 4
     for (int j = 0; j < PR_ITEMS; j++) {
-        uint64_t idx = tile0 + (uint64_t)j * PR_THREADS + threadIdx.x;
-        if (idx < n) {
+        uint64_t idx = T.tile0 + (uint64_t)j * PR_THREADS + threadIdx.x;
+        if (idx < T.end) {
             uint32_t d = AUXDIGIT ? ((aux[idx] >> shift) & 255u) : (uint32_t)((key[idx] >> shift) & 255ull);
             atomicAdd(&hist[d], 1u);
         }
     }
     __syncthreads();
-    ghist[(uint64_t)threadIdx.x * nblk + blockIdx.x] = hist[threadIdx.x];
+    ghist[T.hbase + (uint64_t)threadIdx.x * T.hstride] = hist[threadIdx.x];
 }
 
 // Stable scatter.  512 threads take one tile of PR_TILE items; every warp owns 256 consecutive items and
@@ -224,15 +258,20 @@ struct rs_stage {
     uint32_t aux[PR_TILE];
 };
 
-template <bool AUXDIGIT, bool HASAUX>
+// SEG: the tile and its counters come from the MSD bucket lists (radix_tile); a bucket's items are scattered inside its own
+// range, goff[first counter of the bucket] being the exclusive scan up to the bucket.
+template <bool AUXDIGIT, bool HASAUX, bool SEG = false>
 __global__ void __launch_bounds__(RS_THREADS, 2) k_radix_scatter(const uint64_t* __restrict__ kin, const uint32_t* __restrict__ ain,
                                                                 const uint32_t* __restrict__ vin, uint64_t* __restrict__ kout,
-                                                                uint32_t* __restrict__ aout, uint32_t* __restrict__ vout, uint64_t n,
-                                                                int shift, const uint32_t* __restrict__ goff, uint32_t nblk) {
+                                                                uint32_t* __restrict__ aout, uint32_t* __restrict__ vout, uint64_t n_,
+                                                                int shift, const uint32_t* __restrict__ goff, uint32_t nblk,
+                                                                const uint32_t* __restrict__ tile_bucket = nullptr,
+                                                                const msd_bucket* __restrict__ buckets = nullptr) {
     extern __shared__ __align__(16) uint8_t rs_raw[];
     rs_stage* S = reinterpret_cast<rs_stage*>(rs_raw);
     const unsigned tid = threadIdx.x, w = tid >> 5, lane = tid & 31u;
-    const uint64_t tile0 = (uint64_t)blockIdx.x * PR_TILE;
+    const radix_tile<SEG> T(n_, nblk, tile_bucket, buckets);
+    const uint64_t tile0 = T.tile0, n = T.end;
     const uint64_t warp0 = tile0 + (uint64_t)w * (32 * RS_ITEMS);
     const uint32_t ntile = (uint32_t)((n - tile0 < PR_TILE) ? (n - tile0) : PR_TILE);
     uint64_t key[RS_ITEMS];
@@ -293,7 +332,9 @@ __global__ void __launch_bounds__(RS_THREADS, 2) k_radix_scatter(const uint64_t*
         for (int i = 0; i < 8; i++) if ((unsigned)i < w) wb += S->wtot[i];
         const uint32_t start = wb + incl - tot;
         S->dstart[tid] = start;
-        S->gbase[tid] = goff[(uint64_t)tid * nblk + blockIdx.x] - start;      // global slot = gbase[d] + tile-local slot
+        uint32_t g = goff[T.hbase + (uint64_t)tid * T.hstride];
+        if (SEG) g += T.bstart - goff[T.hfirst];
+        S->gbase[tid] = g - start;      // global slot = gbase[d] + tile-local slot
     }
     __syncthreads();
     // stage the tile in digit order
@@ -668,6 +709,250 @@ __global__ void __launch_bounds__(256) k_key_iota(const uint64_t* __restrict__ k
     for (uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (uint64_t)gridDim.x * blockDim.x) { kout[i] = kin[i]; vout[i] = (uint32_t)i; }
 }
 
+// ---- MSD sort of large key-only inputs ----------------------------------------------------------------------------
+// Round 0 of a row sort is a stable sort of 100 M (key64, row index) records.  LSD needs one global pass per varying byte
+// (8 for packed DNA / QUAL rows); here each global pass splits every still-large bucket by its next 8 varying bits
+// (k_radix_hist / k_radix_scatter in their SEG form, each tile inside one bucket), and a bucket - or a run of
+// consecutive small buckets - of at most PR_TILE items is finished by one CTA in shared memory (k_bucket_sort: stable LSD
+// over the bits that vary inside it).  Uniform keys take 2 global passes and one read/write sweep; skewed keys
+// (quality strings) keep splitting only their large buckets.  Every step is stable, so the result is the stable sort.
+#define MSD_MIN_N (1u << 20)          // smaller sorts keep the LSD passes (not tuned: the bench sorts 100 M keys)
+
+struct msd_counts { uint32_t nseg, nbuck, ntiles, pad; };
+
+struct bs_stage {
+    uint32_t whist[RS_WARPS][256];
+    uint32_t dstart[256];
+    uint32_t wtot[8];
+    unsigned long long or64, and64;
+    uint64_t key[PR_TILE];
+    uint32_t val[PR_TILE];
+};
+
+// one segment (start, size <= PR_TILE) per CTA: load, stable LSD on the segment's varying bits in shared memory, store
+__global__ void __launch_bounds__(RS_THREADS, 2) k_bucket_sort(const uint64_t* __restrict__ kin, const uint32_t* __restrict__ vin,
+                                                              uint64_t* __restrict__ kout, uint32_t* __restrict__ vout,
+                                                              const uint2* __restrict__ segs) {
+    extern __shared__ __align__(16) uint8_t bs_raw[];
+    bs_stage* S = reinterpret_cast<bs_stage*>(bs_raw);
+    const unsigned tid = threadIdx.x, w = tid >> 5, lane = tid & 31u;
+    const uint2 seg = segs[blockIdx.x];
+    const uint64_t base = seg.x;
+    const uint32_t m = seg.y;
+    if (tid == 0) { S->or64 = 0ull; S->and64 = ~0ull; }
+    __syncthreads();
+    unsigned long long o64 = 0ull, a64 = ~0ull;
+    for (uint32_t i = tid; i < m; i += RS_THREADS) {
+        const uint64_t k = kin[base + i];
+        S->key[i] = k;
+        S->val[i] = vin[base + i];
+        o64 |= k; a64 &= k;
+    }
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) {
+        o64 |= __shfl_xor_sync(0xffffffffu, o64, o);
+        a64 &= __shfl_xor_sync(0xffffffffu, a64, o);
+    }
+    if (lane == 0) { atomicOr(&S->or64, o64); atomicAnd(&S->and64, a64); }
+    __syncthreads();
+    uint64_t vary = S->or64 ^ S->and64;
+    while (vary) {                                   // 8-bit windows from the lowest varying bit up (plan_windows)
+        const int shift = __ffsll((long long)vary) - 1;
+        vary = shift + 8 >= 64 ? 0ull : vary & (~0ull << (shift + 8));
+        uint64_t key[RS_ITEMS];
+        uint32_t val[RS_ITEMS], rk[RS_ITEMS];
+#pragma unroll
+        for (int j = 0; j < RS_ITEMS; j++) {
+            const uint32_t i = w * (32 * RS_ITEMS) + j * 32 + lane;
+            key[j] = i < m ? S->key[i] : 0ull;
+            val[j] = i < m ? S->val[i] : 0u;
+        }
+        for (unsigned i = tid; i < RS_WARPS * 256; i += RS_THREADS) (&S->whist[0][0])[i] = 0;
+        __syncthreads();
+#pragma unroll
+        for (int j = 0; j < RS_ITEMS; j++) {
+            const uint32_t i = w * (32 * RS_ITEMS) + j * 32 + lane;
+            const bool valid = i < m;
+            const uint32_t d = valid ? (uint32_t)((key[j] >> shift) & 255ull) : 256u;
+            const unsigned mm = __match_any_sync(0xffffffffu, d);
+            const unsigned r = __popc(mm & ((1u << lane) - 1u));
+            const int leader = __ffs(mm) - 1;
+            uint32_t old = 0;
+            if (valid && (int)lane == leader) {
+                old = S->whist[w][d];
+                S->whist[w][d] = old + __popc(mm);
+            }
+            old = __shfl_sync(0xffffffffu, old, leader);
+            rk[j] = (d << 16) | (old + r);
+            __syncwarp();
+        }
+        __syncthreads();
+        uint32_t tot = 0, incl = 0;
+        if (tid < 256) {
+#pragma unroll
+            for (int w2 = 0; w2 < RS_WARPS; w2++) {
+                const uint32_t c = S->whist[w2][tid];
+                S->whist[w2][tid] = tot;
+                tot += c;
+            }
+            incl = tot;
+#pragma unroll
+            for (int o = 1; o < 32; o <<= 1) {
+                const uint32_t t = __shfl_up_sync(0xffffffffu, incl, o);
+                if (lane >= (unsigned)o) incl += t;
+            }
+            if (lane == 31) S->wtot[w] = incl;
+        }
+        __syncthreads();
+        if (tid < 256) {
+            uint32_t wb = 0;
+#pragma unroll
+            for (int i = 0; i < 8; i++) if ((unsigned)i < w) wb += S->wtot[i];
+            S->dstart[tid] = wb + incl - tot;
+        }
+        __syncthreads();
+#pragma unroll
+        for (int j = 0; j < RS_ITEMS; j++) {
+            const uint32_t i = w * (32 * RS_ITEMS) + j * 32 + lane;
+            if (i < m) {
+                const uint32_t d = rk[j] >> 16;
+                const uint32_t slot = S->dstart[d] + S->whist[w][d] + (rk[j] & 0xffffu);
+                S->key[slot] = key[j];
+                S->val[slot] = val[j];
+            }
+        }
+        __syncthreads();
+    }
+    for (uint32_t i = tid; i < m; i += RS_THREADS) {
+        kout[base + i] = S->key[i];
+        vout[base + i] = S->val[i];
+    }
+}
+
+// One CTA per bucket split by the pass just made: its 256 digit runs (from the scanned counters) are packed greedily, in
+// order, into segments of at most PR_TILE items for k_bucket_sort; larger runs become the buckets of the next pass, with
+// their tiles.  last: no varying bit is left below the digit, every run is a run of equal keys, cut into segments (copies).
+__global__ void __launch_bounds__(256) k_msd_plan(const uint32_t* __restrict__ goff, const msd_bucket* __restrict__ buckets, int last,
+                                                 msd_counts* __restrict__ cnt, uint2* __restrict__ segs, msd_bucket* __restrict__ next,
+                                                 uint32_t* __restrict__ next_tile_bucket) {
+    __shared__ uint32_t st[257];
+    __shared__ uint2 lseg[256], lover[256];
+    __shared__ uint32_t nls, nlo, sbase, obase, t0s;
+    const unsigned tid = threadIdx.x;
+    const msd_bucket b = buckets[blockIdx.x];
+    const uint64_t h0 = (uint64_t)b.t0 * 256;
+    st[tid] = b.start + (goff[h0 + (uint64_t)tid * b.nt] - goff[h0]);
+    if (tid == 0) st[256] = b.start + b.size;
+    __syncthreads();
+    if (last) {
+        const uint32_t s = st[tid + 1] - st[tid], nch = (s + PR_TILE - 1) / PR_TILE;
+        if (nch) {
+            const uint32_t at = atomicAdd(&cnt->nseg, nch);
+            for (uint32_t k = 0; k < nch; k++) segs[at + k] = make_uint2(st[tid] + k * PR_TILE, min((uint32_t)PR_TILE, s - k * PR_TILE));
+        }
+        return;
+    }
+    if (tid == 0) {
+        uint32_t ns = 0, no = 0, cs = 0, cn = 0;
+        for (int d = 0; d < 256; d++) {
+            const uint32_t s = st[d + 1] - st[d];
+            if (s == 0) continue;
+            if (s > PR_TILE) {
+                if (cn) { lseg[ns++] = make_uint2(cs, cn); cn = 0; }
+                lover[no++] = make_uint2(st[d], s);
+            } else {
+                if (cn + s > PR_TILE) { lseg[ns++] = make_uint2(cs, cn); cn = 0; }
+                if (cn == 0) cs = st[d];
+                cn += s;
+            }
+        }
+        if (cn) lseg[ns++] = make_uint2(cs, cn);
+        nls = ns; nlo = no;
+        sbase = ns ? atomicAdd(&cnt->nseg, ns) : 0u;
+        obase = no ? atomicAdd(&cnt->nbuck, no) : 0u;
+    }
+    __syncthreads();
+    for (uint32_t i = tid; i < nls; i += 256) segs[sbase + i] = lseg[i];
+    for (uint32_t k = 0; k < nlo; k++) {
+        const uint2 o = lover[k];
+        const uint32_t nt = (o.y + PR_TILE - 1) / PR_TILE;
+        if (tid == 0) {
+            t0s = atomicAdd(&cnt->ntiles, nt);
+            next[obase + k] = msd_bucket{o.x, o.y, t0s, nt};
+        }
+        __syncthreads();
+        for (uint32_t t = tid; t < nt; t += 256) next_tile_bucket[t0s + t] = obase + k;
+        __syncthreads();
+    }
+}
+
+// highest 8-bit window below bit `below` that holds a varying bit (-1: none)
+static int msd_shift(uint64_t vary, int below) {
+    const uint64_t v = below >= 64 ? vary : vary & ((1ull << below) - 1);
+    if (!v) return -1;
+    const int hi = 63 - __builtin_clzll(v);
+    return hi >= 7 ? hi - 7 : 0;
+}
+
+static int msd_sort(uqb_ctx* ctx, uqb_sortbuf* sb, uint64_t n, const uint64_t* key_first, uint64_t vary) {
+    const uint32_t nblk = (uint32_t)((n + PR_TILE - 1) / PR_TILE);
+    const uint64_t cap_b = n / PR_TILE + 1, cap_t = nblk + cap_b;     // every bucket of a later pass holds > PR_TILE items
+    const int fin = sb->cur ^ 1;                                       // k_bucket_sort writes every segment here
+    msd_bucket* bk[2];
+    uint32_t* tb[2];
+    msd_counts* cnt;
+    UQB_TRY(uqb_dalloc_t(ctx, &bk[0], cap_b));
+    UQB_TRY(uqb_dalloc_t(ctx, &bk[1], cap_b));
+    UQB_TRY(uqb_dalloc_t(ctx, &tb[0], cap_t));
+    UQB_TRY(uqb_dalloc_t(ctx, &tb[1], cap_t));
+    UQB_TRY(uqb_dalloc_t(ctx, &cnt, 1));
+    const msd_bucket all = {0u, (uint32_t)n, 0u, nblk};
+    UQB_CUDA(cudaMemcpyAsync(bk[0], &all, sizeof(all), cudaMemcpyHostToDevice, ctx->stream));
+    UQB_CUDA(cudaMemsetAsync(tb[0], 0, (uint64_t)nblk * 4, ctx->stream));
+    auto k_radix_hist_seg = k_radix_hist<false, true>;
+    auto k_radix_scatter_seg = k_radix_scatter<false, false, true>;
+    UQB_CUDA(cudaFuncSetAttribute(k_radix_scatter_seg, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(rs_stage)));
+    UQB_CUDA(cudaFuncSetAttribute(k_bucket_sort, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(bs_stage)));
+    uint32_t nbuck = 1, ntiles = nblk;
+    uint64_t items = n;
+    int c = sb->cur, shift = msd_shift(vary, 64), lv = 0;
+    while (nbuck) {
+        const int o = c ^ 1, nxt = msd_shift(vary, shift);
+        const uint64_t* kin = (lv == 0 && key_first) ? key_first : sb->key[c];
+        const uint32_t* vin = (lv == 0 && key_first) ? nullptr : sb->val[c];
+        uint32_t* ghist;
+        const uint64_t hist_n = (uint64_t)256 * ntiles;
+        UQB_TRY(uqb_dalloc_t(ctx, &ghist, hist_n));
+        UQB_LAUNCH_B((uint64_t)items * 8, k_radix_hist_seg, ntiles, PR_THREADS, 0, kin, nullptr, n, shift, ghist, 0u, tb[lv & 1], bk[lv & 1]);
+        UQB_TRY(uqb_scan_u32(ctx, ghist, ghist, hist_n, nullptr));
+        UQB_LAUNCH_B((uint64_t)items * 24, k_radix_scatter_seg, ntiles, RS_THREADS, sizeof(rs_stage), kin, nullptr, vin, sb->key[o], nullptr,
+                     sb->val[o], n, shift, ghist, 0u, tb[lv & 1], bk[lv & 1]);
+        uint2* segs;
+        const uint64_t cap_s = (uint64_t)256 * nbuck + n / PR_TILE + 1;
+        UQB_TRY(uqb_dalloc_t(ctx, &segs, cap_s));
+        UQB_CUDA(cudaMemsetAsync(cnt, 0, sizeof(msd_counts), ctx->stream));
+        UQB_LAUNCH(k_msd_plan, nbuck, 256, 0, ghist, bk[lv & 1], nxt < 0 ? 1 : 0, cnt, segs, bk[(lv + 1) & 1], tb[(lv + 1) & 1]);
+        msd_counts got;
+        UQB_TRY(uqb_readback(ctx, &got, cnt, sizeof(got)));
+        if (got.nseg) UQB_LAUNCH_B(0, k_bucket_sort, got.nseg, RS_THREADS, sizeof(bs_stage), sb->key[o], sb->val[o], sb->key[fin], sb->val[fin], segs);
+        UQB_TRY(uqb_dfree(ctx, segs, cap_s * 8));
+        UQB_TRY(uqb_dfree(ctx, ghist, hist_n * 4));
+        nbuck = got.nbuck;
+        ntiles = got.ntiles;
+        items = (uint64_t)ntiles * PR_TILE;                // upper bound, for the byte count only
+        c = o;
+        shift = nxt;
+        lv++;
+    }
+    sb->cur = fin;
+    UQB_TRY(uqb_dfree(ctx, bk[0], cap_b * sizeof(msd_bucket)));
+    UQB_TRY(uqb_dfree(ctx, bk[1], cap_b * sizeof(msd_bucket)));
+    UQB_TRY(uqb_dfree(ctx, tb[0], cap_t * 4));
+    UQB_TRY(uqb_dfree(ctx, tb[1], cap_t * 4));
+    UQB_TRY(uqb_dfree(ctx, cnt, sizeof(msd_counts)));
+    return 0;
+}
+
 int uqb_radix_sort(uqb_ctx* ctx, uqb_sortbuf* sb, uint64_t n, bool use_aux, const uint64_t* key_first) {
     if (key_first && (use_aux || n < 2)) {            // plain path: materialise (key, index) in buffer 0
         if (n) UQB_LAUNCH_B(n * 20, k_key_iota, uqb_grid(ctx, n, 256 * 8), 256, 0, key_first, sb->key[sb->cur], sb->val[sb->cur], n);
@@ -691,6 +976,8 @@ int uqb_radix_sort(uqb_ctx* ctx, uqb_sortbuf* sb, uint64_t n, bool use_aux, cons
         return 0;
     }
 
+    const bool has_aux = sb->aux[0] != nullptr;
+    if (!use_aux && !has_aux && n >= MSD_MIN_N && nk >= 3) return msd_sort(ctx, sb, n, key_first, got.or64 ^ got.and64);
     uint32_t nblk = (uint32_t)((n + PR_TILE - 1) / PR_TILE);
     // Opt-in (UQB_RADIX_ONESWEEP=1): measured on B200 at 100 M keys it is SLOWER than the three kernels below (0.78 ms per
     // pass against 0.45 + 0.13 + 0.06 ms): a tile lasts ~5 us and a new one starts every ~18 ns, so the one-status-word-per-
@@ -725,7 +1012,6 @@ int uqb_radix_sort(uqb_ctx* ctx, uqb_sortbuf* sb, uint64_t n, bool use_aux, cons
     uint32_t* ghist;
     uint64_t hist_n = (uint64_t)256 * nblk;
     UQB_TRY(uqb_dalloc_t(ctx, &ghist, hist_n));
-    const bool has_aux = sb->aux[0] != nullptr;
     for (int p = 0; p < nk + na; p++) {
         bool auxd = p >= nk;
         int shift = auxd ? ashift[p - nk] : kshift[p];
@@ -742,9 +1028,9 @@ int uqb_radix_sort(uqb_ctx* ctx, uqb_sortbuf* sb, uint64_t n, bool use_aux, cons
         UQB_CUDA(cudaFuncSetAttribute(k_radix_scatter_aux, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)rs_smem));
         UQB_CUDA(cudaFuncSetAttribute(k_radix_scatter_key_aux, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)rs_smem));
         UQB_CUDA(cudaFuncSetAttribute(k_radix_scatter_key, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)rs_smem));
-        if (auxd)         UQB_LAUNCH_B(n * 32, k_radix_scatter_aux, nblk, RS_THREADS, rs_smem, kin, sb->aux[c], vin, sb->key[o], sb->aux[o], sb->val[o], n, shift, ghist, nblk);
-        else if (has_aux) UQB_LAUNCH_B(n * 32, k_radix_scatter_key_aux, nblk, RS_THREADS, rs_smem, kin, sb->aux[c], vin, sb->key[o], sb->aux[o], sb->val[o], n, shift, ghist, nblk);
-        else              UQB_LAUNCH_B(n * 24, k_radix_scatter_key, nblk, RS_THREADS, rs_smem, kin, sb->aux[c], vin, sb->key[o], sb->aux[o], sb->val[o], n, shift, ghist, nblk);
+        if (auxd)         UQB_LAUNCH_B(n * 32, k_radix_scatter_aux, nblk, RS_THREADS, rs_smem, kin, sb->aux[c], vin, sb->key[o], sb->aux[o], sb->val[o], n, shift, ghist, nblk, nullptr, nullptr);
+        else if (has_aux) UQB_LAUNCH_B(n * 32, k_radix_scatter_key_aux, nblk, RS_THREADS, rs_smem, kin, sb->aux[c], vin, sb->key[o], sb->aux[o], sb->val[o], n, shift, ghist, nblk, nullptr, nullptr);
+        else              UQB_LAUNCH_B(n * 24, k_radix_scatter_key, nblk, RS_THREADS, rs_smem, kin, sb->aux[c], vin, sb->key[o], sb->aux[o], sb->val[o], n, shift, ghist, nblk, nullptr, nullptr);
         sb->cur = o;
     }
     UQB_TRY(uqb_dfree(ctx, ghist, hist_n * 4));
