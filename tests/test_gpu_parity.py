@@ -502,38 +502,13 @@ def test_mix_feed_serves_every_mix_like_a_fresh_encode(ctx, name):
     dfq.free()
 
 
-@pytest.mark.parametrize("name", ["c1_raw_p01_31", "c2_keyed_sortDNA", "c3_casava_sortQNAME", "c4_twoNquals", "c6_checkpoints", "c7_offset_suffix_keyed"])
-def test_fused_scan_path_matches_reference_container(ctx, name, monkeypatch):
-    """UQB_FUSED_SCAN=1: one sweep (k_scan_hist) does the newline scan with decoupled look-back, line offsets, record
-    checks, histograms and the compact QNAME array; name statistics and the tokeniser then read the side array.  Same
-    containers as the default path, member for member."""
-    from uq_b200 import host
-    monkeypatch.setenv("UQB_FUSED_SCAN", "1")
-    from oracle import uq_literal as lit
-    fq, uq, kw = golden_case(name)
-    want, want_cfg = lit.read_container(uq)
-    got, got_cfg = host.encode(fq, ctx=ctx, **kw)
-    assert_members_equal(got, want, name)
-    assert_config_equal(got_cfg, want_cfg, name)
-    text = host.decode(got, got_cfg, ctx=ctx).tobytes()
-    assert records_multiset(text) == records_multiset(fq)
-
-
-def test_fused_scan_path_large_and_malformed(ctx, monkeypatch):
-    """the fused sweep over many tiles (look-back across tiles, records straddling tile ends) against the default path,
-    plus its error reporting (third line without '+', length mismatch) and its fallbacks (long records)."""
+def test_encode_reports_malformed_record_by_entry(ctx):
+    """host.encode names the record of a third line without '+' and of a quality line shorter than its sequence."""
     from uq_b200 import host
     dev = ctx.synth("genome", 700_000, 150, 77, genome=70_000, pool=100_000)
     data = dev.download().copy()
     dev.free()
-    want, want_cfg = host.encode(data, ctx=ctx, sort="QUAL")
-    monkeypatch.setenv("UQB_FUSED_SCAN", "1")
-    l0 = ctx.launches
-    got, got_cfg = host.encode(data, ctx=ctx, sort="QUAL")
-    assert_members_equal(got, want, "fused scan, 700 k reads")
-    assert_config_equal(got_cfg, want_cfg)
-    bad = bytearray(data[:400_000].tobytes())
-    lines = bytes(bad).split(b"\n")
+    lines = data[:400_000].tobytes().split(b"\n")
     lines[4 * 700 + 2] = b"-"                               # record 700: third line does not start with '+'
     lines[4 * 900 + 3] = lines[4 * 900 + 3][:-3]            # record 900: quality line three symbols short
     broken = b"\n".join(lines[:4 * 1000]) + b"\n"
@@ -543,11 +518,3 @@ def test_fused_scan_path_large_and_malformed(ctx, monkeypatch):
     broken = b"\n".join(lines[:4 * 1000]) + b"\n"
     with pytest.raises(host.UQError, match="for entry 901"):
         host.encode(broken, ctx=ctx)
-    # records longer than a tile's look-ahead: the sweep reports it and the line-offset kernels take over
-    from oracle import synth
-    long_fq = synth.make_fastq(kind="ont", n=40, length=(2000, 6000), seed=3)
-    monkeypatch.setenv("UQB_FUSED_SCAN", "0")
-    w2, c2 = host.encode(long_fq, ctx=ctx, sort="None", raw=["DNA", "QUAL", "QNAME"])
-    monkeypatch.setenv("UQB_FUSED_SCAN", "1")
-    g2, gc2 = host.encode(long_fq, ctx=ctx, sort="None", raw=["DNA", "QUAL", "QNAME"])
-    assert_members_equal(g2, w2, "long reads fall back")

@@ -6,7 +6,7 @@
 //   k_record_stats         generic fallback (names longer than 255 bytes, more than 64 distinct bytes in line 1)
 // Base and quality byte histograms plus "does this base always carry one single quality" (static_qualities,
 // uq.py:369-375, 420-425, read at uq.py:480-494):
-//   k_pair_hist_tiles      records that fit shared-memory tiles (double-buffered TMA tiles, tile.cuh)
+//   k_pair_hist_pipe       records that fit shared-memory tiles (TMA tiles in a three-stage pipeline, hist_units.cuh)
 //   k_pair_hist_long       long reads, straight from global memory
 //   k_pair_hist            generic fallback (bytes outside 32..127)
 // Counters are private per thread (packed 8-bit fields in shared memory or registers, flushed before they can
@@ -43,15 +43,6 @@ __global__ void k_an_init(an_dev* s) {
     }
     if (threadIdx.x == 0) {
         s->dna_min = ~0ull; s->dna_max = 0; s->bad_plus = LLONG_MAX; s->bad_len = LLONG_MAX; s->max_name_len = 0;
-    }
-}
-
-// the QNAME part of the accumulators alone (a new reference line restarts the name statistics, not the histograms)
-__global__ void k_an_init_names(an_dev* s) {
-    for (int i = threadIdx.x; i < 256; i += blockDim.x) s->last_count_mismatch[i] = -1;
-    for (int i = threadIdx.x; i <= UQB_HDR_MAX; i += blockDim.x) {
-        s->first_lcp_eq[i] = LLONG_MAX; s->first_lcs_eq[i] = LLONG_MAX;
-        s->first_short_prefix[i] = LLONG_MAX; s->first_short_suffix[i] = LLONG_MAX;
     }
 }
 
@@ -262,8 +253,8 @@ __global__ void __launch_bounds__(RD_THREADS) k_record_stats_names(const uint8_t
                                                                   const uint8_t* __restrict__ names, uint32_t name_pitch, int checks) {
     // checks == 0: the FASTQ shape checks and the read lengths are produced by the histogram kernel, which has the whole
     // record in shared memory anyway; this kernel then touches the first two line offsets and the name only
-    // names != nullptr: the QNAME lines come from the compact side array of sweep A (row r: length byte + text); the
-    // per-record FASTQ checks and read lengths were done there, only the name statistics are produced here
+    // names != nullptr: the QNAME lines come from the compact side array written by k_pair_hist_pipe (row r: length byte +
+    // text); the per-record FASTQ checks and read lengths were done there, only the name statistics are produced here
     extern __shared__ __align__(16) uint8_t rd_raw[];
     rd_smem* S = reinterpret_cast<rd_smem*>(rd_raw);
     const unsigned tid = threadIdx.x, lane = tid & 31u;
@@ -429,7 +420,7 @@ __global__ void __launch_bounds__(RD_THREADS) k_record_stats_names(const uint8_t
     if (tid < (unsigned)nslots && S->last_mis[tid]) atomicMax(&s->last_count_mismatch[S->slot_char[tid]], (long long)S->last_mis[tid] - 1);
 }
 
-// base / quality histograms from record tiles (one warp per record, lane = position mod 32).
+// base / quality histograms of long reads (k_pair_hist_long below).
 //
 // Qualities: private packed 8-bit counters per thread in shared memory ([word][thread] layout, bank-conflict
 // free), addressed through a LUT that puts neighbouring byte values into different words, flushed through a
@@ -454,10 +445,8 @@ __global__ void __launch_bounds__(RD_THREADS) k_record_stats_names(const uint8_t
 #define PT_CHECK 0x80000000u
 #define PT_GMASK 0xff000000u
 #define PT_NONE 0x7f000000u  // "no pending group yet"
-#define PT_UN 4              // chunks of 32 positions per unrolled step
 
 struct pt_smem {
-    tile2_smem T;
     unsigned priv_q[PT_WORDS * PT_THREADS];
     unsigned hist_b[256], hist_q[PT_LO + 4 * PT_WORDS];
     int state[256];                 // per base byte: -1 unseen, 0..255 its only quality so far, 256 = several
@@ -570,133 +559,13 @@ __device__ __noinline__ uint3 pt_base_slow(pt_smem* S, unsigned b, unsigned q, u
     return make_uint3(cur, pa, pb);
 }
 
-// K chunks of 32 positions of one record: lane handles positions lane + 32 k
-template <int K>
-__device__ __forceinline__ void pt_chunks(pt_smem* S, uint32_t dna_a, uint32_t qual_a, uint32_t lutb_a, uint32_t lutq_a, uint32_t pq_a,
-                                          uint32_t state_a, unsigned& cur, unsigned& pa, unsigned& pb) {
-    unsigned b[K], q[K];
-    uint2 eb[K], eq[K];
-#pragma unroll
-    for (int k = 0; k < K; k++) { b[k] = lds_u8(dna_a + 32 * k); q[k] = lds_u8(qual_a + 32 * k); }
-#pragma unroll
-    for (int k = 0; k < K; k++) { eb[k] = lds_u64(lutb_a + (b[k] << 3)); eq[k] = lds_u64(lutq_a + (q[k] << 3)); }
-#pragma unroll
-    for (int k = 0; k < K; k++) {                    // same-thread shared accesses stay in program order
-        const uint32_t wq = pq_a + eq[k].x;
-        sts_u32(wq, lds_u32(wq) + eq[k].y);
-    }
-#pragma unroll
-    for (int k = 0; k < K; k++) {
-        const unsigned dd = (eb[k].y ^ cur) & PT_GMASK;
-        // dd == PT_CHECK: a base of the current group that had one single quality so far - still the same one?
-        if (dd && (dd != PT_CHECK || lds_u32(state_a + (b[k] << 2)) != q[k])) {
-            const uint3 r = pt_base_slow(S, b[k], q[k], eb[k].y, cur, pa, pb);
-            cur = r.x; pa = r.y; pb = r.z;
-        }
-        pa += eb[k].x;
-        pb += eb[k].y;                               // the top byte collects group ids and is never read
-    }
-}
-
-#include "scan_kernel.cuh"
 #include "hist_units.cuh"
 
-__global__ void __launch_bounds__(PT_THREADS, 1) k_pair_hist_tiles(const uint8_t* __restrict__ d, uint64_t n_bytes,
-                                                               const uint64_t* __restrict__ line_off, uint64_t r_begin, uint64_t n_reads,
-                                                               an_dev* __restrict__ s, unsigned int* __restrict__ fallback) {
-    extern __shared__ __align__(128) uint8_t pt_raw[];
-    pt_smem* S = reinterpret_cast<pt_smem*>(pt_raw);
-    const unsigned tid = threadIdx.x, lane = tid & 31u, wid = tid >> 5;
-    for (unsigned i = tid; i < PT_WORDS * PT_THREADS; i += PT_THREADS) S->priv_q[i] = 0;
-    for (unsigned i = tid; i < PT_LO + 4 * PT_WORDS; i += PT_THREADS) S->hist_q[i] = 0;
-    for (unsigned i = tid; i < PT_GROUPS * 8; i += PT_THREADS) S->rev[i] = 0;
-    if (tid < 256) { S->hist_b[tid] = 0; S->state[tid] = -1; }
-    __syncthreads();
-    if (tid < 256) {
-        const unsigned v = tid;
-        unsigned grp, field;
-        pt_base_group(v, &grp, &field);
-        S->lutb[v] = make_uint2(field < 4 ? 1u << (8 * field) : 0u, ((grp << 24) | PT_CHECK) | (field >= 4 ? 1u << (8 * (field - 4)) : 0u));
-        S->rev[grp * 8 + field] = (uint8_t)v;
-        // qualities: neighbouring byte values go to DIFFERENT counter words (word = idx % 24, field = idx / 24): a
-        // thread that meets two adjacent qualities in a row does not read a word it has just stored
-        const unsigned idx = min(v - PT_LO, PT_OOR);                          // out of range -> slot 96
-        const unsigned word = idx < 96u ? idx % 24u : 24u, qf = idx < 96u ? idx / 24u : 0u;
-        S->lutq[v] = make_uint2(word * PT_ROW, 1u << (8 * qf));
-    }
-    __syncthreads();
-    const uint32_t pq_a = smem_u32(S->priv_q + tid);
-    const uint32_t lutb_a = smem_u32(S->lutb), lutq_a = smem_u32(S->lutq), state_a = smem_u32(S->state);
-    unsigned since_flush = 0;
-    unsigned cur = PT_NONE, pa = 0, pb = 0;                  // pending base group (none yet) and its 7 counters
-    tile2_pipe<PT_THREADS> P;
-    for (P.begin(&S->T, d, n_bytes, line_off, r_begin, n_reads); P.valid(); P.finish()) {
-        const uint32_t nrec = P.acquire();
-        if (!nrec) { if (tid == 0) atomicOr(fallback, 1u); continue; }
-        const uint32_t bytes_a = smem_u32(P.bytes());
-        const uint32_t* loff = P.loff();
-        for (uint32_t i = wid; i < nrec; i += PT_THREADS / 32) {
-            const uint32_t o1 = loff[4 * i + 1], o2 = loff[4 * i + 2], o3 = loff[4 * i + 3], o4 = loff[4 * i + 4];
-            uint32_t len = o2 - o1 - 1;
-            const uint32_t qlen = o4 - o3 - 1;
-            if (qlen < len) len = qlen;            // malformed records are reported by the record-stats kernel
-            const uint32_t full = len >> 5, tail = len & 31u, iters = full + (tail ? 1u : 0u);
-            uint32_t dna_a = bytes_a + o1 + lane, qual_a = bytes_a + o3 + lane;
-            if (iters > 254u) {
-                // a single read longer than 254*32 bases (only when the rest of the tile is tiny): plain shared atomics
-                pt_base_flush_warp(S, cur, pa, pb, lane);
-                for (uint32_t p = lane; p < len; p += 32) {
-                    const unsigned b = lds_u8(dna_a + (p - lane)), q = lds_u8(qual_a + (p - lane));
-                    atomicAdd(&S->hist_b[b], 1u);
-                    atomicAdd(&S->hist_q[q - PT_LO < 96u ? q : PT_LO + PT_OOR], 1u);
-                    const unsigned ey = S->lutb[b].y;
-                    if (ey & PT_CHECK) pt_base_slow(S, b, q, ey, ey & (PT_GMASK & ~PT_CHECK), 0u, 0u);
-                }
-                continue;
-            }
-            if (since_flush + iters > 254u) {      // warp-uniform; a counter is bumped at most once per iteration
-                pt_flush(S->priv_q, S->hist_q, tid);
-                pt_base_flush_warp(S, cur, pa, pb, lane);
-                since_flush = 0;
-            }
-            since_flush += iters;
-            uint32_t it = 0;
-            for (; it + PT_UN <= full; it += PT_UN) {
-                pt_chunks<PT_UN>(S, dna_a, qual_a, lutb_a, lutq_a, pq_a, state_a, cur, pa, pb);
-                dna_a += 32 * PT_UN; qual_a += 32 * PT_UN;
-            }
-            for (; it < full; it++) {
-                pt_chunks<1>(S, dna_a, qual_a, lutb_a, lutq_a, pq_a, state_a, cur, pa, pb);
-                dna_a += 32; qual_a += 32;
-            }
-            if (lane < tail) pt_chunks<1>(S, dna_a, qual_a, lutb_a, lutq_a, pq_a, state_a, cur, pa, pb);
-        }
-    }
-    pt_flush(S->priv_q, S->hist_q, tid);
-    pt_base_flush(S, cur, pa, pb);
-    __syncthreads();
-    if (tid < 256) {
-        if (S->hist_b[tid]) atomicAdd(&s->base_count[tid], (unsigned long long)S->hist_b[tid]);
-        if (tid < 128 && S->hist_q[tid]) atomicAdd(&s->qual_count[tid], (unsigned long long)S->hist_q[tid]);
-        if (tid == 0 && S->hist_q[PT_LO + PT_OOR]) atomicOr(fallback, 1u);
-        const int f = S->state[tid];
-        if (f >= 0) {
-            if (f == 256) {
-                s->multi[tid] = 1;
-                atomicCAS(&s->first_q[tid], -1, 0);                 // mark the base as present
-            } else {
-                const int old = atomicCAS(&s->first_q[tid], -1, f);
-                if (old >= 0 && old != f) s->multi[tid] = 1;
-            }
-        }
-    }
-}
-
-// Long reads (records that do not fit a tile): the same counters, fed straight from global memory.  One warp per
+// Long reads (records that do not fit a tile): the counters above, fed straight from global memory.  One warp per
 // record; a lane takes aligned 16-byte units of the DNA line and, separately, of the QUAL line (the two lines have
 // different alignments, and counting does not need them paired).  Only a base that still carries the CHECK bit needs
-// its own quality: that single byte is fetched on the spot.  Same shared-memory layout as the tile kernel (the tile
-// area is simply unused), same flush rules: at most 15 units (240 increments of one 8-bit field) between flushes.
+// its own quality: that single byte is fetched on the spot.  At most 15 units (240 increments of one 8-bit field)
+// between flushes.
 __device__ __forceinline__ void pt_long_base(pt_smem* S, const uint8_t* __restrict__ d, uint64_t qbase, uint64_t pos0, unsigned b, unsigned k,
                                              uint32_t lutb_a, uint32_t state_a, unsigned& cur, unsigned& pa, unsigned& pb) {
     const uint2 e = lds_u64(lutb_a + (b << 3));
@@ -801,6 +670,7 @@ __global__ void __launch_bounds__(PT_THREADS, 1) k_pair_hist_long(const uint8_t*
 // long reads: names-only record statistics + the direct histogram above
 static int stats_long_range(uqb_ctx* ctx, const uqb_fastq* fq, an_dev* s, unsigned int* d_fb, uint32_t flen, uint64_t r0, uint64_t r1) {
     if (r1 <= r0) return 0;
+    static_assert(sizeof(pt_smem) <= 227 * 1024, "pair histogram shared memory");
     UQB_CUDA(cudaFuncSetAttribute(k_pair_hist_long, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(pt_smem)));
     UQB_LAUNCH_B((r1 - r0) * 128, k_record_stats_names, uqb_grid(ctx, r1 - r0, RD_THREADS, 8), RD_THREADS, sizeof(rd_smem), fq->d, fq->line_off, r0, r1,
                  fq->ref_name ? fq->ref_name : fq->d, fq->rbase, flen, s, d_fb, (const uint8_t*)nullptr, 0u, 1);
@@ -816,26 +686,12 @@ static int stats_long_range(uqb_ctx* ctx, const uqb_fastq* fq, an_dev* s, unsign
 static int stats_tiles_range(uqb_ctx* ctx, const uqb_fastq* fq, an_dev* s, unsigned int* d_fb, uint32_t flen, uint64_t r0, uint64_t r1) {
     if (r1 <= r0) return 0;
     const uint64_t ntiles = (r1 - r0 + TL_R - 1) / TL_R;
-    UQB_CUDA(cudaFuncSetAttribute(k_pair_hist_tiles, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(pt_smem)));
     const unsigned g2 = (unsigned)(ntiles < (uint64_t)ctx->sm_count ? ntiles : (uint64_t)ctx->sm_count);      // one 1024-thread CTA per SM
-    static_assert(sizeof(pt_smem) <= 227 * 1024, "pair histogram shared memory");
     const uint64_t ab = (uint64_t)((double)fq->n * (double)(r1 - r0) / (double)(fq->n_reads ? fq->n_reads : 1)) + 32 * (r1 - r0);
-    static const bool hist_v1 = [] { const char* e = getenv("UQB_HIST_V1"); return e && e[0] == '1'; }();
-    // names only: 32 B of offsets and the name's sectors per record (plus the '+' sector when it also makes the record checks)
-    UQB_LAUNCH_B((r1 - r0) * (hist_v1 ? 128 : 96), k_record_stats_names, uqb_grid(ctx, r1 - r0, RD_THREADS, 8), RD_THREADS, sizeof(rd_smem), fq->d, fq->line_off, r0, r1,
-                 fq->ref_name ? fq->ref_name : fq->d, fq->rbase, flen, s, d_fb, (const uint8_t*)nullptr, 0u, hist_v1 ? 1 : 0);
-    if (hist_v1) {
-        UQB_LAUNCH_B(ab, k_pair_hist_tiles, g2, PT_THREADS, sizeof(pt_smem), fq->d, fq->n, fq->line_off, r0, r1, s, d_fb);
-        return 0;
-    }
-    static_assert(sizeof(h2_smem) <= 227 * 1024, "unit histogram shared memory");
+    // names only: 32 B of offsets and the name's sectors per record
+    UQB_LAUNCH_B((r1 - r0) * 96, k_record_stats_names, uqb_grid(ctx, r1 - r0, RD_THREADS, 8), RD_THREADS, sizeof(rd_smem), fq->d, fq->line_off, r0, r1,
+                 fq->ref_name ? fq->ref_name : fq->d, fq->rbase, flen, s, d_fb, (const uint8_t*)nullptr, 0u, 0);
     static_assert(sizeof(h3_smem) <= 227 * 1024, "pipelined unit histogram shared memory");
-    static const bool hist_v2 = [] { const char* e = getenv("UQB_HIST_V2"); return e && e[0] == '1'; }();
-    if (hist_v2) {
-        UQB_CUDA(cudaFuncSetAttribute(k_pair_hist_units, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(h2_smem)));
-        UQB_LAUNCH_B(ab, k_pair_hist_units, g2, H2_THREADS, sizeof(h2_smem), fq->d, fq->n, fq->line_off, r0, r1, s, d_fb);
-        return 0;
-    }
     UQB_CUDA(cudaFuncSetAttribute(k_pair_hist_pipe, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(h3_smem)));
     UQB_LAUNCH_B(ab, k_pair_hist_pipe, g2, H2_THREADS, sizeof(h3_smem), fq->d, fq->n, fq->line_off, r0, r1, s, d_fb, (uint8_t*)nullptr, 0u);
     return 0;
@@ -847,10 +703,9 @@ static int stats_tiles_range(uqb_ctx* ctx, const uqb_fastq* fq, an_dev* s, unsig
 static int stats_tiles_resident(uqb_ctx* ctx, uqb_fastq* fq, an_dev* s, unsigned int* d_fb, uint32_t flen, uint32_t own_first_len,
                                 unsigned int* fb_out) {
     const uint64_t N = fq->n_reads;
-    static const bool plain = [] { const char* e = getenv("UQB_NO_NAMES"); return (e && e[0] == '1') || getenv("UQB_HIST_V1") || getenv("UQB_HIST_V2"); }();
     uint32_t pitch = (own_first_len + 1 + 24 + 15) / 16 * 16;
     if (pitch < 32) pitch = 32;
-    if (plain || pitch > 256 || fq->names) {
+    if (pitch > 256 || fq->names) {
         UQB_TRY(stats_tiles_range(ctx, fq, s, d_fb, flen, 0, N));
         UQB_TRY(uqb_readback(ctx, fb_out, d_fb, 4));
         return 0;
@@ -938,134 +793,9 @@ static int stats_finish(uqb_ctx* ctx, uqb_fastq* fq, an_dev* s, uqb_stats* out, 
     return 0;
 }
 
-// ================================================================================================
-// Sweep A over a resident file: k_scan_hist (scan_kernel.cuh) in two launches - a short one over the first tiles, whose
-// line count sizes the line-offset and QNAME arrays for the rest - then nothing else touches the FASTQ until the packer.
-// ================================================================================================
-__global__ void k_scan_set_ticket(unsigned int* ticket, unsigned int v) { *ticket = v; }
-
-int uqb_scan_release(uqb_ctx* ctx, uqb_fastq* fq) {
+int uqb_names_release(uqb_ctx* ctx, uqb_fastq* fq) {
     if (fq->names) { UQB_TRY(uqb_dfree(ctx, fq->names, 0)); fq->names = nullptr; }
-    if (fq->scan_acc) { UQB_TRY(uqb_dfree(ctx, fq->scan_acc, 0)); fq->scan_acc = nullptr; }
-    fq->name_pitch = 0; fq->names_cap = 0; fq->line_cap = 0;
-    return 0;
-}
-
-// Opt-in (UQB_FUSED_SCAN=1).  Measured on a B200 at 100 M reads x 150 bp (profiles/README.md, round 2): the fused sweep
-// reads the FASTQ once (DRAM reads of the step: 2.0 x F instead of 5.6 x F) but takes 51 ms + 6 ms of name statistics
-// against 48 ms for the four line-offset based kernels - it is instruction-issue bound (1.0 warp instructions per byte:
-// newline ranking 23 %, histogram loop 40 %, deferred line-offset / QNAME writes 10 %), not bandwidth bound, so fewer
-// bytes did not buy time.  The default path therefore stays with the separate kernels.
-static bool scan_enabled() {
-    const char* e = getenv("UQB_FUSED_SCAN");
-    return e && e[0] == '1';
-}
-
-int uqb_scan_file(uqb_ctx* ctx, uqb_fastq* fq, bool* done) {
-    *done = false;
-    if (!scan_enabled() || fq->n < 64 || (((uintptr_t)fq->d) & 15) != 0) return 0;
-    const uint64_t n = fq->n;
-    if ((n + SC_T - 1) / SC_T >= (1ull << 31)) return 0;
-    // ---- a look at the head of the file: length of the first QNAME line (row pitch of the side array), line density ----
-    uint8_t head[4096];
-    const size_t hn = n < sizeof(head) ? (size_t)n : sizeof(head);
-    UQB_TRY(uqb_readback(ctx, head, fq->d, hn));
-    size_t first_len = 0, head_lines = 0;
-    while (first_len < hn && head[first_len] != '\n') first_len++;
-    if (first_len == hn || first_len > 200) return 0;                 // no newline in sight / long names: line-offset kernels
-    for (size_t i = 0; i < hn; i++) head_lines += head[i] == '\n';
-    uint32_t pitch = (uint32_t)((first_len + 1 + 24 + 15) / 16 * 16);
-    if (pitch < 32) pitch = 32;
-    if (pitch > 256) pitch = 256;
-    const uint32_t ntiles = (uint32_t)((n + SC_T - 1) / SC_T);
-    const uint32_t t_first = ntiles < 192 ? ntiles : 128;              // the first launch: up to 128 tiles (2.7 MB)
-
-    uint64_t* status = nullptr;
-    unsigned int *ticket = nullptr, *d_fb = nullptr;
-    unsigned long long* d_total = nullptr;
-    an_dev* acc = nullptr;
-    UQB_TRY(uqb_dalloc_t(ctx, &status, ntiles));
-    UQB_TRY(uqb_dalloc_t(ctx, &ticket, 1));
-    UQB_TRY(uqb_dalloc_t(ctx, &d_fb, 1));
-    UQB_TRY(uqb_dalloc_t(ctx, &d_total, 1));
-    UQB_TRY(uqb_dalloc_t(ctx, &acc, 1));
-    UQB_CUDA(cudaMemsetAsync(status, 0, (size_t)ntiles * 8, ctx->stream));
-    UQB_CUDA(cudaMemsetAsync(d_fb, 0, 4, ctx->stream));
-    UQB_CUDA(cudaMemsetAsync(d_total, 0, 8, ctx->stream));
-    UQB_LAUNCH(k_an_init, 1, 256, 0, acc);
-    UQB_CUDA(cudaFuncSetAttribute(k_scan_hist, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(sc_smem)));
-    UQB_CUDA(cudaFuncSetAttribute(k_scan_hist, cudaFuncAttributePreferredSharedMemoryCarveout, (int)cudaSharedmemCarveoutMaxShared));
-
-    auto release = [&]() {
-        uqb_dfree(ctx, status, 0); uqb_dfree(ctx, ticket, 0); uqb_dfree(ctx, d_fb, 0); uqb_dfree(ctx, d_total, 0);
-    };
-    uint64_t* line_off = nullptr;
-    uint8_t* names = nullptr;
-    uint64_t cap_lines = 0, cap_records = 0;
-    bool ok = true;
-    for (int pass = 0; pass < 2 && ok; pass++) {
-        const uint32_t t0 = pass == 0 ? 0u : t_first, t1 = pass == 0 ? t_first : ntiles;
-        if (t1 <= t0) break;
-        // capacity: pass 0 from the density of the head (x2), pass 1 from the density of the first tiles (+6 %)
-        uint64_t want_lines;
-        if (pass == 0) {
-            const double dens = (double)(head_lines + 1) / (double)hn;
-            want_lines = (uint64_t)(dens * 2.0 * (double)((uint64_t)t1 * SC_T + SC_LOAD)) + 4096;
-        } else {
-            uint64_t st = 0;
-            UQB_TRY(uqb_readback(ctx, &st, status + (t_first - 1), 8));
-            unsigned int fb = 0;
-            UQB_TRY(uqb_readback(ctx, &fb, d_fb, 4));
-            if (fb || (st >> 62) != 2ull) { ok = false; break; }
-            const uint64_t lines_head = st & ((1ull << 62) - 1);
-            const double dens = (double)(lines_head + 1) / (double)((uint64_t)t_first * SC_T);
-            want_lines = (uint64_t)(dens * 1.06 * (double)n) + (1u << 16);
-        }
-        if (want_lines > n + 1) want_lines = n + 1;
-        const uint64_t want_records = want_lines / 4 + 2;
-        uint64_t* lo2;
-        uint8_t* nm2;
-        UQB_TRY(uqb_dalloc_t(ctx, &lo2, want_lines + 2));
-        UQB_TRY(uqb_dalloc(ctx, (void**)&nm2, want_records * pitch + 64));
-        if (line_off) {                                               // keep what the first launch produced
-            UQB_CUDA(cudaMemcpyAsync(lo2, line_off, (cap_lines + 1 < want_lines + 1 ? cap_lines + 1 : want_lines + 1) * 8, cudaMemcpyDeviceToDevice, ctx->stream));
-            UQB_CUDA(cudaMemcpyAsync(nm2, names, (cap_records < want_records ? cap_records : want_records) * pitch, cudaMemcpyDeviceToDevice, ctx->stream));
-            UQB_TRY(uqb_dfree(ctx, line_off, 0));
-            UQB_TRY(uqb_dfree(ctx, names, 0));
-        } else {
-            UQB_TRY(uqb_split_set_first(ctx, lo2));
-        }
-        line_off = lo2; names = nm2; cap_lines = want_lines; cap_records = want_records;
-        sc_params P;
-        P.d = fq->d; P.n = n; P.n_avail = n; P.tile_end = t1; P.status = status; P.ticket = ticket;
-        P.line_off = line_off; P.cap_lines = cap_lines; P.names = names; P.name_pitch = pitch; P.cap_records = cap_records;
-        P.s = acc; P.fallback = d_fb; P.lines_total = d_total;
-        UQB_LAUNCH(k_scan_set_ticket, 1, 1, 0, ticket, t0);
-        const unsigned gmax = (unsigned)SC_CTAS_PER_SM * (unsigned)ctx->sm_count;
-        const unsigned grid = (t1 - t0) < gmax ? (t1 - t0) : gmax;
-        const uint64_t span = (uint64_t)(t1 - t0) * SC_T;
-        UQB_LAUNCH_B(span < n ? span : n, k_scan_hist, grid, SC_THREADS, sizeof(sc_smem), P);
-    }
-    unsigned int fb = 0;
-    unsigned long long total = 0;
-    if (ok) {
-        UQB_TRY(uqb_readback(ctx, &fb, d_fb, 4));
-        UQB_TRY(uqb_readback(ctx, &total, d_total, 8));
-        if (fb) ok = false;
-        uqb_timer_add_bytes(ctx, 8 * total + total / 4 * pitch);       // line offsets and QNAME rows written
-    }
-    release();
-    if (!ok) {
-        if (line_off) UQB_TRY(uqb_dfree(ctx, line_off, 0));
-        if (names) UQB_TRY(uqb_dfree(ctx, names, 0));
-        UQB_TRY(uqb_dfree(ctx, acc, 0));
-        return 0;                                                     // the caller runs the line-offset based kernels
-    }
-    fq->line_off = line_off; fq->line_cap = cap_lines + 2;
-    fq->n_lines = total; fq->n_reads = total / 4;
-    fq->names = names; fq->name_pitch = pitch; fq->names_cap = cap_records;
-    fq->scan_acc = acc;
-    *done = true;
+    fq->name_pitch = 0; fq->names_cap = 0;
     return 0;
 }
 
@@ -1093,27 +823,6 @@ extern "C" int uqb_analyze(uqb_ctx* ctx, uqb_fastq* fq, uqb_stats* out) {
     uint64_t flen = 0;
     UQB_TRY(stats_names(ctx, fq, out, &flen));
     if (fq->ref_name) flen = fq->ref_len;        // multi-GPU shard: everything is measured against the global line 1
-    if (fq->scan_acc && fq->names) {
-        // sweep A has produced the histograms, the record checks and the compact QNAME array: only the name statistics
-        // (against the current reference line) are left, and they never touch the FASTQ bytes
-        an_dev* acc = (an_dev*)fq->scan_acc;
-        unsigned int* d_fb;
-        UQB_TRY(uqb_dalloc_t(ctx, &d_fb, 1));
-        UQB_CUDA(cudaMemsetAsync(d_fb, 0, 4, ctx->stream));
-        UQB_LAUNCH(k_an_init_names, 1, 256, 0, acc);
-        UQB_LAUNCH_B(N * fq->name_pitch, k_record_stats_names, uqb_grid(ctx, N, RD_THREADS, 8), RD_THREADS, sizeof(rd_smem), fq->d, fq->line_off,
-                     0ull, N, fq->ref_name ? fq->ref_name : fq->d, fq->rbase, (uint32_t)flen, acc, d_fb, (const uint8_t*)fq->names, fq->name_pitch, 1);
-        unsigned int fb = 0;
-        UQB_TRY(uqb_readback(ctx, &fb, d_fb, 4));
-        UQB_TRY(uqb_dfree(ctx, d_fb, 4));
-        if (fb) {                                 // line 1 defeats the packed counters: generic name statistics
-            UQB_LAUNCH(k_an_init_names, 1, 256, 0, acc);
-            UQB_LAUNCH(k_record_stats, uqb_blocks(N, AN_THREADS), AN_THREADS, 0, fq->d, fq->line_off, N,
-                       fq->ref_name ? fq->ref_name : fq->d, fq->rbase, (uint32_t)flen, acc);
-        }
-        UQB_TRY(stats_finish(ctx, fq, acc, out, flen));
-        return 0;
-    }
     an_dev* s;
     UQB_TRY(uqb_dalloc_t(ctx, &s, 1));
     bool done_fast = false;

@@ -83,13 +83,11 @@ struct uqb_fastq {
     uint8_t* ref_name = nullptr;
     uint32_t ref_len = 0;
     uint64_t rbase = 0;
-    // sweep A (k_scan_hist): QNAME lines in a compact side array (row r: length byte + text, name_pitch bytes) and the
-    // device accumulators of the Pass-1 statistics (an_dev*, analyze.cu) - both stay with the handle
+    // QNAME lines in a compact side array (row r: length byte + text, name_pitch bytes), written by the histogram kernel
+    // of uqb_analyze (k_pair_hist_pipe) - it stays with the handle
     uint8_t* names = nullptr;
     uint32_t name_pitch = 0;
     uint64_t names_cap = 0;
-    uint64_t line_cap = 0;        // entries allocated for line_off (the fused scan sizes it from an estimate)
-    void* scan_acc = nullptr;
     bool streamed = false;        // split + Pass-1 statistics were produced while the bytes streamed in
     uqb_stats* cached_stats = nullptr;
     uint32_t prefix_len = 0, suffix_len = 0, ncols = 0;
@@ -187,10 +185,8 @@ int uqb_split_write_tiles(uqb_ctx* ctx, const uint8_t* d, uint64_t n_end, uint64
                           const uint64_t* bases, uint64_t* line_off);
 int uqb_split_set_first(uqb_ctx* ctx, uint64_t* line_off);
 int uqb_copy_stream(uqb_ctx* ctx, cudaStream_t* out);
-// fused sweep A over a resident file (analyze.cu): on success *done = true and the handle holds line offsets, the
-// compact QNAME array and the statistics accumulators; *done = false means "use the line-offset based kernels"
-int uqb_scan_file(uqb_ctx* ctx, uqb_fastq* fq, bool* done);
-int uqb_scan_release(uqb_ctx* ctx, uqb_fastq* fq);
+// frees the compact QNAME array of the handle (analyze.cu)
+int uqb_names_release(uqb_ctx* ctx, uqb_fastq* fq);
 
 // ---- primitives (prims.cu) ---------------------------------------------------------------------
 // exclusive prefix sum of n uint32 values into uint32 / uint64; total written to *d_total (device)

@@ -1,8 +1,8 @@
-// k_pair_hist_units: base / quality byte histograms and "does this base always carry one single quality"
+// k_pair_hist_pipe: base / quality byte histograms and "does this base always carry one single quality"
 // (static_qualities, uq.py:369-375, 420-425, read at uq.py:480-494) over shared-memory record tiles, sixteen
 // positions per work item.
 //
-// A tile is 128 records (tile.cuh, double-buffered TMA bulk copies).  The 1024 threads of the CTA are bound to the
+// A tile is 128 records (TMA bulk copies, see the pipeline below).  The 1024 threads of the CTA are bound to the
 // 256 DNA / QUAL lines of the tile: thread t owns line (t & 255) - lines 0..127 are the DNA lines, 128..255 the QUAL
 // lines of records 0..127 - and walks the ALIGNED 16-byte units k = t >> 8, +4, +8, ... of that line (one
 // ld.shared.v4 each; units are warp-uniform, so the masked first / last units of the lines gather in few warps).
@@ -34,12 +34,6 @@ struct h2_core {                    // CTA-wide results
     unsigned hist_q[H2_ROWS + 1];
     int state[256];                 // per base byte: -1 unseen, 0..255 its only quality so far, 256 = several
     unsigned hints, dirty, oor, qmax;
-};
-
-struct h2_smem {
-    tile2_smem T;
-    alignas(16) uint8_t qcnt[H2_ROWS * H2_COLS];
-    h2_core C;
 };
 
 __device__ __forceinline__ uint4 lds_v4(uint32_t a) {
@@ -214,154 +208,10 @@ __device__ __noinline__ void h2_qual_flush(h2_core* S, uint32_t qcol) {
     }
 }
 
-__global__ void __launch_bounds__(H2_THREADS, 1) k_pair_hist_units(const uint8_t* __restrict__ d, uint64_t n_bytes,
-                                                                  const uint64_t* __restrict__ line_off, uint64_t r_begin, uint64_t n_reads,
-                                                                  an_dev* __restrict__ s, unsigned int* __restrict__ fallback) {
-    static_assert(TL_R == 128, "thread <-> line binding assumes 128 records per tile");
-    extern __shared__ __align__(128) uint8_t h2_raw[];
-    h2_smem* S = reinterpret_cast<h2_smem*>(h2_raw);
-    const unsigned tid = threadIdx.x, lane = tid & 31u, wid = tid >> 5;
-    for (unsigned i = tid; i < H2_ROWS * H2_COLS / 4; i += H2_THREADS) reinterpret_cast<uint32_t*>(S->qcnt)[i] = 0;
-    for (unsigned i = tid; i <= H2_ROWS; i += H2_THREADS) S->C.hist_q[i] = 0;
-    if (tid < 256) { S->C.hist_b[tid] = 0; S->C.state[tid] = -1; }
-    if (tid == 0) { S->C.hints = H2_NOHINT; S->C.dirty = 0; S->C.oor = 0; }
-    __syncthreads();
-    const unsigned line = tid & 255u, rec = line & 127u, k0 = tid >> 8;
-    const bool isq = (line >> 7) != 0;
-    const unsigned cw = ((wid >> 3) << 2) | (wid & 3u);                       // QUAL warps 4-7, 12-15, ... -> 0..15
-    const uint32_t qcol = smem_u32(S->qcnt) + lane * 4u + (cw & 3u) + 128u * (cw >> 2) - (H2_QLO << 9);
-    unsigned qsym = 0;                                                        // increments of this column since its last flush
-    h2_dna_acc A;
-    A.p0 = A.p1 = A.p01 = A.ocnt = A.words = A.zeroed = A.noff = 0;
-    unsigned H = H2_NOHINT;
-    // FASTQ shape checks and read-length range (uq.py:360-366, 382-388): the thread of a record's first DNA unit
-    unsigned long long len_min = ~0ull, len_max = 0ull;
-    long long bad_plus = LLONG_MAX, bad_len = LLONG_MAX;
-    tile2_pipe<H2_THREADS> P;
-    P.begin(&S->T, d, n_bytes, line_off, r_begin, n_reads);
-    while (P.valid()) {
-        const uint32_t nrec = P.acquire();
-        unsigned tile_sym = 0;                                                // symbols this thread took from this tile
-        if (!nrec) {
-            if (tid == 0) atomicOr(fallback, 1u);
-        } else if (rec < nrec) {
-            const uint32_t bytes_a = smem_u32(P.bytes());
-            const uint32_t* loff = P.loff();
-            const uint32_t o1 = loff[4 * rec + 1], o2 = loff[4 * rec + 2], o3 = loff[4 * rec + 3], o4 = loff[4 * rec + 4];
-            uint32_t len = o2 - o1 - 1;
-            const uint32_t qlen = o4 - o3 - 1;
-            if (tid < TL_R) {                          // DNA thread of unit 0: the record's checks
-                const long long r = (long long)(P.first_record() + rec);
-                const uint32_t dlen = len;
-                if (dlen != qlen && r < bad_len) bad_len = r;
-                len_min = dlen < len_min ? dlen : len_min; len_max = dlen > len_max ? dlen : len_max;
-                const unsigned plus = o3 - o2 < 2u ? 0u : lds_u8(bytes_a + o2);
-                if (plus != '+' && r < bad_plus) bad_plus = r;
-            }
-            if (qlen < len) len = qlen;
-            const uint32_t sb = isq ? o3 : o1, eb = sb + len;
-            for (uint32_t u = (sb & ~15u) + 16u * k0; u < eb; u += 64u) {
-                const uint4 v = lds_v4(bytes_a + u);
-                const int lo = (int)sb - (int)u, hi = (int)eb - (int)u;      // valid bytes of the unit: [lo, hi) clipped to 0..16
-                if (isq) {
-                    if (qsym > 255u - 16u) { h2_qual_flush(&S->C, qcol); qsym = 0; }
-                    if (!h2_qual_unit(v, lo, hi, qcol)) S->C.oor = 1u;
-                    qsym += 16u;
-                } else {
-                    if (A.words > 120u || A.noff > 224u) h2_dna_flush(&S->C, A, H);
-                    h2_dna_unit(&S->C, v, bytes_a + u, o3 - o1, lo, hi, H, A);
-                }
-                tile_sym += 16u;
-            }
-        }
-        // CTA-wide flush before any 8-bit field can overflow in the next tile (assumed no larger than this one), or when
-        // a base has become a hint candidate
-        const bool vote = isq ? (qsym + tile_sym > 255u - 16u) : (A.words + (tile_sym >> 2) > 120u || A.noff + tile_sym > 224u || (tid == 0 && S->C.dirty));
-        if (P.finish_or(vote)) {
-            for (unsigned r = wid; r < H2_ROWS; r += H2_THREADS / 32) {
-                uint32_t* row = reinterpret_cast<uint32_t*>(S->qcnt + r * H2_COLS);
-                unsigned e = 0, o = 0;
-#pragma unroll
-                for (int j = 0; j < H2_COLS / 128; j++) {
-                    const unsigned x = row[lane + 32 * j];
-                    row[lane + 32 * j] = 0;
-                    e += x & 0x00FF00FFu; o += (x >> 8) & 0x00FF00FFu;
-                }
-                unsigned tot = (e & 0xFFFFu) + (e >> 16) + (o & 0xFFFFu) + (o >> 16);
-                tot = __reduce_add_sync(0xffffffffu, tot);
-                if (lane == 0) S->C.hist_q[r] += tot;
-            }
-            qsym = 0;
-            h2_dna_flush_warp(&S->C, A, H, lane);
-            __syncthreads();
-            if (S->C.dirty) {                                                   // uniform: written before the barrier above
-                if (wid == 0) {
-                    unsigned best[4] = {0, 0, 0, 0};
-#pragma unroll
-                    for (unsigned j = 0; j < 8; j++) {
-                        const unsigned b = lane + 32u * j;
-                        if (S->C.state[b] == 256) {
-                            const unsigned cnt = S->C.hist_b[b] < 0xFFFFFFu ? S->C.hist_b[b] : 0xFFFFFFu;
-                            const unsigned key = ((cnt + 1u) << 8) | b;
-                            const unsigned c = (b >> 1) & 3u;
-#pragma unroll
-                            for (unsigned cc = 0; cc < 4; cc++) if (c == cc && key > best[cc]) best[cc] = key;
-                        }
-                    }
-                    unsigned h = 0;
-#pragma unroll
-                    for (unsigned c = 0; c < 4; c++) {
-                        const unsigned m = __reduce_max_sync(0xffffffffu, best[c]);
-                        h |= (m ? (m & 255u) : ((H2_NOHINT >> (8 * c)) & 255u)) << (8 * c);
-                    }
-                    if (lane == 0) { S->C.hints = h; S->C.dirty = 0; }
-                }
-                __syncthreads();
-            }
-            H = S->C.hints;
-        }
-    }
-    // ---- final flush ----
-    if (tid < TL_R) {
-#pragma unroll
-        for (int o = 16; o > 0; o >>= 1) {
-            const unsigned long long a = __shfl_xor_sync(0xffffffffu, len_min, o), b = __shfl_xor_sync(0xffffffffu, len_max, o);
-            const long long e = __shfl_xor_sync(0xffffffffu, bad_plus, o), f = __shfl_xor_sync(0xffffffffu, bad_len, o);
-            len_min = a < len_min ? a : len_min; len_max = b > len_max ? b : len_max;
-            bad_plus = e < bad_plus ? e : bad_plus; bad_len = f < bad_len ? f : bad_len;
-        }
-        if (lane == 0) {
-            if (len_min != ~0ull) atomicMin(&s->dna_min, len_min);
-            atomicMax(&s->dna_max, len_max);
-            if (bad_plus != LLONG_MAX) atomicMin(&s->bad_plus, bad_plus);
-            if (bad_len != LLONG_MAX) atomicMin(&s->bad_len, bad_len);
-        }
-    }
-    __syncthreads();
-    if (isq) h2_qual_flush(&S->C, qcol);
-    h2_dna_flush_warp(&S->C, A, H, lane);
-    __syncthreads();
-    if (tid < 256) {
-        if (S->C.hist_b[tid]) atomicAdd(&s->base_count[tid], (unsigned long long)S->C.hist_b[tid]);
-        if (tid < H2_ROWS - 1 && S->C.hist_q[tid]) atomicAdd(&s->qual_count[tid + H2_QLO], (unsigned long long)S->C.hist_q[tid]);
-        if (tid == 0 && S->C.oor) atomicOr(fallback, 1u);
-        const int f = S->C.state[tid];
-        if (f >= 0) {
-            if (f == 256) {
-                s->multi[tid] = 1;
-                atomicCAS(&s->first_q[tid], -1, 0);                 // mark the base as present
-            } else {
-                const int old = atomicCAS(&s->first_q[tid], -1, f);
-                if (old >= 0 && old != f) s->multi[tid] = 1;
-            }
-        }
-    }
-}
-
-// ---- the same counting behind a three-stage, barrier-free tile pipeline ----------------------------------
-// k_pair_hist_units synchronises the whole CTA at the end of every tile (2 us of work): the warps that own the short
-// last units wait for the others, every thread pays the line-offset conversion of the next tile, and the vote for the
-// counter flush rides on that barrier.  Here the tiles flow through THREE buffers guarded by mbarriers:
+// ---- three-stage, barrier-free tile pipeline ----------------------------------------------------------------
+// A barrier of the whole CTA at the end of every tile (2 us of work) would make the warps that own the short last units
+// wait for the others and every thread pay the line-offset conversion of the next tile.  Instead the tiles flow through
+// THREE buffers guarded by mbarriers:
 //   full[s]    32 arrivals + the transaction count of the TMA bulk copy of the tile's bytes: every warp has converted its 17
 //              of the tile's 513 line offsets (their low 32 bits are enough inside a tile), warp 31 has issued the copy;
 //   empty[s]   32 arrivals: every warp is done with the tile that used the buffer.

@@ -6,9 +6,9 @@
 //   k_pp_count   destination of every row (from the round-0 sort keys the packer wrote, or from the row) + per-tile counts
 //   k_pp_scan    per destination: exclusive scan of the tile counts, totals
 //   k_pp_pos     pos[i] = index of row i in the destination-grouped, stable order (first[d] + rows of d before i)
-//   k_scatter_rows_by_pos / k_scatter_u32_by_pos   row i -> byte offset seg_off[d] + (pos[i] - first[d]) * width of a byte
+//   k_scatter_rows_runs / k_scatter_items_by_pos   row i -> byte offset seg_off[d] + (pos[i] - first[d]) * width of a byte
 //                buffer whose segments start at multiples of `align` bytes (what the exchange sends); the tile of rows is
-//                staged in shared memory with 16-byte loads and leaves as 32-bit words.
+//                staged in shared memory with 16-byte loads and leaves in one contiguous run per destination.
 // The same pos moves every per-record payload of global_order, and brings the global ids back with a gather.
 #include "common.cuh"
 #include <cstdlib>
@@ -156,62 +156,13 @@ __device__ __forceinline__ uint32_t pp_seg_of(const pp_segs& S, uint64_t j) {
     return d;
 }
 
-// SUB lanes move one row (32 / SUB rows per warp step): 8 lanes for rows of up to 32 bytes, 16 up to 64, 32 beyond
-template <int SUB>
-__global__ void __launch_bounds__(SR_THREADS) k_scatter_rows_by_pos(const uint8_t* __restrict__ rows, uint64_t n, uint32_t width,
-                                                                   const uint32_t* __restrict__ pos, pp_segs segs, uint8_t* __restrict__ out) {
-    extern __shared__ __align__(16) uint8_t sr_stage[];                 // SR_THREADS * width + 32 bytes
-    __shared__ uint64_t dsts[SR_THREADS];
-    constexpr uint32_t NP = 32u / SUB;
-    const unsigned tid = threadIdx.x, lane = tid & 31u, w = tid >> 5;
-    const unsigned sg = lane / SUB, sl = lane % SUB;
-    const uint32_t* stage32 = reinterpret_cast<const uint32_t*>(sr_stage);
-    const uint64_t ntiles = (n + SR_THREADS - 1) / SR_THREADS;
-    for (uint64_t t = blockIdx.x; t < ntiles; t += gridDim.x) {
-        const uint64_t r0 = t * SR_THREADS;
-        const uint32_t nr = (uint32_t)(n - r0 < SR_THREADS ? n - r0 : SR_THREADS);
-        __syncthreads();
-        // the tile's rows are one contiguous, 16-byte aligned range (the last unit may reach into the table's slack)
-        const uint4* src = reinterpret_cast<const uint4*>(rows + r0 * width);
-        const uint32_t nvec = (nr * width + 15u) / 16u;
-        uint64_t j = 0;
-        if (tid < nr) j = __ldg(pos + r0 + tid);
-#pragma unroll 4
-        for (uint32_t v = tid; v < nvec; v += SR_THREADS) reinterpret_cast<uint4*>(sr_stage)[v] = __ldg(src + v);
-        if (tid < nr) {
-            const uint32_t d = pp_seg_of(segs, j);
-            dsts[tid] = segs.off[d] + (j - segs.first[d]) * width;
-        }
-        __syncthreads();
-        // warp w moves rows 32 w .. 32 w + 31, NP rows per step
-#pragma unroll 2
-        for (uint32_t k = 0; k < 32; k += NP) {
-            const uint32_t r = w * 32 + k + sg;
-            if (r < nr) {
-                uint8_t* D = out + dsts[r];
-                const uint32_t so = r * width;
-                uint32_t head = (4u - ((uint32_t)(uintptr_t)D & 3u)) & 3u;
-                head = head < width ? head : width;
-                if (sl < head) D[sl] = sr_stage[so + sl];
-                const uint32_t nwords = (width - head) >> 2;
-                uint32_t* Dw = reinterpret_cast<uint32_t*>(D + head);
-                for (uint32_t q = sl; q < nwords; q += SUB) {
-                    const uint32_t b = so + head + 4u * q;
-                    Dw[q] = __funnelshift_r(stage32[b >> 2], stage32[(b >> 2) + 1], (b & 3u) * 8u);
-                }
-                const uint32_t fin = head + 4u * nwords;
-                if (sl < width - fin) D[fin + sl] = sr_stage[so + fin + sl];
-            }
-        }
-    }
-}
-
-// The same move with CONTIGUOUS RUNS on the output side.  The rows of one tile that go to destination d are consecutive in
+// Rows -> place with CONTIGUOUS RUNS on the output side.  The rows of one tile that go to destination d are consecutive in
 // d's stream (pos is stable), so the CTA first regroups the tile by destination inside shared memory - the run of d starts
 // at an image offset with the same 16-byte phase as its global address - and then writes every run with aligned 16-byte
-// stores (only the first / last few bytes of a run go one by one).  The row-at-a-time kernel above writes 113-byte rows as
-// unaligned 4-byte words: fine for local memory, but over NVLink (peer windows) that is a packet per sector - measured 240
-// GB/s against 770 GB/s for large aligned stores.
+// stores (only the first / last few bytes of a run go one by one).  Rows written one at a time leave as unaligned 4-byte
+// words: fine for local memory, but over NVLink (peer windows) that is a packet per sector - measured 240 GB/s against
+// 770 GB/s for large aligned stores.  SUB lanes move one row into the image (32 / SUB rows per warp step): 8 lanes for
+// rows of up to 32 bytes, 16 up to 64, 32 beyond.
 #define SRR_MAXD 64
 // TMA = true: the 16-byte aligned interior of every run leaves shared memory as ONE bulk store (cp.async.bulk.global.shared,
 // issued by the thread that owns the destination); the TMA unit does the address generation and keeps more bytes in flight
@@ -343,57 +294,36 @@ static int scatter_rows_impl(uqb_ctx* ctx, const uqb_array* table, const uqb_arr
     } else if (w == 1) {
         UQB_LAUNCH_B(ab, k_scatter_items_by_pos<uint8_t>, uqb_grid(ctx, n, SR_THREADS, iw), SR_THREADS, 0, (const uint8_t*)table->d, n, (const uint32_t*)pos->d, S, o);
     } else {
-        static const bool by_rows = [] { const char* e = getenv("UQB_SCATTER_ROWS"); return e && e[0] == '1'; }();
         static const bool tma = [] { const char* e = getenv("UQB_SCATTER_TMA"); return e && e[0] == '1'; }();
-        if (!by_rows) {
-            // contiguous runs per destination, regrouped in shared memory
-            const size_t in_bytes = ((size_t)SR_THREADS * w + 32 + 15) & ~(size_t)15;
-            const size_t smem = in_bytes + (size_t)SR_THREADS * w + 32 * (size_t)S.n + 64;
-            const unsigned per_sm = (unsigned)(200 * 1024 / (smem + 5 * 1024)) ? (unsigned)(200 * 1024 / (smem + 5 * 1024)) : 1u;
-            unsigned ctas = per_sm > 8 ? 8 : per_sm;
-            if (ctx->side_ctas_per_sm && ctas > ctx->side_ctas_per_sm) ctas = ctx->side_ctas_per_sm;
-            const uint64_t ntiles = (n + SR_THREADS - 1) / SR_THREADS, cap = (uint64_t)ctx->sm_count * ctas;
-            const unsigned grid = (unsigned)(ntiles < cap ? ntiles : cap);
-            if (w <= 32) {
-                auto k_scatter_rows_runs_8 = k_scatter_rows_runs<8, false>;
-                auto k_scatter_rows_tma_8 = k_scatter_rows_runs<8, true>;
-                UQB_CUDA(cudaFuncSetAttribute(k_scatter_rows_runs_8, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-                UQB_CUDA(cudaFuncSetAttribute(k_scatter_rows_tma_8, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-                if (tma) UQB_LAUNCH_B(ab, k_scatter_rows_tma_8, grid, SR_THREADS, smem, (const uint8_t*)table->d, n, w, (const uint32_t*)pos->d, S, o);
-                else UQB_LAUNCH_B(ab, k_scatter_rows_runs_8, grid, SR_THREADS, smem, (const uint8_t*)table->d, n, w, (const uint32_t*)pos->d, S, o);
-            } else if (w <= 64) {
-                auto k_scatter_rows_runs_16 = k_scatter_rows_runs<16, false>;
-                auto k_scatter_rows_tma_16 = k_scatter_rows_runs<16, true>;
-                UQB_CUDA(cudaFuncSetAttribute(k_scatter_rows_runs_16, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-                UQB_CUDA(cudaFuncSetAttribute(k_scatter_rows_tma_16, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-                if (tma) UQB_LAUNCH_B(ab, k_scatter_rows_tma_16, grid, SR_THREADS, smem, (const uint8_t*)table->d, n, w, (const uint32_t*)pos->d, S, o);
-                else UQB_LAUNCH_B(ab, k_scatter_rows_runs_16, grid, SR_THREADS, smem, (const uint8_t*)table->d, n, w, (const uint32_t*)pos->d, S, o);
-            } else {
-                auto k_scatter_rows_runs_32 = k_scatter_rows_runs<32, false>;
-                auto k_scatter_rows_tma_32 = k_scatter_rows_runs<32, true>;
-                UQB_CUDA(cudaFuncSetAttribute(k_scatter_rows_runs_32, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-                UQB_CUDA(cudaFuncSetAttribute(k_scatter_rows_tma_32, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-                if (tma) UQB_LAUNCH_B(ab, k_scatter_rows_tma_32, grid, SR_THREADS, smem, (const uint8_t*)table->d, n, w, (const uint32_t*)pos->d, S, o);
-                else UQB_LAUNCH_B(ab, k_scatter_rows_runs_32, grid, SR_THREADS, smem, (const uint8_t*)table->d, n, w, (const uint32_t*)pos->d, S, o);
-            }
-            return 0;
-        }
-        const size_t smem = (size_t)SR_THREADS * w + 32;
-        const unsigned per_sm = (unsigned)(200 * 1024 / (smem + 3 * 1024)) ? (unsigned)(200 * 1024 / (smem + 3 * 1024)) : 1u;
-        const uint64_t ntiles = (n + SR_THREADS - 1) / SR_THREADS, cap = (uint64_t)ctx->sm_count * (per_sm > 8 ? 8 : per_sm);
+        // contiguous runs per destination, regrouped in shared memory
+        const size_t in_bytes = ((size_t)SR_THREADS * w + 32 + 15) & ~(size_t)15;
+        const size_t smem = in_bytes + (size_t)SR_THREADS * w + 32 * (size_t)S.n + 64;
+        const unsigned per_sm = (unsigned)(200 * 1024 / (smem + 5 * 1024)) ? (unsigned)(200 * 1024 / (smem + 5 * 1024)) : 1u;
+        unsigned ctas = per_sm > 8 ? 8 : per_sm;
+        if (ctx->side_ctas_per_sm && ctas > ctx->side_ctas_per_sm) ctas = ctx->side_ctas_per_sm;
+        const uint64_t ntiles = (n + SR_THREADS - 1) / SR_THREADS, cap = (uint64_t)ctx->sm_count * ctas;
         const unsigned grid = (unsigned)(ntiles < cap ? ntiles : cap);
         if (w <= 32) {
-            auto k_scatter_rows_by_pos_8 = k_scatter_rows_by_pos<8>;
-            UQB_CUDA(cudaFuncSetAttribute(k_scatter_rows_by_pos_8, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-            UQB_LAUNCH_B(ab, k_scatter_rows_by_pos_8, grid, SR_THREADS, smem, (const uint8_t*)table->d, n, w, (const uint32_t*)pos->d, S, o);
+            auto k_scatter_rows_runs_8 = k_scatter_rows_runs<8, false>;
+            auto k_scatter_rows_tma_8 = k_scatter_rows_runs<8, true>;
+            UQB_CUDA(cudaFuncSetAttribute(k_scatter_rows_runs_8, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+            UQB_CUDA(cudaFuncSetAttribute(k_scatter_rows_tma_8, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+            if (tma) UQB_LAUNCH_B(ab, k_scatter_rows_tma_8, grid, SR_THREADS, smem, (const uint8_t*)table->d, n, w, (const uint32_t*)pos->d, S, o);
+            else UQB_LAUNCH_B(ab, k_scatter_rows_runs_8, grid, SR_THREADS, smem, (const uint8_t*)table->d, n, w, (const uint32_t*)pos->d, S, o);
         } else if (w <= 64) {
-            auto k_scatter_rows_by_pos_16 = k_scatter_rows_by_pos<16>;
-            UQB_CUDA(cudaFuncSetAttribute(k_scatter_rows_by_pos_16, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-            UQB_LAUNCH_B(ab, k_scatter_rows_by_pos_16, grid, SR_THREADS, smem, (const uint8_t*)table->d, n, w, (const uint32_t*)pos->d, S, o);
+            auto k_scatter_rows_runs_16 = k_scatter_rows_runs<16, false>;
+            auto k_scatter_rows_tma_16 = k_scatter_rows_runs<16, true>;
+            UQB_CUDA(cudaFuncSetAttribute(k_scatter_rows_runs_16, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+            UQB_CUDA(cudaFuncSetAttribute(k_scatter_rows_tma_16, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+            if (tma) UQB_LAUNCH_B(ab, k_scatter_rows_tma_16, grid, SR_THREADS, smem, (const uint8_t*)table->d, n, w, (const uint32_t*)pos->d, S, o);
+            else UQB_LAUNCH_B(ab, k_scatter_rows_runs_16, grid, SR_THREADS, smem, (const uint8_t*)table->d, n, w, (const uint32_t*)pos->d, S, o);
         } else {
-            auto k_scatter_rows_by_pos_32 = k_scatter_rows_by_pos<32>;
-            UQB_CUDA(cudaFuncSetAttribute(k_scatter_rows_by_pos_32, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-            UQB_LAUNCH_B(ab, k_scatter_rows_by_pos_32, grid, SR_THREADS, smem, (const uint8_t*)table->d, n, w, (const uint32_t*)pos->d, S, o);
+            auto k_scatter_rows_runs_32 = k_scatter_rows_runs<32, false>;
+            auto k_scatter_rows_tma_32 = k_scatter_rows_runs<32, true>;
+            UQB_CUDA(cudaFuncSetAttribute(k_scatter_rows_runs_32, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+            UQB_CUDA(cudaFuncSetAttribute(k_scatter_rows_tma_32, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+            if (tma) UQB_LAUNCH_B(ab, k_scatter_rows_tma_32, grid, SR_THREADS, smem, (const uint8_t*)table->d, n, w, (const uint32_t*)pos->d, S, o);
+            else UQB_LAUNCH_B(ab, k_scatter_rows_runs_32, grid, SR_THREADS, smem, (const uint8_t*)table->d, n, w, (const uint32_t*)pos->d, S, o);
         }
     }
     return 0;

@@ -477,8 +477,7 @@ __global__ void __launch_bounds__(256) k_pairs_apply(const uint32_t* __restrict_
 // out[idx[p]] = val[p]; idx must be a permutation of 0..n-1 (n < 2^32).  Small arrays are scattered directly.
 int uqb_scatter_pairs_u32(uqb_ctx* ctx, const uint32_t* idx, const uint32_t* val, uint64_t n, uint32_t* out) {
     if (n == 0) return 0;
-    static const uint32_t wshift0 = [] { const char* e = getenv("UQB_PAIR_WSHIFT"); return e ? (uint32_t)atoi(e) : 23u; }();
-    uint32_t wshift = wshift0;                                     // 2^23 entries = 32 MB of `out` per window
+    uint32_t wshift = 23;                                          // 2^23 entries = 32 MB of `out` per window
     while (((n + (1ull << wshift) - 1) >> wshift) > 256) wshift++;
     const uint32_t nwin = (uint32_t)((n + (1ull << wshift) - 1) >> wshift);
     const uint32_t nblk = (uint32_t)((n + PR_TILE - 1) / PR_TILE);
@@ -496,178 +495,6 @@ int uqb_scatter_pairs_u32(uqb_ctx* ctx, const uint32_t* idx, const uint32_t* val
     UQB_TRY(uqb_dfree(ctx, idx2, 0));
     UQB_TRY(uqb_dfree(ctx, val2, 0));
     return 0;
-}
-
-// ---- one sweep per digit -------------------------------------------------------------------------
-// The three-kernel pass above reads the keys twice (histogram, scatter) and runs a 3-launch scan over 256 x tiles
-// counters in between.  k_radix_onesweep does a whole pass in one launch (Adinets & Merrill's Onesweep):
-//   * tiles are taken in ticket order; the CTA ranks its tile exactly like k_radix_scatter;
-//   * the first global slot of digit d for this tile = (number of keys with a smaller digit: an exclusive scan of the GLOBAL
-//     digit histogram, 256 counters) + (keys with digit d in earlier tiles: a decoupled look-back over one 32-bit status
-//     word per (tile, digit): flag 1 = the tile's own count, flag 2 = inclusive count of all tiles up to it);
-//   * while the keys are in registers the CTA also counts the NEXT pass's digit and adds it to that pass's global
-//     histogram, so only the first pass of a sort needs a histogram kernel of its own.
-// Keys are read once per pass, nothing is scanned between passes, and a sort of P digits is P + 1 launches.
-struct os_stage {
-    uint32_t whist[RS_WARPS][256];
-    uint32_t dstart[256];
-    uint32_t gbase[256];
-    uint32_t nhist[256];
-    uint32_t wtot[8], gtot[8];
-    uint32_t tile, pad_;
-    uint64_t key[PR_TILE];
-    uint32_t val[PR_TILE];
-};
-
-#define OS_FLAG_AGG 0x40000000u
-#define OS_FLAG_INC 0x80000000u
-#define OS_COUNT 0x3FFFFFFFu
-
-__device__ __forceinline__ uint32_t os_ld(const uint32_t* p) {
-    uint32_t v;
-    asm volatile("ld.volatile.global.u32 %0, [%1];" : "=r"(v) : "l"(p) : "memory");
-    return v;
-}
-__device__ __forceinline__ void os_st(uint32_t* p, uint32_t v) {
-    asm volatile("st.volatile.global.u32 [%0], %1;" ::"l"(p), "r"(v) : "memory");
-}
-
-// global histogram of one digit (first pass of a sort): one shared-memory histogram per CTA over a grid-stride range
-__global__ void __launch_bounds__(PR_THREADS) k_radix_hist_global(const uint64_t* __restrict__ key, uint64_t n, int shift, uint32_t* __restrict__ ghist) {
-    __shared__ uint32_t hist[256];
-    hist[threadIdx.x] = 0;
-    __syncthreads();
-    for (uint64_t i = (uint64_t)blockIdx.x * PR_THREADS + threadIdx.x; i < n; i += (uint64_t)gridDim.x * PR_THREADS)
-        atomicAdd(&hist[(uint32_t)((__ldg(key + i) >> shift) & 255ull)], 1u);
-    __syncthreads();
-    if (hist[threadIdx.x]) atomicAdd(&ghist[threadIdx.x], hist[threadIdx.x]);
-}
-
-__global__ void __launch_bounds__(RS_THREADS, 2) k_radix_onesweep(const uint64_t* __restrict__ kin, const uint32_t* __restrict__ vin,
-                                                                 uint64_t* __restrict__ kout, uint32_t* __restrict__ vout, uint64_t n,
-                                                                 int shift, int next_shift, const uint32_t* __restrict__ ghist,
-                                                                 uint32_t* __restrict__ ghist_next, uint32_t* __restrict__ status,
-                                                                 unsigned int* __restrict__ ticket) {
-    extern __shared__ __align__(16) uint8_t os_raw[];
-    os_stage* S = reinterpret_cast<os_stage*>(os_raw);
-    const unsigned tid = threadIdx.x, w = tid >> 5, lane = tid & 31u;
-    if (tid == 0) S->tile = atomicAdd(ticket, 1u);
-    for (unsigned i = tid; i < RS_WARPS * 256; i += RS_THREADS) (&S->whist[0][0])[i] = 0;
-    if (tid < 256) S->nhist[tid] = 0;
-    __syncthreads();
-    const uint32_t tile = S->tile;
-    const uint64_t tile0 = (uint64_t)tile * PR_TILE;
-    const uint64_t warp0 = tile0 + (uint64_t)w * (32 * RS_ITEMS);
-    const uint32_t ntile = (uint32_t)((n - tile0 < PR_TILE) ? (n - tile0) : PR_TILE);
-    uint64_t key[RS_ITEMS];
-    uint32_t val[RS_ITEMS];
-#pragma unroll
-    for (int j = 0; j < RS_ITEMS; j++) {
-        const uint64_t idx = warp0 + (uint64_t)j * 32 + lane;
-        key[j] = 0; val[j] = 0;
-        if (idx < n) {
-            key[j] = kin[idx];
-            val[j] = vin ? vin[idx] : (uint32_t)idx;
-        }
-    }
-    uint32_t rk[RS_ITEMS];
-#pragma unroll
-    for (int j = 0; j < RS_ITEMS; j++) {
-        const uint64_t idx = warp0 + (uint64_t)j * 32 + lane;
-        const bool valid = idx < n;
-        uint32_t d = 256u;
-        if (valid) d = (uint32_t)((key[j] >> shift) & 255ull);
-        const unsigned m = __match_any_sync(0xffffffffu, d);
-        const unsigned r = __popc(m & ((1u << lane) - 1u));
-        const int leader = __ffs(m) - 1;
-        uint32_t old = 0;
-        if (valid && (int)lane == leader) {
-            old = S->whist[w][d];
-            S->whist[w][d] = old + __popc(m);
-        }
-        old = __shfl_sync(0xffffffffu, old, leader);
-        rk[j] = (d << 16) | (old + r);
-        if (next_shift >= 0 && valid) atomicAdd(&S->nhist[(uint32_t)((key[j] >> next_shift) & 255ull)], 1u);
-        __syncwarp();
-    }
-    __syncthreads();
-    uint32_t tot = 0, incl = 0;
-    if (tid < 256) {
-#pragma unroll
-        for (int w2 = 0; w2 < RS_WARPS; w2++) {
-            const uint32_t c = S->whist[w2][tid];
-            S->whist[w2][tid] = tot;
-            tot += c;
-        }
-        // publish this tile's count of digit `tid` before anything else: later tiles are waiting for it
-        uint32_t* st = status + (uint64_t)tile * 256 + tid;
-        __threadfence();
-        os_st(st, (tile == 0 ? OS_FLAG_INC : OS_FLAG_AGG) | tot);
-        incl = tot;
-#pragma unroll
-        for (int o = 1; o < 32; o <<= 1) {
-            const uint32_t t = __shfl_up_sync(0xffffffffu, incl, o);
-            if (lane >= (unsigned)o) incl += t;
-        }
-        if (lane == 31) S->wtot[w] = incl;
-        if (next_shift >= 0 && S->nhist[tid]) atomicAdd(&ghist_next[tid], S->nhist[tid]);
-    }
-    __syncthreads();
-    if (tid < 256) {
-        uint32_t wb = 0;
-#pragma unroll
-        for (int i = 0; i < 8; i++) if ((unsigned)i < w) wb += S->wtot[i];
-        const uint32_t start = wb + incl - tot;
-        S->dstart[tid] = start;
-        // keys with a smaller digit anywhere: exclusive scan of the global histogram (256 values, the same shuffle scan)
-        const uint32_t gh = __ldg(ghist + tid);
-        uint32_t gin = gh;
-#pragma unroll
-        for (int o = 1; o < 32; o <<= 1) {
-            const uint32_t t = __shfl_up_sync(0xffffffffu, gin, o);
-            if (lane >= (unsigned)o) gin += t;
-        }
-        if (lane == 31) S->gtot[w] = gin;
-        asm volatile("bar.sync 1, 256;" ::: "memory");     // warps 0..7 only
-        uint32_t gb = 0;
-#pragma unroll
-        for (int i = 0; i < 8; i++) if ((unsigned)i < w) gb += S->gtot[i];
-        const uint32_t gexcl = gb + gin - gh;
-        // keys with this digit in earlier tiles: look back
-        uint32_t before = 0;
-        if (tile) {
-            uint32_t j = tile - 1;
-            while (true) {
-                uint32_t v = os_ld(status + (uint64_t)j * 256 + tid);
-                while ((v & (OS_FLAG_AGG | OS_FLAG_INC)) == 0) { __nanosleep(32); v = os_ld(status + (uint64_t)j * 256 + tid); }
-                before += v & OS_COUNT;
-                if ((v & OS_FLAG_INC) || j == 0) break;
-                j--;
-            }
-            __threadfence();
-            os_st(status + (uint64_t)tile * 256 + tid, OS_FLAG_INC | (before + tot));
-        }
-        S->gbase[tid] = gexcl + before - start;
-    }
-    __syncthreads();
-#pragma unroll
-    for (int j = 0; j < RS_ITEMS; j++) {
-        const uint64_t idx = warp0 + (uint64_t)j * 32 + lane;
-        if (idx < n) {
-            const uint32_t d = rk[j] >> 16;
-            const uint32_t slot = S->dstart[d] + S->whist[w][d] + (rk[j] & 0xffffu);
-            S->key[slot] = key[j];
-            S->val[slot] = val[j];
-        }
-    }
-    __syncthreads();
-    for (uint32_t i = tid; i < ntile; i += RS_THREADS) {
-        const uint64_t k = S->key[i];
-        const uint32_t d = (uint32_t)((k >> shift) & 255ull);
-        const uint32_t pos = S->gbase[d] + i;
-        kout[pos] = k;
-        vout[pos] = S->val[i];
-    }
 }
 
 int uqb_sortbuf_alloc(uqb_ctx* ctx, uqb_sortbuf* sb, uint64_t n, bool with_aux) {
@@ -979,36 +806,6 @@ int uqb_radix_sort(uqb_ctx* ctx, uqb_sortbuf* sb, uint64_t n, bool use_aux, cons
     const bool has_aux = sb->aux[0] != nullptr;
     if (!use_aux && !has_aux && n >= MSD_MIN_N && nk >= 3) return msd_sort(ctx, sb, n, key_first, got.or64 ^ got.and64);
     uint32_t nblk = (uint32_t)((n + PR_TILE - 1) / PR_TILE);
-    // Opt-in (UQB_RADIX_ONESWEEP=1): measured on B200 at 100 M keys it is SLOWER than the three kernels below (0.78 ms per
-    // pass against 0.45 + 0.13 + 0.06 ms): a tile lasts ~5 us and a new one starts every ~18 ns, so the one-status-word-per-
-    // thread look-back (one L2 round trip per predecessor) cannot keep up with the tiles; a 32-wide window per digit would
-    // read 32 KB of status words per 48 KB tile.  Kept for the record and for the parity tests that run it.
-    static const bool one_sweep = [] { const char* e = getenv("UQB_RADIX_ONESWEEP"); return e && e[0] == '1'; }();
-    if (!use_aux && sb->aux[0] == nullptr && n < (1ull << 30) && one_sweep) {
-        // one sweep per digit: [nk] global histograms, [nk] tickets, [nk][tiles][256] status words, zeroed once
-        const uint64_t words = (uint64_t)nk * 256 + 64 + (uint64_t)nk * nblk * 256;
-        uint32_t* ws;
-        UQB_TRY(uqb_dalloc_t(ctx, &ws, words));
-        UQB_CUDA(cudaMemsetAsync(ws, 0, words * 4, ctx->stream));
-        uint32_t* gh = ws;
-        unsigned int* tickets = ws + (uint64_t)nk * 256;
-        uint32_t* status = ws + (uint64_t)nk * 256 + 64;
-        const uint64_t* k0 = key_first ? key_first : sb->key[sb->cur];
-        UQB_LAUNCH_B(n * 8, k_radix_hist_global, uqb_grid(ctx, n, PR_THREADS * 16, 8), PR_THREADS, 0, k0, n, kshift[0], gh);
-        const size_t os_smem = sizeof(os_stage);
-        UQB_CUDA(cudaFuncSetAttribute(k_radix_onesweep, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)os_smem));
-        for (int p = 0; p < nk; p++) {
-            const int c = sb->cur, o = c ^ 1;
-            const uint64_t* kin = (p == 0 && key_first) ? key_first : sb->key[c];
-            const uint32_t* vin = (p == 0 && key_first) ? nullptr : sb->val[c];
-            UQB_LAUNCH_B(n * 24, k_radix_onesweep, nblk, RS_THREADS, os_smem, kin, vin, sb->key[o], sb->val[o], n, kshift[p],
-                         p + 1 < nk ? kshift[p + 1] : -1, gh + 256 * p, gh + 256 * (p + 1 < nk ? p + 1 : p),
-                         status + (uint64_t)p * nblk * 256, tickets + p);
-            sb->cur = o;
-        }
-        UQB_TRY(uqb_dfree(ctx, ws, words * 4));
-        return 0;
-    }
     uint32_t* ghist;
     uint64_t hist_n = (uint64_t)256 * nblk;
     UQB_TRY(uqb_dalloc_t(ctx, &ghist, hist_n));

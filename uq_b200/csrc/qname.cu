@@ -37,7 +37,7 @@ __global__ void __launch_bounds__(QN) k_qname_tokens(const uint8_t* __restrict__
                                                     const uint8_t* __restrict__ names, uint32_t name_pitch) {
     const uint64_t r = (uint64_t)blockIdx.x * QN + threadIdx.x;
     if (r >= n_reads) return;
-    // names != nullptr: QNAME lines from the compact side array of sweep A (row r: length byte + text)
+    // names != nullptr: QNAME lines from the compact side array (uqb_fastq::names, row r: length byte + text)
     uint64_t n;
     const uint8_t* name;
     if (names) {

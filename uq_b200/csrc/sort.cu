@@ -807,27 +807,6 @@ __global__ void __launch_bounds__(ST) k_scatter_key(const uint32_t* __restrict__
     key[perm[p]] = gid[p];
 }
 
-// The same scatter for arrays much larger than the L2: the destination is taken in windows of 2^wshift entries, one window
-// per sweep over perm, so that the 4-byte stores of a window meet in the L2 and leave as full sectors (a plain random
-// scatter over 400 MB costs a sector fill and a write-back per element).  perm is read once per window (sequential).
-__global__ void __launch_bounds__(ST) k_scatter_key_windows(const uint32_t* __restrict__ perm, const uint32_t* __restrict__ gid, uint64_t n,
-                                                           uint32_t wshift, uint32_t nwin, uint32_t* __restrict__ key) {
-    const uint64_t stride = (uint64_t)gridDim.x * ST * 4;
-    for (uint32_t w = 0; w < nwin; w++) {
-        for (uint64_t p0 = ((uint64_t)blockIdx.x * ST + threadIdx.x) * 4; p0 < n; p0 += stride) {
-            if (p0 + 4 <= n) {
-                const uint4 d = __ldg(reinterpret_cast<const uint4*>(perm + p0));
-                if ((d.x >> wshift) == w) key[d.x] = __ldg(gid + p0);
-                if ((d.y >> wshift) == w) key[d.y] = __ldg(gid + p0 + 1);
-                if ((d.z >> wshift) == w) key[d.z] = __ldg(gid + p0 + 2);
-                if ((d.w >> wshift) == w) key[d.w] = __ldg(gid + p0 + 3);
-            } else {
-                for (uint64_t p = p0; p < n; p++) { const uint32_t d = perm[p]; if ((d >> wshift) == w) key[d] = gid[p]; }
-            }
-        }
-    }
-}
-
 // key[perm[p]] = gid[p] for all p
 static int scatter_key(uqb_ctx* ctx, const uint32_t* perm, const uint32_t* gid, uint64_t n, uint32_t* key) {
     if (n == 0) return 0;
@@ -836,11 +815,7 @@ static int scatter_key(uqb_ctx* ctx, const uint32_t* perm, const uint32_t* gid, 
         UQB_LAUNCH_B(n * 12, k_scatter_key, uqb_blocks(n, ST), ST, 0, perm, gid, n, key);
         return 0;
     }
-    static const bool sweeps = [] { const char* e = getenv("UQB_SCATTER_SWEEPS"); return e && e[0] == '1'; }();
-    if (!sweeps) return uqb_scatter_pairs_u32(ctx, perm, gid, n, key);      // regrouped by window first: 3 sweeps instead of one per window
-    const uint32_t nwin = (uint32_t)((n + (1ull << wshift) - 1) >> wshift);
-    UQB_LAUNCH_B(n * 12, k_scatter_key_windows, uqb_grid(ctx, n, ST * 4, 4), ST, 0, perm, gid, n, wshift, nwin, key);
-    return 0;
+    return uqb_scatter_pairs_u32(ctx, perm, gid, n, key);          // regrouped by window first: 3 sweeps instead of one per window
 }
 
 __global__ void __launch_bounds__(ST) k_first_of_group(const uint32_t* __restrict__ perm, const uint32_t* __restrict__ gid, uint64_t n,

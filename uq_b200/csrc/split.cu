@@ -318,7 +318,7 @@ int uqb_fastq_free_qcols(uqb_ctx* ctx, uqb_fastq* fq) { return free_qcols(ctx, f
 extern "C" int uqb_fastq_free(uqb_ctx* ctx, uqb_fastq* fq) {
     if (!fq) return 0;
     UQB_TRY(free_qcols(ctx, fq));
-    UQB_TRY(uqb_scan_release(ctx, fq));
+    UQB_TRY(uqb_names_release(ctx, fq));
     if (fq->line_off) UQB_TRY(uqb_dfree(ctx, fq->line_off, (fq->n_lines + 1) * 8));
     delete fq->cached_stats;
     if (fq->ref_name) UQB_TRY(uqb_dfree(ctx, fq->ref_name, 0));
@@ -358,21 +358,10 @@ extern "C" int uqb_split(uqb_ctx* ctx, uqb_fastq* fq, uqb_split_info* info) {
     }
     info->n_bytes = fq->n;
     if (fq->line_off) { UQB_TRY(uqb_dfree(ctx, fq->line_off, (fq->n_lines + 1) * 8)); fq->line_off = nullptr; }
-    UQB_TRY(uqb_scan_release(ctx, fq));
-    {   // sweep A: newline scan, line offsets, record checks, histograms and the compact QNAME array in ONE pass
-        bool done = false;
-        UQB_TRY(uqb_scan_file(ctx, fq, &done));
-        if (done) {
-            info->n_lines = fq->n_lines;
-            info->n_reads = fq->n_reads;
-            info->status = (fq->n_lines % 4 == 0) ? 0 : 1;
-            return 0;
-        }
-    }
+    UQB_TRY(uqb_names_release(ctx, fq));
     uint64_t ntiles = (fq->n + SP_TILE - 1) / SP_TILE;
     uint64_t total = 0;
-    static const bool two_pass = [] { const char* e = getenv("UQB_SPLIT_TWO_PASS"); return e && e[0] == '1'; }();
-    if (ntiles >= 64 && !two_pass) {
+    if (ntiles >= 64) {
         // one pass (k_newline_scan1).  line_off is sized from the newline density of the first 64 MB (or the whole file) plus 2 % and 1 M lines;
         // if the rest of the file is denser than that, the pass reports it and the two-pass path below runs instead.
         const uint64_t head_tiles = ntiles < 4096 ? ntiles : 4096;

@@ -40,6 +40,14 @@ __device__ __forceinline__ uint2 lds_u64(uint32_t a) {
     asm volatile("ld.shared.v2.u32 {%0, %1}, [%2];" : "=r"(v.x), "=r"(v.y) : "r"(a));
     return v;
 }
+__device__ __forceinline__ uint32_t lds_u8m(uint32_t a) {        // with memory clobber: the private counters are read back
+    uint32_t v;
+    asm volatile("ld.shared.u8 %0, [%1];" : "=r"(v) : "r"(a) : "memory");
+    return v;
+}
+__device__ __forceinline__ void sts_u8(uint32_t a, uint32_t v) {
+    asm volatile("st.shared.u8 [%0], %1;" ::"r"(a), "r"(v) : "memory");
+}
 __device__ __forceinline__ void sts_u32(uint32_t a, uint32_t v) {
     asm volatile("st.shared.u32 [%0], %1;" ::"r"(a), "r"(v) : "memory");
 }
@@ -103,142 +111,3 @@ __device__ __forceinline__ uint32_t tile_load(tile_smem* T, const uint8_t* __res
     __syncthreads();
     return nrec;
 }
-
-// ---- double-buffered record tiles ----------------------------------------------------------------
-// Same staging, but the bulk copy of tile k+1 runs while tile k is processed:
-//   start of tile k   thread 0 issues the copy of tile k+1 (its byte bounds were loaded one tile earlier and
-//                     wait in registers), every thread issues the loads of tile k+1's line offsets;
-//   end of tile k     the line offsets are rebased and stored (other buffer), one __syncthreads();
-//   tile k+1          its mbarrier has normally completed long ago.
-// Used by persistent CTAs that walk tiles blockIdx.x, blockIdx.x + gridDim.x, ...
-struct tile2_smem {
-    alignas(128) uint8_t bytes[2][TL_CAP + 32];
-    uint32_t loff[2][4 * TL_R + 4];
-    alignas(8) uint64_t bar[2];
-    uint32_t ok[2];                 // 0: the tile does not fit TL_CAP (nothing was copied)
-};
-
-template <int NTHREADS>
-struct tile2_pipe {
-    static constexpr int NV = (4 * TL_R + 1 + NTHREADS - 1) / NTHREADS;       // line offsets per thread
-    tile2_smem* T;
-    const uint8_t* d;
-    const uint64_t* line_off;
-    uint64_t n_bytes, r_begin, n_reads, ntiles;
-    uint64_t nb0, nb1;              // thread 0: byte bounds of the tile after the one in flight
-    uint64_t v[NV], vb0, vb1;       // line offsets of the tile in flight (held until the end of the current tile)
-    uint64_t t;                     // current tile
-    unsigned buf, phases;           // bit b of phases: mbarrier parity of the next use of buffer b
-    bool has_next;
-
-    __device__ __forceinline__ void bounds(uint64_t tile, uint64_t* b0, uint64_t* b1) const {
-        const uint64_t r0 = r_begin + tile * TL_R, r1 = (r0 + TL_R < n_reads) ? r0 + TL_R : n_reads;
-        *b0 = line_off[4 * r0]; *b1 = line_off[4 * r1];
-    }
-    __device__ __forceinline__ uint32_t nrec_of(uint64_t tile) const {
-        const uint64_t r0 = r_begin + tile * TL_R, r1 = (r0 + TL_R < n_reads) ? r0 + TL_R : n_reads;
-        return (uint32_t)(r1 - r0);
-    }
-    // thread 0: start the bulk copy of the byte range [b0, b1) into buffer bf
-    __device__ __forceinline__ void issue(unsigned bf, uint64_t b0, uint64_t b1) {
-        const uint64_t a0 = b0 & ~15ull;
-        if (b1 - a0 > TL_CAP) { T->ok[bf] = 0; return; }
-        uint64_t a1 = (b1 + 15) & ~15ull;
-        const uint64_t lim = n_bytes & ~15ull;
-        if (a1 > lim) a1 = lim;
-        if (a1 < a0) a1 = a0;
-        const uint32_t bulk = (uint32_t)(a1 - a0);
-        T->ok[bf] = 1;
-        asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-        mbar_expect_tx(&T->bar[bf], bulk);
-        if (bulk) bulk_g2s(T->bytes[bf], d + a0, bulk, &T->bar[bf]);
-    }
-    __device__ __forceinline__ void load_offsets(uint64_t tile) {
-        const uint64_t r0 = r_begin + tile * TL_R;
-        const uint32_t n = 4 * nrec_of(tile);
-        vb0 = line_off[4 * r0];
-        vb1 = line_off[4 * r0 + n];
-#pragma unroll
-        for (int k = 0; k < NV; k++) {
-            const uint32_t i = threadIdx.x + k * NTHREADS;
-            v[k] = i <= n ? line_off[4 * r0 + i] : 0;
-        }
-    }
-    __device__ __forceinline__ void store_offsets(uint64_t tile, unsigned bf) {
-        const uint32_t n = 4 * nrec_of(tile);
-        const uint64_t a0 = vb0 & ~15ull;
-#pragma unroll
-        for (int k = 0; k < NV; k++) {
-            const uint32_t i = threadIdx.x + k * NTHREADS;
-            if (i <= n) T->loff[bf][i] = (uint32_t)(v[k] - a0);
-        }
-        // tail of the stream that is not a full 16-byte unit (last tile of the buffer only)
-        const uint64_t b1 = vb1;
-        uint64_t a1 = (b1 + 15) & ~15ull;
-        const uint64_t lim = n_bytes & ~15ull;
-        if (a1 > lim) a1 = lim;
-        if (a1 < a0) a1 = a0;
-        if (b1 - a0 <= TL_CAP)
-            for (uint64_t q = a1 + threadIdx.x; q < b1; q += NTHREADS) T->bytes[bf][q - a0] = d[q];
-    }
-
-    // call with every thread of the CTA; afterwards `valid()` tells whether there is a current tile
-    __device__ __forceinline__ void begin(tile2_smem* T_, const uint8_t* d_, uint64_t n_bytes_, const uint64_t* line_off_, uint64_t r_begin_,
-                                          uint64_t n_reads_) {
-        T = T_; d = d_; n_bytes = n_bytes_; line_off = line_off_; r_begin = r_begin_; n_reads = n_reads_;
-        ntiles = (n_reads - r_begin + TL_R - 1) / TL_R;
-        t = blockIdx.x; buf = 0; phases = 0; has_next = false; nb0 = nb1 = 0;
-        if (threadIdx.x == 0) {
-            mbar_init(&T->bar[0], 1);
-            mbar_init(&T->bar[1], 1);
-            asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-        }
-        __syncthreads();
-        if (t >= ntiles) return;
-        if (threadIdx.x == 0) {
-            uint64_t b0, b1;
-            bounds(t, &b0, &b1);
-            issue(0, b0, b1);
-            if (t + gridDim.x < ntiles) bounds(t + gridDim.x, &nb0, &nb1);
-        }
-        load_offsets(t);
-        store_offsets(t, 0);
-        __syncthreads();
-    }
-    __device__ __forceinline__ bool valid() const { return t < ntiles; }
-    // start of a tile: prefetch the next one, wait for the current one.  Returns the number of records of the
-    // current tile, or 0 when it does not fit (the caller reports it and calls finish() all the same).
-    __device__ __forceinline__ uint32_t acquire() {
-        const uint64_t tn = t + gridDim.x;
-        has_next = tn < ntiles;
-        if (has_next) {
-            if (threadIdx.x == 0) {
-                issue(buf ^ 1u, nb0, nb1);
-                if (tn + gridDim.x < ntiles) bounds(tn + gridDim.x, &nb0, &nb1);
-            }
-            load_offsets(tn);
-        }
-        if (!T->ok[buf]) return 0;
-        mbar_wait(&T->bar[buf], (phases >> buf) & 1u);
-        phases ^= 1u << buf;
-        return nrec_of(t);
-    }
-    __device__ __forceinline__ const uint8_t* bytes() const { return T->bytes[buf]; }
-    __device__ __forceinline__ const uint32_t* loff() const { return T->loff[buf]; }
-    __device__ __forceinline__ uint64_t first_record() const { return r_begin + t * TL_R; }
-    // end of a tile (every thread)
-    __device__ __forceinline__ void finish() {
-        if (has_next) store_offsets(t + gridDim.x, buf ^ 1u);
-        __syncthreads();
-        t += gridDim.x;
-        buf ^= 1u;
-    }
-    // the same, and the barrier also tells every thread whether any thread raised `pred`
-    __device__ __forceinline__ bool finish_or(bool pred) {
-        if (has_next) store_offsets(t + gridDim.x, buf ^ 1u);
-        const int any = __syncthreads_or(pred ? 1 : 0);
-        t += gridDim.x;
-        buf ^= 1u;
-        return any != 0;
-    }
-};
