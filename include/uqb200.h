@@ -170,13 +170,14 @@ int uqb_qname_dict_info(uqb_ctx* ctx, uqb_fastq* fq, uint32_t col, uint64_t* cou
 int uqb_qname_dict(uqb_ctx* ctx, uqb_fastq* fq, uint32_t col, uint8_t* host, uint64_t nbytes);
 
 typedef struct {
-    uint8_t  format;     /* 0 mapping (bisect_left rank, uq.py:724), 1 integers (uq.py:725-726) */
-    uint8_t  itemsize;   /* 1, 2, 4, 8 */
+    uint8_t  format;     /* 0 mapping (bisect_left rank, uq.py:724), 1 integers (uq.py:725-726),
+                            2 strings (declared extension E1: the token's bytes, left-aligned, zero padded) */
+    uint8_t  itemsize;   /* 1, 2, 4, 8; for strings the width W (1..255): at least the longest token */
     uint8_t  offset;     /* subtract min (uq.py:725) */
     uint8_t  _pad[5];
     int64_t  min_val;
 } uqb_colspec;
-/* Pass 4 (uq.py:717-735): one little-endian array per column, width = itemsize */
+/* Pass 4 (uq.py:717-735): one little-endian array per column, width = itemsize (strings: W bytes per record) */
 int uqb_qname_encode(uqb_ctx* ctx, uqb_fastq* fq, uint32_t ncols, const uqb_colspec* spec, uqb_array** cols);
 
 /* ---- stage 2: symbol mapping + bit packing (replaces encoder_fixed uq.py:108-182 and
@@ -243,6 +244,11 @@ int uqb_narrow_u32(uqb_ctx* ctx, const uqb_array* a, uint32_t itemsize, uqb_arra
  * which makes memcmp order equal numpy's field-by-field unsigned comparison (uq.py:814-816, 828-830) */
 int uqb_columns_to_rows(uqb_ctx* ctx, uint32_t ncols, uqb_array* const* cols, uqb_array** rows);
 int uqb_rows_to_columns(uqb_ctx* ctx, const uqb_array* rows, uint32_t ncols, const uint32_t* itemsizes, uqb_array** cols);
+/* the same with a kind per column (kinds NULL = all 0): 0 little-endian integer (stored big-endian in the row), 1 bytes
+ * copied in order ('strings' columns, E1: memcmp of zero-padded bytes is numpy's order of S values) */
+int uqb_columns_to_rows_ex(uqb_ctx* ctx, uint32_t ncols, uqb_array* const* cols, const uint8_t* kinds, uqb_array** rows);
+int uqb_rows_to_columns_ex(uqb_ctx* ctx, const uqb_array* rows, uint32_t ncols, const uint32_t* itemsizes, const uint8_t* kinds,
+                           uqb_array** cols);
 
 /* ---- stage 4: physical layouts (replaces write_pattern uq.py:257-270) ------------------------ */
 /* pattern ids: 0='0.1' 1='1.1' 2='2.1' 3='3.1' 4='0.2' 5='1.2' 6='2.2' 7='3.2'.  Produces the exact
@@ -253,7 +259,7 @@ int uqb_unlayout(uqb_ctx* ctx, const uqb_array* stream, uint64_t n, uint32_t wid
 
 /* ---- stage 5: decode (replaces uq.py:1002-1058) -------------------------------------------- */
 typedef struct {
-    uint8_t  format, itemsize, offset, _pad[5];
+    uint8_t  format, itemsize, offset, _pad[5];   /* format and itemsize as in uqb_colspec; strings: text = bytes up to the first NUL */
     int64_t  min_val;
     const uint8_t* dict;       /* host: mapping strings, dict_count rows x dict_width bytes zero padded */
     uint64_t dict_count;
@@ -274,10 +280,10 @@ typedef struct {
 int uqb_decode(uqb_ctx* ctx, const uqb_array* dna, const uqb_array* qual, uqb_array* const* cols,
                const uqb_decode_params* p, uqb_array** fastq);
 
-/* ---- synthetic inputs for bench/tests (same generator as oracle/synth.py) ------------------- */
+/* ---- synthetic inputs for bench/tests (same generator as oracle/synth.py, oracle/synth_umi.py) - */
 typedef struct {
-    uint32_t kind;        /* 0 illumina, 1 genome, 2 casava, 3 ont */
-    uint32_t length;      /* read length (kinds 0-2) */
+    uint32_t kind;        /* 0 illumina, 1 genome, 2 casava, 3 ont, 4 umi (illumina header + '_' + 6-12 of ACGTN) */
+    uint32_t length;      /* read length (kinds 0-2, 4) */
     uint32_t len_lo, len_hi; /* kind 3 */
     uint64_t seed, first, n; /* records first .. first+n-1 */
     uint64_t genome, pool;   /* kind 1 */

@@ -131,6 +131,8 @@ SIGNATURES = {
     "uqb_narrow_u32": (C.c_int, [P, P, C.c_uint32, PP]),
     "uqb_columns_to_rows": (C.c_int, [P, C.c_uint32, PP, PP]),
     "uqb_rows_to_columns": (C.c_int, [P, P, C.c_uint32, C.POINTER(C.c_uint32), PP]),
+    "uqb_columns_to_rows_ex": (C.c_int, [P, C.c_uint32, PP, P, PP]),
+    "uqb_rows_to_columns_ex": (C.c_int, [P, P, C.c_uint32, C.POINTER(C.c_uint32), P, PP]),
     "uqb_layout": (C.c_int, [P, P, C.c_int, PP]),
     "uqb_unlayout": (C.c_int, [P, P, C.c_uint64, C.c_uint32, C.c_int, PP]),
     "uqb_decode": (C.c_int, [P, P, P, PP, C.POINTER(DecodeParams), PP]),

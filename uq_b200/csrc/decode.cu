@@ -38,6 +38,13 @@ __device__ __forceinline__ unsigned long long load_le(const uint8_t* p, uint32_t
     return v;
 }
 
+// 'strings' column (format 2, E1): the token is the value's bytes up to the first NUL
+__device__ __forceinline__ uint32_t str_len(const uint8_t* p, uint32_t w) {
+    uint32_t n = 0;
+    while (n < w && p[n]) n++;
+    return n;
+}
+
 __device__ __forceinline__ uint32_t dec_digits(long long v) {
     uint32_t n = v < 0 ? 1u : 0u;
     unsigned long long a = v < 0 ? (unsigned long long)(-(v + 1)) + 1ull : (unsigned long long)v;
@@ -76,11 +83,14 @@ __device__ __forceinline__ uint32_t row_read_len(const uint8_t* row, uint32_t w,
     return 0;
 }
 
+template <bool STR>
 __device__ __forceinline__ uint32_t qname_text_len(const dec_params& P, uint64_t r) {
     uint32_t n = P.prefix_len + P.suffix_len;
     for (uint32_t c = 0; c < P.ncols; c++) {
         const dec_col& dc = P.cols[c];
-        unsigned long long raw = load_le(dc.data + r * dc.itemsize, dc.itemsize);
+        const uint8_t* p = dc.data + r * dc.itemsize;
+        if (STR && dc.format == 2) { n += str_len(p, dc.itemsize); if (c < P.nseps) n += 1; continue; }
+        unsigned long long raw = load_le(p, dc.itemsize);
         if (dc.format == 0) n += raw < dc.dict_count ? dc.dict_len[raw] : 0u;
         else n += dec_digits((long long)raw + (dc.offset ? dc.min_val : 0ll));
         if (c < P.nseps) n += 1;
@@ -88,7 +98,8 @@ __device__ __forceinline__ uint32_t qname_text_len(const dec_params& P, uint64_t
     return n;
 }
 
-__global__ void __launch_bounds__(DC) k_decode_len(const dec_params* __restrict__ Pp, const uint8_t* __restrict__ dna, uint64_t n,
+template <bool STR>
+__device__ __forceinline__ void decode_len_body(const dec_params* __restrict__ Pp, const uint8_t* __restrict__ dna, uint64_t n,
                                                   uint32_t* __restrict__ rec_len, unsigned long long* __restrict__ bad_row) {
     const uint64_t r = (uint64_t)blockIdx.x * DC + threadIdx.x;
     if (r >= n) return;
@@ -96,7 +107,7 @@ __global__ void __launch_bounds__(DC) k_decode_len(const dec_params* __restrict_
     bool bad = false;
     const uint32_t len = row_read_len(dna + r * P.wd, P.wd, P.bb, P.dna_max, P.variable, &bad);
     if (bad) atomicMin(bad_row, (unsigned long long)r);
-    rec_len[r] = qname_text_len(P, r) + 1 + len + 1 + 2 + len + 1;
+    rec_len[r] = qname_text_len<STR>(P, r) + 1 + len + 1 + 2 + len + 1;
 }
 
 __device__ __forceinline__ unsigned row_symbol(const uint8_t* row, uint32_t w, uint32_t bits, uint32_t pos) {
@@ -106,7 +117,8 @@ __device__ __forceinline__ unsigned row_symbol(const uint8_t* row, uint32_t w, u
     return (v >> (16 - (pos & 7u) - bits)) & ((1u << bits) - 1u);
 }
 
-__global__ void __launch_bounds__(DC) k_decode_write(const dec_params* __restrict__ Pp, const uint8_t* __restrict__ dna,
+template <bool STR>
+__device__ __forceinline__ void decode_write_body(const dec_params* __restrict__ Pp, const uint8_t* __restrict__ dna,
                                                     const uint8_t* __restrict__ qual, uint64_t n, const uint64_t* __restrict__ rec_off,
                                                     uint8_t* __restrict__ out) {
     __shared__ uint8_t base_char[256], qual_char[256];
@@ -133,10 +145,13 @@ __global__ void __launch_bounds__(DC) k_decode_write(const dec_params* __restric
             long long v = 0;
             if (c < P.ncols) {
                 const dec_col& dc = P.cols[c];
-                raw = load_le(dc.data + r * dc.itemsize, dc.itemsize);
-                if (dc.format == 0) {
+                if (STR && dc.format == 2) {
+                    tl = str_len(dc.data + r * dc.itemsize, dc.itemsize);
+                } else if (dc.format == 0) {
+                    raw = load_le(dc.data + r * dc.itemsize, dc.itemsize);
                     tl = raw < dc.dict_count ? dc.dict_len[raw] : 0u;
                 } else {
+                    raw = load_le(dc.data + r * dc.itemsize, dc.itemsize);
                     v = (long long)raw + (dc.offset ? dc.min_val : 0ll);
                     tl = dec_digits(v);
                 }
@@ -152,7 +167,10 @@ __global__ void __launch_bounds__(DC) k_decode_write(const dec_params* __restric
                 const dec_col& dc = P.cols[c];
                 uint8_t* w = o + run + incl - tl;
                 uint32_t body = tl - (c < P.nseps ? 1u : 0u);
-                if (dc.format == 0) {
+                if (STR && dc.format == 2) {
+                    const uint8_t* sp = dc.data + r * dc.itemsize;
+                    for (uint32_t i = 0; i < body; i++) w[i] = sp[i];
+                } else if (dc.format == 0) {
                     if (raw < dc.dict_count) {
                         const uint8_t* sp = dc.dict + raw * dc.dict_width;
                         for (uint32_t i = 0; i < body; i++) w[i] = sp[i];
@@ -236,11 +254,18 @@ __device__ __forceinline__ void extract_chunk16_any(uint32_t bits, const uint32_
 }
 
 // QNAME text of record r -> w (prefix, columns with separators, suffix, newline); returns its length
+template <bool STR>
 __device__ __forceinline__ uint32_t qname_write(const dec_params& P, uint64_t r, uint8_t* w) {
     uint32_t n = 0;
     for (uint32_t i = 0; i < P.prefix_len; i++) w[n++] = P.prefix[i];
     for (uint32_t c = 0; c < P.ncols; c++) {
         const dec_col& dc = P.cols[c];
+        if (STR && dc.format == 2) {
+            const uint8_t* sp = dc.data + r * dc.itemsize;
+            for (uint32_t i = 0; i < dc.itemsize && sp[i]; i++) w[n++] = sp[i];
+            if (c < P.nseps) w[n++] = P.seps[c];
+            continue;
+        }
         const unsigned long long raw = load_le(dc.data + r * dc.itemsize, dc.itemsize);
         if (dc.format == 0) {
             if (raw < dc.dict_count) {
@@ -266,7 +291,9 @@ __device__ __forceinline__ uint32_t qname_write(const dec_params& P, uint64_t r,
 // One QNAME column of record r -> text at w + (offset of that column inside the line): every (record, column) pair is a
 // work item of its own, so the QNAME lines of a tile are formatted by all threads instead of one thread per record.
 // The item recomputes the text lengths of the columns in front of it (a few compares each) to find its place.
+template <bool STR>
 __device__ __forceinline__ uint32_t col_text_len(const dec_col& dc, uint64_t r, unsigned long long* raw_out, long long* v_out) {
+    if (STR && dc.format == 2) { *raw_out = 0; *v_out = 0; return str_len(dc.data + r * dc.itemsize, dc.itemsize); }
     const unsigned long long raw = load_le(dc.data + r * dc.itemsize, dc.itemsize);
     *raw_out = raw;
     if (dc.format == 0) { *v_out = 0; return raw < dc.dict_count ? dc.dict_len[raw] : 0u; }
@@ -275,15 +302,19 @@ __device__ __forceinline__ uint32_t col_text_len(const dec_col& dc, uint64_t r, 
     return dec_digits(v);
 }
 
+template <bool STR>
 __device__ __forceinline__ void qname_write_col(const dec_params& P, uint64_t r, uint32_t c, uint8_t* w) {
     uint32_t at = P.prefix_len;
     unsigned long long raw = 0;
     long long v = 0;
-    for (uint32_t k = 0; k < c; k++) at += col_text_len(P.cols[k], r, &raw, &v) + 1u;      // + separator (k < nseps since k < c <= ncols - 1)
+    for (uint32_t k = 0; k < c; k++) at += col_text_len<STR>(P.cols[k], r, &raw, &v) + 1u;      // + separator (k < nseps since k < c <= ncols - 1)
     const dec_col& dc = P.cols[c];
-    const uint32_t tl = col_text_len(dc, r, &raw, &v);
+    const uint32_t tl = col_text_len<STR>(dc, r, &raw, &v);
     uint8_t* o = w + at;
-    if (dc.format == 0) {
+    if (STR && dc.format == 2) {
+        const uint8_t* sp = dc.data + r * dc.itemsize;
+        for (uint32_t i = 0; i < tl; i++) o[i] = sp[i];
+    } else if (dc.format == 0) {
         if (raw < dc.dict_count) {
             const uint8_t* sp = dc.dict + raw * dc.dict_width;
             for (uint32_t i = 0; i < tl; i++) o[i] = sp[i];
@@ -313,7 +344,8 @@ struct dt_smem {
     uint32_t fix[DT_FIX_CAP];
 };
 
-__global__ void __launch_bounds__(DT_THREADS) k_decode_tiles(const dec_params* __restrict__ Pp, const uint8_t* __restrict__ dna,
+template <bool STR>
+__device__ __forceinline__ void decode_tiles_body(const dec_params* __restrict__ Pp, const uint8_t* __restrict__ dna,
                                                             const uint8_t* __restrict__ qual, uint64_t n, const uint64_t* __restrict__ rec_off,
                                                             uint64_t total, uint8_t* __restrict__ out, unsigned int* __restrict__ fallback) {
     extern __shared__ __align__(16) uint8_t dt_raw[];
@@ -400,9 +432,9 @@ __global__ void __launch_bounds__(DT_THREADS) k_decode_tiles(const dec_params* _
                 const uint32_t qi = item - nsymitems - ndnaitems, c = qi / nrec, i = qi - c * nrec;       // record index fastest
                 uint8_t* w = S->text + S->toff[i];
                 if (P.ncols == 0) {
-                    qname_write(P, r0 + i, w);
+                    qname_write<STR>(P, r0 + i, w);
                 } else {
-                    qname_write_col(P, r0 + i, c, w);
+                    qname_write_col<STR>(P, r0 + i, c, w);
                 }
                 if (c == 0) {
                     const uint32_t hl = S->toff[i + 1] - S->toff[i] - 2u * L - 4u;             // record length - (2 L + 4) = QNAME line length
@@ -491,6 +523,25 @@ __global__ void __launch_bounds__(DT_THREADS) k_decode_tiles(const dec_params* _
     if (tid == 0) asm volatile("cp.async.bulk.wait_group 0;" ::: "memory");     // the last bulk store has landed
 }
 
+// The decode kernels: the plain ones for containers without 'strings' QNAME columns (exactly the kernels those always
+// ran), the _str ones when a column holds strings (E1).
+__global__ void __launch_bounds__(DC) k_decode_len(const dec_params* __restrict__ Pp, const uint8_t* __restrict__ dna, uint64_t n,
+                                                  uint32_t* __restrict__ rec_len, unsigned long long* __restrict__ bad_row) { decode_len_body<false>(Pp, dna, n, rec_len, bad_row); }
+__global__ void __launch_bounds__(DC) k_decode_len_str(const dec_params* __restrict__ Pp, const uint8_t* __restrict__ dna, uint64_t n,
+                                                  uint32_t* __restrict__ rec_len, unsigned long long* __restrict__ bad_row) { decode_len_body<true>(Pp, dna, n, rec_len, bad_row); }
+__global__ void __launch_bounds__(DC) k_decode_write(const dec_params* __restrict__ Pp, const uint8_t* __restrict__ dna,
+                                                    const uint8_t* __restrict__ qual, uint64_t n, const uint64_t* __restrict__ rec_off,
+                                                    uint8_t* __restrict__ out) { decode_write_body<false>(Pp, dna, qual, n, rec_off, out); }
+__global__ void __launch_bounds__(DC) k_decode_write_str(const dec_params* __restrict__ Pp, const uint8_t* __restrict__ dna,
+                                                    const uint8_t* __restrict__ qual, uint64_t n, const uint64_t* __restrict__ rec_off,
+                                                    uint8_t* __restrict__ out) { decode_write_body<true>(Pp, dna, qual, n, rec_off, out); }
+__global__ void __launch_bounds__(DT_THREADS) k_decode_tiles(const dec_params* __restrict__ Pp, const uint8_t* __restrict__ dna,
+                                                            const uint8_t* __restrict__ qual, uint64_t n, const uint64_t* __restrict__ rec_off,
+                                                            uint64_t total, uint8_t* __restrict__ out, unsigned int* __restrict__ fallback) { decode_tiles_body<false>(Pp, dna, qual, n, rec_off, total, out, fallback); }
+__global__ void __launch_bounds__(DT_THREADS) k_decode_tiles_str(const dec_params* __restrict__ Pp, const uint8_t* __restrict__ dna,
+                                                            const uint8_t* __restrict__ qual, uint64_t n, const uint64_t* __restrict__ rec_off,
+                                                            uint64_t total, uint8_t* __restrict__ out, unsigned int* __restrict__ fallback) { decode_tiles_body<true>(Pp, dna, qual, n, rec_off, total, out, fallback); }
+
 extern "C" int uqb_decode(uqb_ctx* ctx, const uqb_array* dna, const uqb_array* qual, uqb_array* const* cols,
                           const uqb_decode_params* p, uqb_array** fastq) {
     const uint64_t n = dna->n;
@@ -519,6 +570,7 @@ extern "C" int uqb_decode(uqb_ctx* ctx, const uqb_array* dna, const uqb_array* q
         const uqb_decode_col& sc = p->cols[c];
         dec_col& dc = hp->cols[c];
         if (cols[c]->n != n || cols[c]->width != sc.itemsize) { rc = uqb_fail(ctx, "decode: column %u shape mismatch", c); break; }
+        if (sc.format > 2 || (sc.format == 2 && sc.itemsize == 0)) { rc = uqb_fail(ctx, "decode: column %u has format %u, width %u", c, sc.format, sc.itemsize); break; }
         dc.data = (const uint8_t*)cols[c]->d;
         dc.itemsize = sc.itemsize; dc.format = sc.format; dc.offset = sc.offset; dc.min_val = sc.min_val;
         dc.dict_count = sc.dict_count; dc.dict_width = sc.dict_width;
@@ -559,7 +611,10 @@ extern "C" int uqb_decode(uqb_ctx* ctx, const uqb_array* dna, const uqb_array* q
     unsigned long long* d_bad;
     UQB_TRY(uqb_dalloc_t(ctx, &d_bad, 1));
     UQB_CUDA(cudaMemsetAsync(d_bad, 0xFF, 8, ctx->stream));
-    if (n) UQB_LAUNCH(k_decode_len, uqb_blocks(n, DC), DC, 0, dp, (const uint8_t*)dna->d, n, rec_len, d_bad);
+    bool has_str = false;
+    for (uint32_t c = 0; c < p->ncols; c++) has_str |= p->cols[c].format == 2;
+    if (n && has_str) UQB_LAUNCH(k_decode_len_str, uqb_blocks(n, DC), DC, 0, dp, (const uint8_t*)dna->d, n, rec_len, d_bad);
+    else if (n) UQB_LAUNCH(k_decode_len, uqb_blocks(n, DC), DC, 0, dp, (const uint8_t*)dna->d, n, rec_len, d_bad);
     UQB_TRY(uqb_scan_u32_to_u64(ctx, rec_len, rec_off, n, d_total));
     UQB_TRY(uqb_readback(ctx, &total, d_total, 8));
     unsigned long long bad_row = ~0ull;
@@ -581,17 +636,24 @@ extern "C" int uqb_decode(uqb_ctx* ctx, const uqb_array* dna, const uqb_array* q
         unsigned int* d_fb;
         UQB_TRY(uqb_dalloc_t(ctx, &d_fb, 1));
         UQB_CUDA(cudaMemsetAsync(d_fb, 0, 4, ctx->stream));
-        UQB_CUDA(cudaFuncSetAttribute(k_decode_tiles, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(dt_smem)));
         uint64_t tab = 0;
         for (uint32_t c = 0; c < p->ncols; c++) tab += n * cols[c]->width;
-        UQB_LAUNCH_B(n * ((uint64_t)dna->width + qual->width + 8) + tab + total, k_decode_tiles, uqb_grid(ctx, n, DT_R, 4), DT_THREADS, sizeof(dt_smem), dp,
-                     (const uint8_t*)dna->d, (const uint8_t*)qual->d, n, rec_off, total, (uint8_t*)(*fastq)->d, d_fb);
+        if (has_str) {
+            UQB_CUDA(cudaFuncSetAttribute(k_decode_tiles_str, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(dt_smem)));
+            UQB_LAUNCH_B(n * ((uint64_t)dna->width + qual->width + 8) + tab + total, k_decode_tiles_str, uqb_grid(ctx, n, DT_R, 4), DT_THREADS, sizeof(dt_smem), dp,
+                         (const uint8_t*)dna->d, (const uint8_t*)qual->d, n, rec_off, total, (uint8_t*)(*fastq)->d, d_fb);
+        } else {
+            UQB_CUDA(cudaFuncSetAttribute(k_decode_tiles, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(dt_smem)));
+            UQB_LAUNCH_B(n * ((uint64_t)dna->width + qual->width + 8) + tab + total, k_decode_tiles, uqb_grid(ctx, n, DT_R, 4), DT_THREADS, sizeof(dt_smem), dp,
+                         (const uint8_t*)dna->d, (const uint8_t*)qual->d, n, rec_off, total, (uint8_t*)(*fastq)->d, d_fb);
+        }
         unsigned int fb = 0;
         UQB_TRY(uqb_readback(ctx, &fb, d_fb, 4));
         UQB_TRY(uqb_dfree(ctx, d_fb, 4));
         done = fb == 0;
     }
-    if (n && !done) UQB_LAUNCH(k_decode_write, uqb_grid(ctx, n, DC / 32, 16), DC, 0, dp, (const uint8_t*)dna->d, (const uint8_t*)qual->d, n, rec_off, (uint8_t*)(*fastq)->d);
+    if (n && !done && has_str) UQB_LAUNCH(k_decode_write_str, uqb_grid(ctx, n, DC / 32, 16), DC, 0, dp, (const uint8_t*)dna->d, (const uint8_t*)qual->d, n, rec_off, (uint8_t*)(*fastq)->d);
+    else if (n && !done) UQB_LAUNCH(k_decode_write, uqb_grid(ctx, n, DC / 32, 16), DC, 0, dp, (const uint8_t*)dna->d, (const uint8_t*)qual->d, n, rec_off, (uint8_t*)(*fastq)->d);
     UQB_TRY(uqb_dfree(ctx, rec_len, n * 4));
     UQB_TRY(uqb_dfree(ctx, rec_off, n * 8));
     UQB_TRY(uqb_dfree(ctx, d_total, 8));

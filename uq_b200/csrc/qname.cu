@@ -357,6 +357,43 @@ __global__ void __launch_bounds__(QN) k_encode_rank(const uint32_t* __restrict__
     for (uint64_t i = (uint64_t)blockIdx.x * QN + threadIdx.x; i < n; i += (uint64_t)gridDim.x * QN) out[i] = (T)rank[i];
 }
 
+// 'strings' column (format 2, declared extension E1): every record's token, left-aligned and zero padded to w bytes.
+// A CTA takes QS_R consecutive records, whose output is ONE contiguous range of QS_R * w bytes: the token bytes are
+// gathered into shared memory (all threads over the flat range, so narrow columns keep every thread busy) and the
+// range leaves as aligned 16-byte stores.
+#define QS_R 128
+__global__ void __launch_bounds__(QN) k_encode_str(const uint8_t* __restrict__ d, const uint64_t* __restrict__ line_off,
+                                                  const uint32_t* __restrict__ span, uint32_t prefix_len, uint32_t w, uint64_t n,
+                                                  uint8_t* __restrict__ out, const uint8_t* __restrict__ names, uint32_t name_pitch) {
+    __shared__ __align__(16) uint8_t stage[QS_R * 255 + 16];
+    __shared__ const uint8_t* src[QS_R];
+    __shared__ uint32_t len[QS_R];
+    const uint64_t ntiles = (n + QS_R - 1) / QS_R;
+    for (uint64_t t = blockIdx.x; t < ntiles; t += gridDim.x) {
+        const uint64_t r0 = t * QS_R;
+        const uint32_t nr = (uint32_t)(n - r0 < QS_R ? n - r0 : QS_R);
+        __syncthreads();                                             // previous tile stored
+        if (threadIdx.x < nr) {
+            const uint64_t r = r0 + threadIdx.x;
+            const uint32_t sp = __ldg(span + r);
+            const uint32_t rel = (sp >> SPAN_LEN_BITS) & SPAN_MAXLEN;
+            src[threadIdx.x] = (names ? names + r * name_pitch + 1 : d + __ldg(line_off + 4 * r)) + prefix_len + rel;
+            len[threadIdx.x] = sp & SPAN_MAXLEN;
+        }
+        __syncthreads();
+        const uint32_t total = nr * w;
+        for (uint32_t k = threadIdx.x; k < total; k += QN) {
+            const uint32_t i = k / w, b = k - i * w;
+            stage[k] = b < len[i] ? __ldg(src[i] + b) : (uint8_t)0;
+        }
+        __syncthreads();
+        uint8_t* o = out + r0 * w;                                   // QS_R * w bytes per tile: a multiple of 16
+        const uint32_t nvec = (reinterpret_cast<uintptr_t>(out) & 15u) ? 0u : total >> 4;
+        for (uint32_t v = threadIdx.x; v < nvec; v += QN) reinterpret_cast<uint4*>(o)[v] = reinterpret_cast<const uint4*>(stage)[v];
+        for (uint32_t k = 16u * nvec + threadIdx.x; k < total; k += QN) o[k] = stage[k];
+    }
+}
+
 template <typename T>
 static int encode_col(uqb_ctx* ctx, const uqb_qcol& qc, const uqb_colspec& sp, uint64_t n, void* out) {
     unsigned g = uqb_grid(ctx, n, QN * 4, 8);
@@ -371,7 +408,16 @@ extern "C" int uqb_qname_encode(uqb_ctx* ctx, uqb_fastq* fq, uint32_t ncols, con
     for (uint32_t c = 0; c < ncols; c++) {
         const uqb_qcol& qc = fq->qcols[c];
         if (spec[c].format == 0 && !qc.rank) return uqb_fail(ctx, "qname_encode: column %u has no dictionary ranks", c);
+        if (spec[c].format > 2) return uqb_fail(ctx, "qname_encode: column %u has format %u", c, spec[c].format);
+        if (spec[c].format == 2 && spec[c].itemsize == 0) return uqb_fail(ctx, "qname_encode: string column %u has width 0", c);
         UQB_TRY(uqb_new_array(ctx, N, spec[c].itemsize, &cols[c]));
+        if (spec[c].format == 2) {          // token bytes, zero padded to itemsize (the host sizes it to the longest token)
+            const uint32_t w = spec[c].itemsize;
+            const uint64_t src_bytes = N * 4 + N * w + (fq->names ? 0 : 8 * N);
+            if (N) UQB_LAUNCH_B(src_bytes + N * w, k_encode_str, uqb_grid(ctx, N, QS_R, 16), QN, 0, fq->d, fq->line_off, qc.span,
+                                fq->prefix_len, w, N, (uint8_t*)cols[c]->d, (const uint8_t*)fq->names, fq->name_pitch);
+            continue;
+        }
         switch (spec[c].itemsize) {
             case 1: UQB_TRY(encode_col<uint8_t>(ctx, qc, spec[c], N, cols[c]->d)); break;
             case 2: UQB_TRY(encode_col<uint16_t>(ctx, qc, spec[c], N, cols[c]->d)); break;

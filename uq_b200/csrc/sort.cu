@@ -1133,14 +1133,125 @@ __global__ void __launch_bounds__(ST) k_rows_to_cols_staged(col_desc_out cd, uin
     }
 }
 
-static bool cr_staged_ok(const uint32_t* sizes, uint32_t ncols, uint32_t width, const void* rows) {
+// ---- the same transforms with byte columns (kind 1: 'strings' QNAME columns, E1) -------------------------------
+// A byte column enters the row as it is: memcmp of its zero-padded bytes is numpy's order of S values.  Bit c of
+// `bytes_mask` marks column c as such a column.  These kernels are separate from the ones above so that tables of
+// integer columns only keep exactly the kernels they always had.
+__global__ void __launch_bounds__(ST) k_cols_to_rows_mixed(col_desc cd, uint64_t bytes_mask, uint64_t n, uint8_t* __restrict__ rows) {
+    for (uint64_t t = (uint64_t)blockIdx.x * ST + threadIdx.x; t < n * cd.ncols; t += (uint64_t)gridDim.x * ST) {
+        uint64_t r = t / cd.ncols;
+        uint32_t c = (uint32_t)(t - r * cd.ncols);
+        uint32_t sz = cd.size[c];
+        const uint8_t* src = cd.p[c] + r * sz;
+        uint8_t* dst = rows + r * cd.width + cd.off[c];
+        if ((bytes_mask >> c) & 1ull) for (uint32_t b = 0; b < sz; b++) dst[b] = src[b];
+        else                          for (uint32_t b = 0; b < sz; b++) dst[b] = src[sz - 1 - b];
+    }
+}
+
+__global__ void __launch_bounds__(ST) k_rows_to_cols_mixed(col_desc_out cd, uint64_t bytes_mask, uint64_t n, const uint8_t* __restrict__ rows) {
+    for (uint64_t t = (uint64_t)blockIdx.x * ST + threadIdx.x; t < n * cd.ncols; t += (uint64_t)gridDim.x * ST) {
+        uint64_t r = t / cd.ncols;
+        uint32_t c = (uint32_t)(t - r * cd.ncols);
+        uint32_t sz = cd.size[c];
+        uint8_t* dst = cd.p[c] + r * sz;
+        const uint8_t* src = rows + r * cd.width + cd.off[c];
+        if ((bytes_mask >> c) & 1ull) for (uint32_t b = 0; b < sz; b++) dst[b] = src[b];
+        else                          for (uint32_t b = 0; b < sz; b++) dst[b] = src[sz - 1 - b];
+    }
+}
+
+// Staged form: integer columns as in k_cols_to_rows_staged (one thread per row, typed loads); a byte column's values of
+// the CTA's rows are one contiguous range of nr * size bytes, which all threads copy together (coalesced) into the rows.
+__global__ void __launch_bounds__(ST) k_cols_to_rows_staged_mixed(col_desc cd, uint64_t bytes_mask, uint64_t n, uint8_t* __restrict__ rows) {
+    __shared__ __align__(16) uint8_t stage[ST * CR_MAXW];
+    const uint64_t nblk = (n + ST - 1) / ST;
+    for (uint64_t blk = blockIdx.x; blk < nblk; blk += gridDim.x) {
+        const uint64_t r0 = blk * ST, r = r0 + threadIdx.x;
+        const uint32_t nr = (uint32_t)(n - r0 < ST ? n - r0 : ST);
+        __syncthreads();
+        for (uint32_t c = 0; c < cd.ncols; c++) {
+            const uint32_t sz = cd.size[c];
+            if ((bytes_mask >> c) & 1ull) {
+                const uint8_t* src = cd.p[c] + r0 * sz;
+                for (uint32_t k = threadIdx.x; k < nr * sz; k += ST) {
+                    const uint32_t i = k / sz;
+                    stage[i * cd.width + cd.off[c] + (k - i * sz)] = src[k];
+                }
+            } else if (r < n) {
+                uint8_t* dst = stage + threadIdx.x * cd.width;
+                const unsigned long long v = sz == 1 ? cr_load<uint8_t>(cd.p[c], r) : sz == 2 ? cr_load<uint16_t>(cd.p[c], r)
+                                           : sz == 4 ? cr_load<uint32_t>(cd.p[c], r) : cr_load<uint64_t>(cd.p[c], r);
+                for (uint32_t b = 0; b < sz; b++) dst[cd.off[c] + b] = (uint8_t)(v >> (8 * (sz - 1 - b)));   // big-endian key bytes
+            }
+        }
+        __syncthreads();
+        const uint32_t total = nr * cd.width;
+        uint8_t* out = rows + r0 * cd.width;                                  // ST * width bytes per block: 4-byte aligned
+        for (uint32_t k = threadIdx.x; k < (total >> 2); k += ST) reinterpret_cast<uint32_t*>(out)[k] = reinterpret_cast<const uint32_t*>(stage)[k];
+        if (threadIdx.x < (total & 3u)) out[(total & ~3u) + threadIdx.x] = stage[(total & ~3u) + threadIdx.x];
+    }
+}
+
+__global__ void __launch_bounds__(ST) k_rows_to_cols_staged_mixed(col_desc_out cd, uint64_t bytes_mask, uint64_t n, const uint8_t* __restrict__ rows) {
+    __shared__ __align__(16) uint8_t stage[ST * CR_MAXW];
+    const uint64_t nblk = (n + ST - 1) / ST;
+    for (uint64_t blk = blockIdx.x; blk < nblk; blk += gridDim.x) {
+        const uint64_t r0 = blk * ST, r = r0 + threadIdx.x;
+        const uint32_t nr = (uint32_t)(n - r0 < ST ? n - r0 : ST);
+        const uint32_t total = nr * cd.width;
+        const uint8_t* in = rows + r0 * cd.width;
+        __syncthreads();
+        for (uint32_t k = threadIdx.x; k < (total >> 2); k += ST) reinterpret_cast<uint32_t*>(stage)[k] = reinterpret_cast<const uint32_t*>(in)[k];
+        if (threadIdx.x < (total & 3u)) stage[(total & ~3u) + threadIdx.x] = in[(total & ~3u) + threadIdx.x];
+        __syncthreads();
+        for (uint32_t c = 0; c < cd.ncols; c++) {
+            const uint32_t sz = cd.size[c];
+            if ((bytes_mask >> c) & 1ull) {
+                uint8_t* dst = cd.p[c] + r0 * sz;
+                for (uint32_t k = threadIdx.x; k < nr * sz; k += ST) {
+                    const uint32_t i = k / sz;
+                    dst[k] = stage[i * cd.width + cd.off[c] + (k - i * sz)];
+                }
+            } else if (r < n) {
+                const uint8_t* src = stage + threadIdx.x * cd.width;
+                unsigned long long v = 0;
+                for (uint32_t b = 0; b < sz; b++) v = (v << 8) | src[cd.off[c] + b];
+                if (sz == 1) reinterpret_cast<uint8_t*>(cd.p[c])[r] = (uint8_t)v;
+                else if (sz == 2) reinterpret_cast<uint16_t*>(cd.p[c])[r] = (uint16_t)v;
+                else if (sz == 4) reinterpret_cast<uint32_t*>(cd.p[c])[r] = (uint32_t)v;
+                else reinterpret_cast<uint64_t*>(cd.p[c])[r] = v;
+            }
+        }
+    }
+}
+
+// kinds == NULL or all 0: integer columns only
+static int cr_bytes_mask(uqb_ctx* ctx, const uint8_t* kinds, uint32_t ncols, uint64_t* mask) {
+    *mask = 0;
+    if (!kinds) return 0;
+    for (uint32_t c = 0; c < ncols; c++) {
+        if (kinds[c] > 1) return uqb_fail(ctx, "columns/rows: column %u has kind %u (0 integer, 1 bytes)", c, kinds[c]);
+        if (kinds[c]) *mask |= 1ull << c;
+    }
+    return 0;
+}
+
+static bool cr_staged_ok(const uint32_t* sizes, uint32_t ncols, uint32_t width, const void* rows, uint64_t bytes_mask = 0) {
     if (width > CR_MAXW || (reinterpret_cast<uintptr_t>(rows) & 3u)) return false;
-    for (uint32_t c = 0; c < ncols; c++) if (sizes[c] != 1 && sizes[c] != 2 && sizes[c] != 4 && sizes[c] != 8) return false;
+    for (uint32_t c = 0; c < ncols; c++)
+        if (!((bytes_mask >> c) & 1ull) && sizes[c] != 1 && sizes[c] != 2 && sizes[c] != 4 && sizes[c] != 8) return false;
     return true;
 }
 
 extern "C" int uqb_columns_to_rows(uqb_ctx* ctx, uint32_t ncols, uqb_array* const* cols, uqb_array** rows) {
+    return uqb_columns_to_rows_ex(ctx, ncols, cols, nullptr, rows);
+}
+
+extern "C" int uqb_columns_to_rows_ex(uqb_ctx* ctx, uint32_t ncols, uqb_array* const* cols, const uint8_t* kinds, uqb_array** rows) {
     if (ncols == 0 || ncols > UQB_MAX_COLS) return uqb_fail(ctx, "columns_to_rows: bad column count %u", ncols);
+    uint64_t bm;
+    UQB_TRY(cr_bytes_mask(ctx, kinds, ncols, &bm));
     col_desc cd;
     cd.ncols = ncols;
     uint32_t w = 0;
@@ -1151,13 +1262,25 @@ extern "C" int uqb_columns_to_rows(uqb_ctx* ctx, uint32_t ncols, uqb_array* cons
     }
     cd.width = w;
     UQB_TRY(uqb_new_array(ctx, n, w, rows));
+    if (bm) {
+        if (n && cr_staged_ok(cd.size, ncols, w, (*rows)->d, bm)) UQB_LAUNCH_B(2 * n * w, k_cols_to_rows_staged_mixed, uqb_grid(ctx, n, ST, 16), ST, 0, cd, bm, n, (uint8_t*)(*rows)->d);
+        else if (n) UQB_LAUNCH_B(2 * n * w, k_cols_to_rows_mixed, uqb_grid(ctx, n * ncols, ST, 16), ST, 0, cd, bm, n, (uint8_t*)(*rows)->d);
+        return 0;
+    }
     if (n && cr_staged_ok(cd.size, ncols, w, (*rows)->d)) UQB_LAUNCH_B(2 * n * w, k_cols_to_rows_staged, uqb_grid(ctx, n, ST, 16), ST, 0, cd, n, (uint8_t*)(*rows)->d);
     else if (n) UQB_LAUNCH(k_cols_to_rows, uqb_grid(ctx, n * ncols, ST, 16), ST, 0, cd, n, (uint8_t*)(*rows)->d);
     return 0;
 }
 
 extern "C" int uqb_rows_to_columns(uqb_ctx* ctx, const uqb_array* rows, uint32_t ncols, const uint32_t* itemsizes, uqb_array** cols) {
+    return uqb_rows_to_columns_ex(ctx, rows, ncols, itemsizes, nullptr, cols);
+}
+
+extern "C" int uqb_rows_to_columns_ex(uqb_ctx* ctx, const uqb_array* rows, uint32_t ncols, const uint32_t* itemsizes, const uint8_t* kinds,
+                                      uqb_array** cols) {
     if (ncols == 0 || ncols > UQB_MAX_COLS) return uqb_fail(ctx, "rows_to_columns: bad column count %u", ncols);
+    uint64_t bm;
+    UQB_TRY(cr_bytes_mask(ctx, kinds, ncols, &bm));
     col_desc_out cd;
     cd.ncols = ncols;
     uint32_t w = 0;
@@ -1167,6 +1290,11 @@ extern "C" int uqb_rows_to_columns(uqb_ctx* ctx, const uqb_array* rows, uint32_t
     }
     cd.width = w;
     if (w != rows->width) return uqb_fail(ctx, "rows_to_columns: widths sum to %u, rows are %u wide", w, rows->width);
+    if (bm) {
+        if (rows->n && cr_staged_ok(cd.size, ncols, w, rows->d, bm)) UQB_LAUNCH_B(2 * rows->n * w, k_rows_to_cols_staged_mixed, uqb_grid(ctx, rows->n, ST, 16), ST, 0, cd, bm, rows->n, (const uint8_t*)rows->d);
+        else if (rows->n) UQB_LAUNCH_B(2 * rows->n * w, k_rows_to_cols_mixed, uqb_grid(ctx, rows->n * ncols, ST, 16), ST, 0, cd, bm, rows->n, (const uint8_t*)rows->d);
+        return 0;
+    }
     if (rows->n && cr_staged_ok(cd.size, ncols, w, rows->d)) UQB_LAUNCH_B(2 * rows->n * w, k_rows_to_cols_staged, uqb_grid(ctx, rows->n, ST, 16), ST, 0, cd, rows->n, (const uint8_t*)rows->d);
     else if (rows->n) UQB_LAUNCH(k_rows_to_cols, uqb_grid(ctx, rows->n * ncols, ST, 16), ST, 0, cd, rows->n, (const uint8_t*)rows->d);
     return 0;

@@ -1,5 +1,5 @@
 // Synthetic FASTQ generator on the device (bench / tests only): the same counter-based generator as
-// oracle/synth.py, so bench.py can create the 100 M-read inputs of BASELINE.json directly in HBM.
+// oracle/synth.py (kind 4 'umi': oracle/synth_umi.py), so bench.py can create the 100 M-read inputs of BASELINE.json directly in HBM.
 #include "common.cuh"
 
 #define SY 256
@@ -7,7 +7,8 @@
 #define IDXK 0x632BE59BD9B4E019ull
 
 enum { ST_LANE = 1, ST_TILE = 2, ST_X = 3, ST_Y = 4, ST_NPOS = 5, ST_BASE = 6, ST_QA = 7, ST_QB = 8, ST_FLAG = 9, ST_EVEN = 10,
-       ST_BARCODE = 11, ST_OFF = 12, ST_SUB = 13, ST_SUBV = 14, ST_POOL = 15, ST_LEN = 16, ST_RUN = 17, ST_CH = 18, ST_GENOME = 100 };
+       ST_BARCODE = 11, ST_OFF = 12, ST_SUB = 13, ST_SUBV = 14, ST_POOL = 15, ST_LEN = 16, ST_RUN = 17, ST_CH = 18,
+       ST_UMI_LEN = 20, ST_UMI = 21, ST_GENOME = 100 };
 
 __device__ __forceinline__ unsigned long long mix64(unsigned long long x) {
     x ^= x >> 30; x *= 0xBF58476D1CE4E5B9ull;
@@ -44,10 +45,18 @@ __device__ unsigned synth_header(uint8_t* w, const uqb_synth_params& p, unsigned
     const unsigned long long x = 1000 + rnd(p.seed, ST_X, r) % 29000, y = 1000 + rnd(p.seed, ST_Y, r) % 199000;
     unsigned n = 0;
 #define W (w ? w + n : nullptr)
-    if (p.kind == 0 || p.kind == 1) {
+    if (p.kind == 0 || p.kind == 1 || p.kind == 4) {
         n += put_str(W, "@SIM001:1:FCX123:");
         n += put_uint(W, lane); n += put_str(W, ":"); n += put_uint(W, tile); n += put_str(W, ":");
         n += put_uint(W, x); n += put_str(W, ":"); n += put_uint(W, y);
+        if (p.kind == 4) {          // umi: '_' + 6-12 symbols of ACGTN, as UMI extraction tools append them
+            const unsigned ulen = 6 + (unsigned)(rnd(p.seed, ST_UMI_LEN, r) % 7);
+            n += put_str(W, "_");
+            for (unsigned j = 0; j < ulen; j++) {
+                if (w) w[n] = (uint8_t)"ACGTN"[rnd(p.seed, ST_UMI, r * 16 + j) % 5];
+                n++;
+            }
+        }
     } else if (p.kind == 2) {
         const bool flag = rnd(p.seed, ST_FLAG, r) % 8 == 0;
         const unsigned long long even = 2 * (rnd(p.seed, ST_EVEN, r) % 20), bc = rnd(p.seed, ST_BARCODE, r) % 4;
@@ -123,7 +132,7 @@ __global__ void __launch_bounds__(SY) k_synth_write(uqb_synth_params p, const lo
 }
 
 extern "C" int uqb_synth(uqb_ctx* ctx, const uqb_synth_params* p, const int64_t* ont_len_table, uqb_array** bytes) {
-    if (p->kind > 3) return uqb_fail(ctx, "synth: kind %u", p->kind);
+    if (p->kind > 4) return uqb_fail(ctx, "synth: kind %u", p->kind);
     if (p->kind == 3 && !ont_len_table) return uqb_fail(ctx, "synth: ont needs a length table");
     if (p->kind == 1 && (p->genome <= p->length || p->pool == 0)) return uqb_fail(ctx, "synth: genome/pool too small");
     if (p->n >= (1ull << 32)) return uqb_fail(ctx, "synth: too many records");

@@ -253,7 +253,7 @@ class Context:
         return fq
 
     def synth(self, kind, n, length, seed, first=0, genome=0, pool=0, len_table=None):
-        kinds = {"illumina": 0, "genome": 1, "casava": 2, "ont": 3}
+        kinds = {"illumina": 0, "genome": 1, "casava": 2, "ont": 3, "umi": 4}
         p = L.SynthParams()
         p.kind = kinds[kind]
         if kind == "ont":
@@ -293,17 +293,26 @@ class Context:
         self.check(self.lib.uqb_narrow_u32(self.h, a.h, int(itemsize), C.byref(h)))
         return DeviceArray(self, h)
 
-    def columns_to_rows(self, cols):
+    def columns_to_rows(self, cols, kinds=None):
+        """columns -> sort rows; kinds[c]: 0 little-endian integer (big-endian in the row), 1 bytes as they are"""
         arr = (C.c_void_p * len(cols))(*[c.h for c in cols])
         h = C.c_void_p()
-        self.check(self.lib.uqb_columns_to_rows(self.h, len(cols), arr, C.byref(h)))
+        if kinds is None:
+            self.check(self.lib.uqb_columns_to_rows(self.h, len(cols), arr, C.byref(h)))
+        else:
+            k = np.ascontiguousarray(kinds, dtype=np.uint8)
+            self.check(self.lib.uqb_columns_to_rows_ex(self.h, len(cols), arr, _ptr(k), C.byref(h)))
         return DeviceArray(self, h)
 
-    def rows_to_columns(self, rows, itemsizes):
+    def rows_to_columns(self, rows, itemsizes, kinds=None):
         n = len(itemsizes)
         sizes = (C.c_uint32 * n)(*[int(s) for s in itemsizes])
         outs = (C.c_void_p * n)()
-        self.check(self.lib.uqb_rows_to_columns(self.h, rows.h, n, sizes, outs))
+        if kinds is None:
+            self.check(self.lib.uqb_rows_to_columns(self.h, rows.h, n, sizes, outs))
+        else:
+            k = np.ascontiguousarray(kinds, dtype=np.uint8)
+            self.check(self.lib.uqb_rows_to_columns_ex(self.h, rows.h, n, sizes, _ptr(k), outs))
         return [DeviceArray(self, C.c_void_p(outs[i])) for i in range(n)]
 
     def layout(self, table, pattern):

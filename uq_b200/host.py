@@ -27,6 +27,7 @@ PATTERNS = ['0.1', '1.1', '2.1', '3.1', '0.2', '1.2', '2.2', '3.2']
 PATTERN_DESC = {'0.1': (0, 0, 0), '1.2': (0, 0, 1), '3.2': (0, 1, 0), '2.1': (0, 1, 1),
                 '0.2': (1, 0, 0), '1.1': (1, 0, 1), '3.1': (1, 1, 0), '2.2': (1, 1, 1)}
 _DT = [(255, 'uint8', 1), (65535, 'uint16', 2), (4294967295, 'uint32', 4), (18446744073709551615, 'uint64', 8)]
+STRING_MAX = 255     # widest 'strings' column (E1): uqb_colspec.itemsize / uqb_decode_col.itemsize are uint8
 
 
 class UQError(Exception):
@@ -251,8 +252,19 @@ def decide_columns(colstats, n_reads, fetch_dict):
         if not demoted and cs.n_distinct > last // 10:       # uq.py:638
             demoted = True
         if demoted:
-            if not cs.all_int:                     # 'strings' (uq.py:598-601, 624-630) -> uq.py:672-673
-                raise UQError('I havent implimented this yet')
+            if not cs.all_int:                     # 'strings' (uq.py:598-601, 624-630); the reference stops at uq.py:672-673
+                # declared extension E1: the tokens themselves, zero padded to the longest one over ALL records (the
+                # reference's own `longest` undercounts after an integers -> strings switch).  An all-empty column still
+                # gets one byte: numpy has no zero-width S dtype.
+                w = int(cs.max_len)
+                if w > STRING_MAX:
+                    raise UQError('ERROR: QNAME column %d holds a token of %d bytes; a string column holds at most %d'
+                                  % (i + 1, w, STRING_MAX))
+                col['format'] = 'strings'
+                col['longest'] = w
+                col['dtype'] = '|S%d' % max(w, 1)
+                columns.append(col)
+                continue
             col['format'] = 'integers'
             col['min'], col['max'] = int(cs.min_val), int(cs.max_val)
             span = col['max'] - col['min']
@@ -280,6 +292,8 @@ def column_specs(columns):
         size = np.dtype(c['dtype']).itemsize
         if c['format'] == 'mapping':
             out.append((0, size, False, 0))
+        elif c['format'] == 'strings':
+            out.append((2, size, False, 0))
         else:
             out.append((1, size, c['offset'], c['min'] if c['offset'] else 0))
     return out
@@ -455,11 +469,29 @@ def _mix_dna_qual(ctx, out, table, name, order, raw, pattern, prepared=None):
     return order
 
 
+def qname_kinds(columns):
+    """per column: 1 = 'strings' (its bytes go into the sort row as they are, E1), 0 = integer value (big-endian in the
+    row); None when every column is an integer column"""
+    kinds = [1 if c['format'] == 'strings' else 0 for c in columns]
+    return kinds if any(kinds) else None
+
+
+def qname_rows(ctx, cols, columns):
+    """QNAME columns -> sort rows, whose memcmp order is the row order of E1: column by column, integers and mapping
+    ranks as unsigned numbers (uq.py:814-816, 828-830), strings bytewise like numpy compares S values"""
+    return ctx.columns_to_rows(cols, qname_kinds(columns))
+
+
+def qname_columns(ctx, rows, columns):
+    """sort rows (e.g. the unique ones) -> typed QNAME columns again (uq.py:842-847)"""
+    return ctx.rows_to_columns(rows, [np.dtype(m['dtype']).itemsize for m in columns], qname_kinds(columns))
+
+
 def _mix_qname(ctx, out, cols, columns, order, raw):
     """encode_qname (uq.py:808-851)."""
     if raw:
         if order is False:
-            rows = ctx.columns_to_rows(cols)
+            rows = qname_rows(ctx, cols, columns)
             order, _, _, _ = ctx.sort_rows(rows, want_perm=True)                   # uq.py:816
             rows.free()
         for c, meta in zip(cols, columns):
@@ -468,14 +500,14 @@ def _mix_qname(ctx, out, cols, columns, order, raw):
             else:
                 out.add_vector(meta['name'] + '.raw', c, meta['dtype'])
     else:
-        rows = ctx.columns_to_rows(cols)
+        rows = qname_rows(ctx, cols, columns)
         key, uniq, nu, order = _keyed(ctx, rows, order)                            # uq.py:830, 833
         rows.free()
         size = key_itemsize(nu)
         narrow = ctx.narrow_u32(key, size)
         key.free()
         out.add_vector('QNAME.key', narrow, 'uint%d' % (8 * size))
-        ucols = ctx.rows_to_columns(uniq, [np.dtype(m['dtype']).itemsize for m in columns])   # uq.py:842-847
+        ucols = qname_columns(ctx, uniq, columns)                                  # uq.py:842-847
         uniq.free()
         for c, meta in zip(ucols, columns):
             out.add_vector(meta['name'], c, meta['dtype'])
@@ -603,8 +635,8 @@ class MixFeed:
         return config_of(p['dec'], p['total'], p['prefix'], p['suffix'], p['separators'], p['columns'], sort, raw, pattern)
 
     def _table(self, t):
-        if self.tables[t] is None:                       # QNAME sort rows: the columns concatenated big-endian (uq.py:814-816)
-            self.tables[t] = self.ctx.columns_to_rows(self.p['cols'])
+        if self.tables[t] is None:                       # QNAME sort rows (uq.py:814-816)
+            self.tables[t] = qname_rows(self.ctx, self.p['cols'], self.p['columns'])
         return self.tables[t]
 
     def _sorted(self, t):
@@ -661,7 +693,7 @@ class MixFeed:
             out['QNAME.key'] = self._key('QNAME', s_on, order)
 
             def make_cols():
-                ucols = ctx.rows_to_columns(srt['uniq'], [np.dtype(m['dtype']).itemsize for m in columns])
+                ucols = qname_columns(ctx, srt['uniq'], columns)
                 host = [u.download(dtype=np.dtype(m['dtype'])).reshape(-1) for u, m in zip(ucols, columns)]
                 for u in ucols:
                     u.free()
@@ -816,8 +848,13 @@ def decode_device(ctx, dna, qual, dcols, config):
             carr[i].format = 1
             carr[i].offset = 1 if meta['offset'] else 0
             carr[i].min_val = int(meta['min']) if meta['offset'] else 0
+        elif meta['format'] == 'strings':                                          # E1 (the reference stops, uq.py:1020-1021)
+            w = np.dtype(meta['dtype'])
+            if w.kind != 'S' or not 1 <= w.itemsize <= STRING_MAX:
+                raise UQError('ERROR: QNAME column %d: a string column needs dtype |S1 .. |S%d, not %s' % (i + 1, STRING_MAX, w.str))
+            carr[i].format = 2
         else:
-            raise UQError('ERROR: I dont support string encoding yet.')          # uq.py:1020-1021
+            raise UQError('ERROR: QNAME column %d has the unknown format %r' % (i + 1, meta['format']))
     p.cols = carr
     h = C.c_void_p()
     handles = (C.c_void_p * max(ncol, 1))(*[c.h for c in dcols])

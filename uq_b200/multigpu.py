@@ -1089,7 +1089,7 @@ def encode_sharded(ctx, comm, fq, sort=None, raw=None, pattern=None, pad=False, 
         res.add(name, stream, 'table', dict(width=rows_arr.width, pattern=pat, rows=rows_arr.n))
 
     sorted_on = sort if sort in ('DNA', 'QUAL', 'QNAME') else None
-    tables = {'DNA': dna, 'QUAL': qual, 'QNAME': ctx.columns_to_rows(cols)}
+    tables = {'DNA': dna, 'QUAL': qual, 'QNAME': host.qname_rows(ctx, cols, columns)}
     keyed = {t: (t not in raw) for t in tables}
     uniq = {}
     payload = {}
@@ -1115,7 +1115,7 @@ def encode_sharded(ctx, comm, fq, sort=None, raw=None, pattern=None, pad=False, 
             else:
                 payload[t + '.key'] = g['key']
             if t == 'QNAME':                        # unique rows back to typed columns (uq.py:842-847)
-                ucols = ctx.rows_to_columns(g['uniq'], [np.dtype(m['dtype']).itemsize for m in columns])
+                ucols = host.qname_columns(ctx, g['uniq'], columns)
                 for c, meta in zip(ucols, columns):
                     res.add(meta['name'], c, 'vector', meta['dtype'])
                 g['uniq'].free()
