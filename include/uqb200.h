@@ -38,11 +38,6 @@ int         uqb_version(void);
  * on it so that callers can time the path with events recorded on the same stream. */
 int         uqb_ctx_create(int device, void* stream, uqb_ctx** out);
 void        uqb_ctx_destroy(uqb_ctx* ctx);
-/* launches that follow go to `stream` (a cudaStream_t) instead; *previous receives the stream that was installed.
- * Used for the side stream of a multi-GPU row exchange that runs next to the sort of the previous table: the caller
- * orders the streams with its own events and keeps the arrays of the side-stream work alive until they are joined.
- * max_ctas_per_sm > 0 caps the grid of the row-exchange kernels (NVLink bound) while the side stream is installed. */
-int         uqb_ctx_swap_stream(uqb_ctx* ctx, void* stream, uint32_t max_ctas_per_sm, void** previous);
 const char* uqb_last_error(const uqb_ctx* ctx);
 int         uqb_ctx_sync(uqb_ctx* ctx);
 /* number of kernels this context has launched so far (bench.py's gpu_launches) */
@@ -207,24 +202,21 @@ int uqb_add_scalar_u32(uqb_ctx* ctx, uqb_array* a, uint32_t value);   /* a[i] +=
 /* lower_bound of k host rows in a table sorted in memcmp order (splitter search of the multi-GPU sample sort) */
 int uqb_rows_lower_bound(uqb_ctx* ctx, const uqb_array* sorted_table, const uint8_t* probes_host, uint32_t k, uint64_t* out_host);
 /* partition-first sample sort (multi-GPU, replaces nothing in uq.py: the reference is single process): rows are sent
- * to rank d = number of splitter keys <= big-endian first 8 bytes of the row.  order = uint32[n] row indices grouped
- * by destination (stable), counts_host[0..nsplit] = rows per destination */
-int uqb_partition_rows(uqb_ctx* ctx, const uqb_array* table, const uint64_t* split_keys_host, uint32_t nsplit,
-                       uqb_array** order, uint64_t* counts_host);
-/* exchange buffers of the sample sort: the rows of segment d (order[first_d .. first_d + seg_counts[d])) gathered into a
- * byte array in which every segment starts at a multiple of `align` bytes (NCCL moves 16 bytes per thread only between
- * 16-byte aligned pointers); seg_offsets_host receives the byte offset of every segment */
-int uqb_gather_rows_segmented(uqb_ctx* ctx, const uqb_array* table, const uqb_array* order, uint32_t nseg,
-                              const uint64_t* seg_counts_host, uint32_t align, uqb_array** out, uint64_t* seg_offsets_host);
-/* The streaming form of the two calls above (rows of up to 224 bytes): the table is read once, sequentially.
- * uqb_partition_positions: pos = uint32[n], pos[i] = index of row i in the destination-grouped, stable order (what
- * order^-1 would be); counts_host[0..nsplit] = rows per destination.  uqb_scatter_rows_segmented: row i of `table`
- * (the partitioned table itself, or any per-record payload that has to follow it) lands at byte
- * seg_offsets[d] + (pos[i] - first row of d) * width of a byte array laid out like uqb_gather_rows_segmented's. */
+ * to rank d = number of splitter keys <= big-endian first 8 bytes of the row.  The table is read once, sequentially.
+ * pos = uint32[n], pos[i] = index of row i in the destination-grouped, stable order; counts_host[0..nsplit] = rows per
+ * destination */
 int uqb_partition_positions(uqb_ctx* ctx, const uqb_array* table, const uint64_t* split_keys_host, uint32_t nsplit,
                             uqb_array** pos, uint64_t* counts_host);
+/* exchange buffers of the sample sort: byte arrays in which every segment starts at a multiple of `align` bytes (NCCL
+ * moves 16 bytes per thread only between 16-byte aligned pointers); seg_offsets_host receives the byte offset of every
+ * segment.  uqb_scatter_rows_segmented: row i of `table` (the partitioned table itself, or any per-record payload that
+ * has to follow it) lands at byte seg_offsets[d] + (pos[i] - first row of d) * width; rows of up to 224 bytes.
+ * uqb_gather_rows_segmented: the same buffer from order = pos^-1 (rows of any width): the rows of segment d are
+ * table[order[first_d .. first_d + seg_counts[d])). */
 int uqb_scatter_rows_segmented(uqb_ctx* ctx, const uqb_array* table, const uqb_array* pos, uint32_t nseg,
                                const uint64_t* seg_counts_host, uint32_t align, uqb_array** out, uint64_t* seg_offsets_host);
+int uqb_gather_rows_segmented(uqb_ctx* ctx, const uqb_array* table, const uqb_array* order, uint32_t nseg,
+                              const uint64_t* seg_counts_host, uint32_t align, uqb_array** out, uint64_t* seg_offsets_host);
 /* device-initiated exchange: the rows of segment d go straight to the device address dst_addrs_host[d] (dense, in position
  * order) - normally the receive buffer of rank d mapped into this process (peer memory over NVLink).  The caller brackets
  * the call with its own barriers. */

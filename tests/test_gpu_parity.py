@@ -199,10 +199,12 @@ def test_sort_rows_matches_numpy_stable(ctx, n, width, alphabet):
         a.free()
 
 
-@pytest.mark.parametrize("n,width,nsplit", [(1, 9, 1), (5000, 113, 1), (70001, 38, 3), (30000, 10, 7), (9000, 4, 2), (4100, 224, 2), (3000, 3, 4)])
+@pytest.mark.parametrize("n,width,nsplit", [(1, 9, 1), (5000, 113, 1), (70001, 38, 3), (30000, 10, 7), (9000, 4, 2), (4100, 224, 2), (3000, 3, 4),
+                                           (3000, 225, 2), (2000, 788, 3), (1500, 0, 2)])
 def test_streaming_partition_equals_stable_order(ctx, n, width, nsplit):
     """uqb_partition_positions / uqb_scatter_rows_segmented (multi-GPU sample sort) against numpy: pos is the inverse of
-    the stable destination order, the byte buffer holds the rows of every destination in input order."""
+    the stable destination order, the byte buffer holds the rows of every destination in input order.  Rows the
+    scatter does not take (wider than Context.SCATTER_MAX_WIDTH, or empty) are gathered through order = pos^-1."""
     rng = np.random.default_rng(n + width)
     t = rng.integers(0, 256, size=(n, width), dtype=np.uint8)
     if n > 100:
@@ -220,7 +222,13 @@ def test_streaming_partition_equals_stable_order(ctx, n, width, nsplit):
     pos, counts = ctx.partition_positions(d, splits)
     assert counts == counts_w.tolist()
     assert np.array_equal(pos.download(dtype=np.uint32).reshape(-1), pos_w)
-    buf, offs = ctx.scatter_rows_segmented(d, pos, counts, 128)
+    if 0 < width <= ctx.SCATTER_MAX_WIDTH:
+        buf, offs = ctx.scatter_rows_segmented(d, pos, counts, 128)
+    else:
+        iota = ctx.upload(np.arange(n, dtype=np.uint32))
+        order = ctx.scatter_u32(iota, pos)
+        buf, offs = ctx.gather_rows_segmented(d, order, counts, 128)
+        iota.free(); order.free()
     got = buf.download().reshape(-1)
     first = 0
     for k, c in enumerate(counts):

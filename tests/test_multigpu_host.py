@@ -168,7 +168,8 @@ def test_shared_memory_board_matches_gloo(use_board):
 
 # ---- partition-first sample sort: the host side of global_unique, emulated with numpy ---------------------------
 def _emu_partition(rows, split_keys):
-    """contract of uqb_partition_rows: dest = number of splitter keys <= big-endian first 8 bytes; stable grouping"""
+    """contract of uqb_partition_positions: dest = number of splitter keys <= big-endian first 8 bytes; stable grouping
+    (order = pos^-1)"""
     key = mg.row_key64(rows)
     dest = np.searchsorted(np.asarray(split_keys, dtype=np.uint64), key, side="right")
     order = np.argsort(dest, kind="stable")

@@ -1,8 +1,8 @@
 """The sharded (one container from W ranks) encode and decode on ONE GPU: W emulated ranks (host threads, one context
 each, uq_b200.multigpu.LocalComm) run exactly the code the NCCL ranks run - merged statistics, partition-first sample
-sort (uqb_partition_rows, uqb_gather_rows_segmented, uqb_compact_segments, uqb_scatter_u32), global order, per-rank
-layouts and their placement, sharded decode - and the result must equal the single-GPU encode of the whole file
-member by member.  SURVEY section 4(d) / 8(e)."""
+sort (uqb_partition_positions, uqb_scatter_rows_segmented / uqb_gather_rows_segmented, uqb_compact_segments,
+uqb_scatter_u32), global order, per-rank layouts and their placement, sharded decode - and the result must equal the
+single-GPU encode of the whole file member by member.  SURVEY section 4(d) / 8(e)."""
 import json
 
 import numpy as np
@@ -24,6 +24,9 @@ CASES = [
     ("illumina", 7000, 30, dict()),
     ("genome", 9000, 40, dict(sort="DNA", pattern=["2.2", "1.1"])),
     ("genome", 9000, 40, dict(sort="QNAME", raw=["QUAL"], pattern=["3.1", "3.2"])),
+    # variable-length reads of up to 900 bases: DNA and QUAL rows wider than Context.SCATTER_MAX_WIDTH
+    ("ont", 6000, (50, 900), dict(sort="QUAL")),
+    ("ont", 6000, (50, 900), dict(sort="QNAME", raw=["DNA", "QUAL"])),
 ]
 
 
@@ -104,7 +107,7 @@ def test_sharded_encode_through_peer_window(ctx, world, case):
     assert_members_equal(got, want, "window %s world=%d %r" % (kind, world, kw))
 
 
-@pytest.mark.parametrize("case", [0, 2, 3])
+@pytest.mark.parametrize("case", [0, 2, 3, 8, 9])
 def test_sharded_encode_merge_variant(ctx, case):
     """the skew-proof variant (local sort first, only locally unique rows travel) gives the same container"""
     from uq_b200 import host

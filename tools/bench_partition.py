@@ -1,6 +1,6 @@
 #!/usr/bin/env python3
-"""Diagnostics: the two ways of grouping the rows of a packed table by destination rank (multi-GPU sample sort) on one device:
-partition_rows + gather_rows_segmented (radix pass + gathers) against partition_positions + scatter_rows_segmented (streaming)."""
+"""Diagnostics: grouping the rows of a packed table by destination rank (multi-GPU sample sort) on one device,
+partition_positions + scatter_rows_segmented, per kernel, for 2 and 8 destinations."""
 import json, os, sys
 import numpy as np
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
@@ -18,20 +18,14 @@ for name in ("dna", "qual"):
     for world in (2, 8):
         samples = multigpu._sample_rows(ctx, t, 1024)
         keys = np.sort(multigpu.row_key64(multigpu.pick_splitters(samples, world)))
-        for mode in ("gather", "scatter"):
-            for it in range(2):
-                ctx.sync(); ctx.timing(True); ctx.timing_reset()
-                if mode == "gather":
-                    order, counts = ctx.partition_rows(t, keys)
-                    buf, offs = ctx.gather_rows_segmented(t, order, counts, 128)
-                    order.free()
-                else:
-                    pos, counts = ctx.partition_positions(t, keys)
-                    buf, offs = ctx.scatter_rows_segmented(t, pos, counts, 128)
-                    pos.free()
-                ctx.sync()
-                rep = ctx.timing_report()
-                buf.free()
-            out["%s W=%d %s" % (name, world, mode)] = {"ms": round(sum(v[1] for v in rep.values()), 3),
-                                                       "kernels": {k: round(v[1], 3) for k, v in rep.items() if v[1] > 0.05}}
+        for it in range(2):
+            ctx.sync(); ctx.timing(True); ctx.timing_reset()
+            pos, counts = ctx.partition_positions(t, keys)
+            buf, offs = ctx.scatter_rows_segmented(t, pos, counts, 128)
+            pos.free()
+            ctx.sync()
+            rep = ctx.timing_report()
+            buf.free()
+        out["%s W=%d" % (name, world)] = {"ms": round(sum(v[1] for v in rep.values()), 3),
+                                          "kernels": {k: round(v[1], 3) for k, v in rep.items() if v[1] > 0.05}}
 print(json.dumps(out, indent=1))

@@ -76,7 +76,6 @@ SIGNATURES = {
     "uqb_version": (C.c_int, []),
     "uqb_ctx_create": (C.c_int, [C.c_int, P, PP]),
     "uqb_ctx_destroy": (None, [P]),
-    "uqb_ctx_swap_stream": (C.c_int, [P, P, C.c_uint32, PP]),
     "uqb_last_error": (C.c_char_p, [P]),
     "uqb_ctx_sync": (C.c_int, [P]),
     "uqb_ctx_launch_count": (C.c_uint64, [P]),
@@ -114,7 +113,6 @@ SIGNATURES = {
     "uqb_qname_dict_first": (C.c_int, [P, P, C.c_uint32, P, C.c_uint64]),
     "uqb_rows_lower_bound": (C.c_int, [P, P, P, C.c_uint32, P]),
     "uqb_add_scalar_u32": (C.c_int, [P, P, C.c_uint32]),
-    "uqb_partition_rows": (C.c_int, [P, P, P, C.c_uint32, PP, P]),
     "uqb_scatter_u32": (C.c_int, [P, P, P, PP]),
     "uqb_gather_rows_segmented": (C.c_int, [P, P, P, C.c_uint32, P, C.c_uint32, PP, P]),
     "uqb_compact_segments": (C.c_int, [P, P, C.c_uint32, P, P, C.c_uint32, PP]),

@@ -41,7 +41,6 @@ struct uqb_ctx {
     uint64_t bytes_in_use = 0;
     int sm_count = UQB_SM_COUNT;
     std::vector<const void*> copies_in_flight;   // sources of async device->host copies queued since the last copy sync
-    unsigned side_ctas_per_sm = 0;           // > 0 while a side stream is installed (uqb_ctx_swap_stream): CTA cap of the exchange kernels
     // pinned scratch for small device->host read-backs
     void* pinned = nullptr;
     size_t pinned_bytes = 0;

@@ -147,17 +147,6 @@ extern "C" int uqb_ctx_create(int device, void* stream, uqb_ctx** out) {
     return 0;
 }
 
-// Install another stream for the launches that follow (the side stream of an exchange that runs next to the sort of the
-// previous table); the caller orders the two streams with its own events.  max_ctas_per_sm > 0 caps the grid of the
-// row-exchange kernels, which are NVLink bound and should leave the SMs to the kernels of the main stream.
-extern "C" int uqb_ctx_swap_stream(uqb_ctx* ctx, void* stream, uint32_t max_ctas_per_sm, void** previous) {
-    if (!stream) return uqb_fail(ctx, "swap_stream: a stream is required");
-    if (previous) *previous = (void*)ctx->stream;
-    ctx->stream = (cudaStream_t)stream;
-    ctx->side_ctas_per_sm = max_ctas_per_sm;
-    return 0;
-}
-
 extern "C" void uqb_ctx_destroy(uqb_ctx* ctx) {
     if (!ctx) return;
     cudaSetDevice(ctx->device);

@@ -1,8 +1,8 @@
 // Multi-GPU sample sort, streaming partition (SURVEY section 8e): rows leave for the rank whose key range holds their first
-// 8 bytes.  uqb_partition_rows + uqb_gather_rows_segmented (sort.cu) do this as "stable radix pass over (destination,
-// index), then gather table[order] segment by segment": every segment reads every W-th row of the table, i.e. whole
-// 128-byte lines for a 113-byte row, and the global ids come back through a random 4-byte scatter.  Here the table is
-// read ONCE, sequentially, and written as W sequential streams:
+// 8 bytes, so rows that agree in those bytes (identical rows in particular) meet on one rank, and the ranks' ranges are
+// ordered like the rows: each rank sorts / uniques what it receives on its own.  A stable radix pass over (destination,
+// index) followed by a gather of table[order] segment by segment would read every W-th row of the table per segment, i.e.
+// whole 128-byte lines for a 113-byte row.  Here the table is read ONCE, sequentially, and written as W sequential streams:
 //   k_pp_count   destination of every row (from the round-0 sort keys the packer wrote, or from the row) + per-tile counts
 //   k_pp_scan    per destination: exclusive scan of the tile counts, totals
 //   k_pp_pos     pos[i] = index of row i in the destination-grouped, stable order (first[d] + rows of d before i)
@@ -11,7 +11,6 @@
 //                staged in shared memory with 16-byte loads and leaves in one contiguous run per destination.
 // The same pos moves every per-record payload of global_order, and brings the global ids back with a gather.
 #include "common.cuh"
-#include <cstdlib>
 
 #define PP_THREADS 256
 #define PP_TILE 2048
@@ -164,10 +163,7 @@ __device__ __forceinline__ uint32_t pp_seg_of(const pp_segs& S, uint64_t j) {
 // 770 GB/s for large aligned stores.  SUB lanes move one row into the image (32 / SUB rows per warp step): 8 lanes for
 // rows of up to 32 bytes, 16 up to 64, 32 beyond.
 #define SRR_MAXD 64
-// TMA = true: the 16-byte aligned interior of every run leaves shared memory as ONE bulk store (cp.async.bulk.global.shared,
-// issued by the thread that owns the destination); the TMA unit does the address generation and keeps more bytes in flight
-// towards a peer than 16-byte stores of the SM do.
-template <int SUB, bool TMA>
+template <int SUB>
 __global__ void __launch_bounds__(SR_THREADS) k_scatter_rows_runs(const uint8_t* __restrict__ rows, uint64_t n, uint32_t width,
                                                                  const uint32_t* __restrict__ pos, pp_segs segs, uint8_t* __restrict__ out) {
     extern __shared__ __align__(16) uint8_t srr_smem[];                 // [input tile | output image]
@@ -181,11 +177,9 @@ __global__ void __launch_bounds__(SR_THREADS) k_scatter_rows_runs(const uint8_t*
     uint8_t* img = srr_smem + in_bytes;
     const uint32_t* in32 = reinterpret_cast<const uint32_t*>(in);
     const uint64_t ntiles = (n + SR_THREADS - 1) / SR_THREADS;
-    bool bulk_pending = false;
     for (uint64_t t = blockIdx.x; t < ntiles; t += gridDim.x) {
         const uint64_t r0 = t * SR_THREADS;
         const uint32_t nr = (uint32_t)(n - r0 < SR_THREADS ? n - r0 : SR_THREADS);
-        if (TMA && bulk_pending) { asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory"); bulk_pending = false; }   // the image has been read
         __syncthreads();
         if (tid < segs.n) { cnt[tid] = 0; minpos[tid] = 0xFFFFFFFFu; }
         const uint4* src = reinterpret_cast<const uint4*>(rows + r0 * width);
@@ -233,28 +227,14 @@ __global__ void __launch_bounds__(SR_THREADS) k_scatter_rows_runs(const uint8_t*
         }
         __syncthreads();
         // image runs -> global
-        if (TMA && tid < segs.n && cnt[tid]) {
-            const uint32_t i0 = ioff[tid], i1 = i0 + cnt[tid] * width;
-            const uint32_t a = (i0 + 15u) & ~15u, b = i1 & ~15u;
-            if (a < b) {
-                uint8_t* G = reinterpret_cast<uint8_t*>((uintptr_t)gaddr[tid]) - i0;
-                asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-                asm volatile("cp.async.bulk.global.shared::cta.bulk_group [%0], [%1], %2;" ::"l"(G + a),
-                             "r"((uint32_t)__cvta_generic_to_shared(img + a)), "r"(b - a)
-                             : "memory");
-                asm volatile("cp.async.bulk.commit_group;" ::: "memory");
-                bulk_pending = true;
-            }
-        }
         for (uint32_t k = 0; k < segs.n; k++) {
             if (!cnt[k]) continue;
             const uint32_t i0 = ioff[k], i1 = i0 + cnt[k] * width;
             const uint32_t a = (i0 + 15u) & ~15u, b = i1 & ~15u;
             uint8_t* G = reinterpret_cast<uint8_t*>((uintptr_t)gaddr[k]) - i0;     // image offset x <-> G + x
             if (a <= b) {
-                if (!TMA)
-                    for (uint32_t x = a + 16u * tid; x < b; x += 16u * SR_THREADS)
-                        *reinterpret_cast<uint4*>(G + x) = *reinterpret_cast<const uint4*>(img + x);
+                for (uint32_t x = a + 16u * tid; x < b; x += 16u * SR_THREADS)
+                    *reinterpret_cast<uint4*>(G + x) = *reinterpret_cast<const uint4*>(img + x);
                 if (tid < a - i0) G[i0 + tid] = img[i0 + tid];
                 if (tid < i1 - b) G[b + tid] = img[b + tid];
             } else {
@@ -262,7 +242,6 @@ __global__ void __launch_bounds__(SR_THREADS) k_scatter_rows_runs(const uint8_t*
             }
         }
     }
-    if (TMA && bulk_pending) asm volatile("cp.async.bulk.wait_group 0;" ::: "memory");     // the last bulk stores have landed
 }
 
 template <typename T>
@@ -284,46 +263,34 @@ static int scatter_rows_impl(uqb_ctx* ctx, const uqb_array* table, const uqb_arr
     if (n == 0) return 0;
     if ((reinterpret_cast<uintptr_t>(table->d) & 15u) != 0) return uqb_fail(ctx, "scatter_rows: the table must be 16-byte aligned");
     const uint64_t ab = n * (2ull * w + 4);
-    const unsigned iw = ctx->side_ctas_per_sm ? 2u * ctx->side_ctas_per_sm : 8u;      // waves of the item kernels
     if (w == 4) {
-        UQB_LAUNCH_B(ab, k_scatter_items_by_pos<uint32_t>, uqb_grid(ctx, n, SR_THREADS, iw), SR_THREADS, 0, (const uint32_t*)table->d, n, (const uint32_t*)pos->d, S, o);
+        UQB_LAUNCH_B(ab, k_scatter_items_by_pos<uint32_t>, uqb_grid(ctx, n, SR_THREADS, 8), SR_THREADS, 0, (const uint32_t*)table->d, n, (const uint32_t*)pos->d, S, o);
     } else if (w == 8) {
-        UQB_LAUNCH_B(ab, k_scatter_items_by_pos<uint64_t>, uqb_grid(ctx, n, SR_THREADS, iw), SR_THREADS, 0, (const uint64_t*)table->d, n, (const uint32_t*)pos->d, S, o);
+        UQB_LAUNCH_B(ab, k_scatter_items_by_pos<uint64_t>, uqb_grid(ctx, n, SR_THREADS, 8), SR_THREADS, 0, (const uint64_t*)table->d, n, (const uint32_t*)pos->d, S, o);
     } else if (w == 2) {
-        UQB_LAUNCH_B(ab, k_scatter_items_by_pos<uint16_t>, uqb_grid(ctx, n, SR_THREADS, iw), SR_THREADS, 0, (const uint16_t*)table->d, n, (const uint32_t*)pos->d, S, o);
+        UQB_LAUNCH_B(ab, k_scatter_items_by_pos<uint16_t>, uqb_grid(ctx, n, SR_THREADS, 8), SR_THREADS, 0, (const uint16_t*)table->d, n, (const uint32_t*)pos->d, S, o);
     } else if (w == 1) {
-        UQB_LAUNCH_B(ab, k_scatter_items_by_pos<uint8_t>, uqb_grid(ctx, n, SR_THREADS, iw), SR_THREADS, 0, (const uint8_t*)table->d, n, (const uint32_t*)pos->d, S, o);
+        UQB_LAUNCH_B(ab, k_scatter_items_by_pos<uint8_t>, uqb_grid(ctx, n, SR_THREADS, 8), SR_THREADS, 0, (const uint8_t*)table->d, n, (const uint32_t*)pos->d, S, o);
     } else {
-        static const bool tma = [] { const char* e = getenv("UQB_SCATTER_TMA"); return e && e[0] == '1'; }();
         // contiguous runs per destination, regrouped in shared memory
         const size_t in_bytes = ((size_t)SR_THREADS * w + 32 + 15) & ~(size_t)15;
         const size_t smem = in_bytes + (size_t)SR_THREADS * w + 32 * (size_t)S.n + 64;
         const unsigned per_sm = (unsigned)(200 * 1024 / (smem + 5 * 1024)) ? (unsigned)(200 * 1024 / (smem + 5 * 1024)) : 1u;
-        unsigned ctas = per_sm > 8 ? 8 : per_sm;
-        if (ctx->side_ctas_per_sm && ctas > ctx->side_ctas_per_sm) ctas = ctx->side_ctas_per_sm;
+        const unsigned ctas = per_sm > 8 ? 8 : per_sm;
         const uint64_t ntiles = (n + SR_THREADS - 1) / SR_THREADS, cap = (uint64_t)ctx->sm_count * ctas;
         const unsigned grid = (unsigned)(ntiles < cap ? ntiles : cap);
         if (w <= 32) {
-            auto k_scatter_rows_runs_8 = k_scatter_rows_runs<8, false>;
-            auto k_scatter_rows_tma_8 = k_scatter_rows_runs<8, true>;
+            auto k_scatter_rows_runs_8 = k_scatter_rows_runs<8>;
             UQB_CUDA(cudaFuncSetAttribute(k_scatter_rows_runs_8, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-            UQB_CUDA(cudaFuncSetAttribute(k_scatter_rows_tma_8, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-            if (tma) UQB_LAUNCH_B(ab, k_scatter_rows_tma_8, grid, SR_THREADS, smem, (const uint8_t*)table->d, n, w, (const uint32_t*)pos->d, S, o);
-            else UQB_LAUNCH_B(ab, k_scatter_rows_runs_8, grid, SR_THREADS, smem, (const uint8_t*)table->d, n, w, (const uint32_t*)pos->d, S, o);
+            UQB_LAUNCH_B(ab, k_scatter_rows_runs_8, grid, SR_THREADS, smem, (const uint8_t*)table->d, n, w, (const uint32_t*)pos->d, S, o);
         } else if (w <= 64) {
-            auto k_scatter_rows_runs_16 = k_scatter_rows_runs<16, false>;
-            auto k_scatter_rows_tma_16 = k_scatter_rows_runs<16, true>;
+            auto k_scatter_rows_runs_16 = k_scatter_rows_runs<16>;
             UQB_CUDA(cudaFuncSetAttribute(k_scatter_rows_runs_16, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-            UQB_CUDA(cudaFuncSetAttribute(k_scatter_rows_tma_16, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-            if (tma) UQB_LAUNCH_B(ab, k_scatter_rows_tma_16, grid, SR_THREADS, smem, (const uint8_t*)table->d, n, w, (const uint32_t*)pos->d, S, o);
-            else UQB_LAUNCH_B(ab, k_scatter_rows_runs_16, grid, SR_THREADS, smem, (const uint8_t*)table->d, n, w, (const uint32_t*)pos->d, S, o);
+            UQB_LAUNCH_B(ab, k_scatter_rows_runs_16, grid, SR_THREADS, smem, (const uint8_t*)table->d, n, w, (const uint32_t*)pos->d, S, o);
         } else {
-            auto k_scatter_rows_runs_32 = k_scatter_rows_runs<32, false>;
-            auto k_scatter_rows_tma_32 = k_scatter_rows_runs<32, true>;
+            auto k_scatter_rows_runs_32 = k_scatter_rows_runs<32>;
             UQB_CUDA(cudaFuncSetAttribute(k_scatter_rows_runs_32, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-            UQB_CUDA(cudaFuncSetAttribute(k_scatter_rows_tma_32, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-            if (tma) UQB_LAUNCH_B(ab, k_scatter_rows_tma_32, grid, SR_THREADS, smem, (const uint8_t*)table->d, n, w, (const uint32_t*)pos->d, S, o);
-            else UQB_LAUNCH_B(ab, k_scatter_rows_runs_32, grid, SR_THREADS, smem, (const uint8_t*)table->d, n, w, (const uint32_t*)pos->d, S, o);
+            UQB_LAUNCH_B(ab, k_scatter_rows_runs_32, grid, SR_THREADS, smem, (const uint8_t*)table->d, n, w, (const uint32_t*)pos->d, S, o);
         }
     }
     return 0;

@@ -1336,60 +1336,7 @@ extern "C" int uqb_rows_lower_bound(uqb_ctx* ctx, const uqb_array* sorted_table,
     return 0;
 }
 
-// ---- multi-GPU sample sort, partition-first variant ------------------------------------------------
-// Destination rank of every row from its first 8 bytes: dest = number of splitter keys <= be64(row[0:8]).
-// Rows that agree in their first 8 bytes (in particular identical rows) always share a destination, and the
-// destinations are ordered like the rows, so each rank can sort / unique what it receives on its own.
-#define PD_MAX 64
-struct pd_split { uint64_t key[PD_MAX]; uint32_t n; };
-
-__global__ void __launch_bounds__(ST) k_partition_dest(const uint8_t* __restrict__ rows, uint64_t n, uint32_t width, pd_split sp,
-                                                      uint64_t* __restrict__ key, uint32_t* __restrict__ val, unsigned long long* __restrict__ counts) {
-    __shared__ unsigned int cnt[PD_MAX + 1];
-    if (threadIdx.x <= PD_MAX) cnt[threadIdx.x] = 0;
-    __syncthreads();
-    const uint64_t i = (uint64_t)blockIdx.x * ST + threadIdx.x;
-    if (i < n) {
-        const uint64_t k = load_be64(rows + i * width, width < 8 ? width : 8);
-        uint32_t d = 0;
-        for (uint32_t j = 0; j < sp.n; j++) d += sp.key[j] <= k ? 1u : 0u;
-        key[i] = d;
-        val[i] = (uint32_t)i;
-        atomicAdd(&cnt[d], 1u);
-    }
-    __syncthreads();
-    if (threadIdx.x <= sp.n && cnt[threadIdx.x]) atomicAdd(&counts[threadIdx.x], (unsigned long long)cnt[threadIdx.x]);
-}
-
-// order[j] = rows grouped by destination (stable inside a destination), counts_host[d] = rows going to rank d
-extern "C" int uqb_partition_rows(uqb_ctx* ctx, const uqb_array* table, const uint64_t* split_keys_host, uint32_t nsplit,
-                                  uqb_array** order, uint64_t* counts_host) {
-    if (nsplit > PD_MAX) return uqb_fail(ctx, "partition_rows: more than %d splitters", PD_MAX);
-    const uint64_t n = table->n;
-    if (n >= (1ull << 32)) return uqb_fail(ctx, "partition_rows: %llu rows exceed the 32-bit index range", (unsigned long long)n);
-    UQB_TRY(uqb_new_array(ctx, n, 4, order));
-    for (uint32_t d = 0; d <= nsplit; d++) counts_host[d] = 0;
-    if (n == 0) return 0;
-    pd_split sp;
-    sp.n = nsplit;
-    for (uint32_t j = 0; j < nsplit; j++) sp.key[j] = split_keys_host[j];
-    unsigned long long* d_counts;
-    UQB_TRY(uqb_dalloc_t(ctx, &d_counts, PD_MAX + 1));
-    UQB_CUDA(cudaMemsetAsync(d_counts, 0, (PD_MAX + 1) * 8, ctx->stream));
-    uqb_sortbuf sb;
-    UQB_TRY(uqb_sortbuf_alloc(ctx, &sb, n, false));
-    UQB_LAUNCH_B(n * ((table->width < 8 ? table->width : 8) + 12), k_partition_dest, uqb_blocks(n, ST), ST, 0, (const uint8_t*)table->d, n,
-                 table->width, sp, sb.key[0], sb.val[0], d_counts);
-    UQB_TRY(uqb_radix_sort(ctx, &sb, n, false));                 // one 8-bit pass: only the low bits of the key vary
-    UQB_CUDA(cudaMemcpyAsync((*order)->d, sb.val[sb.cur], n * 4, cudaMemcpyDeviceToDevice, ctx->stream));
-    unsigned long long hc[PD_MAX + 1];
-    UQB_TRY(uqb_readback(ctx, hc, d_counts, (PD_MAX + 1) * 8));
-    for (uint32_t d = 0; d <= nsplit; d++) counts_host[d] = hc[d];
-    UQB_TRY(uqb_sortbuf_free(ctx, &sb));
-    UQB_TRY(uqb_dfree(ctx, d_counts, (PD_MAX + 1) * 8));
-    return 0;
-}
-
+// ---- multi-GPU sample sort: exchange buffers (the partition is uqb_partition_positions, partition.cu) ------------
 // Row exchange buffers: NCCL's send/recv path only moves 16 bytes per thread when both user pointers are 16-byte
 // aligned, and the per-peer segments of a table of 113-byte rows start anywhere.  The rows of segment d
 // (order[first_d .. first_d + count_d)) are therefore gathered into a byte buffer in which every segment starts at a

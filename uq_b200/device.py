@@ -1,6 +1,5 @@
 """Thin object wrappers over the C ABI (include/uqb200.h).  No computation happens here: every method
 is one call into libuqb200.so; numpy is used only as host memory."""
-import contextlib
 import ctypes as C
 
 import numpy as np
@@ -50,17 +49,6 @@ class Context:
 
     def sync(self):
         self.check(self.lib.uqb_ctx_sync(self.h))
-
-    @contextlib.contextmanager
-    def on_stream(self, stream, max_ctas_per_sm=0):
-        """launches inside the block go to `stream` (raw cudaStream_t) instead of the context's stream; the caller orders
-        the two streams with events and keeps the arrays of that work alive until the streams are joined"""
-        prev = C.c_void_p()
-        self.check(self.lib.uqb_ctx_swap_stream(self.h, C.c_void_p(stream), int(max_ctas_per_sm), C.byref(prev)))
-        try:
-            yield
-        finally:
-            self.check(self.lib.uqb_ctx_swap_stream(self.h, prev, 0, None))
 
     @property
     def launches(self):
@@ -142,15 +130,6 @@ class Context:
     def add_scalar_u32(self, arr, value):
         self.check(self.lib.uqb_add_scalar_u32(self.h, arr.h, int(value)))
 
-    def partition_rows(self, table, split_keys):
-        """rows -> destination ranks by their big-endian first 8 bytes (dest = number of split_keys <= key).
-        -> (order: uint32[n] row indices grouped by destination, stable; counts per destination)"""
-        keys = np.ascontiguousarray(split_keys, dtype=np.uint64)
-        counts = np.zeros(len(keys) + 1, dtype=np.uint64)
-        h = C.c_void_p()
-        self.check(self.lib.uqb_partition_rows(self.h, table.h, _ptr(keys), len(keys), C.byref(h), _ptr(counts)))
-        return DeviceArray(self, h), [int(c) for c in counts]
-
     def gather_rows_segmented(self, table, order, seg_counts, align=128):
         """rows table[order[...]] gathered segment by segment into a byte array whose segments start at multiples of
         `align` bytes -> (DeviceArray of bytes, byte offset of every segment)"""
@@ -163,8 +142,8 @@ class Context:
     SCATTER_MAX_WIDTH = 224
 
     def partition_positions(self, table, split_keys):
-        """streaming form of partition_rows: -> (pos: uint32[n], pos[i] = index of row i in the destination-grouped stable
-        order; counts per destination)"""
+        """rows -> destination ranks by their big-endian first 8 bytes (dest = number of split_keys <= key).
+        -> (pos: uint32[n], pos[i] = index of row i in the destination-grouped stable order; counts per destination)"""
         keys = np.ascontiguousarray(split_keys, dtype=np.uint64)
         counts = np.zeros(len(keys) + 1, dtype=np.uint64)
         h = C.c_void_p()

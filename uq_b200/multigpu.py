@@ -188,23 +188,21 @@ def trace_dump():
 # communication
 # ------------------------------------------------------------------------------------------------
 def _segmented(ctx, table, router, seg_counts, align=128):
-    """the rows of `table` grouped by destination in a byte buffer with aligned segments.  router = ("pos", pos) from
-    uqb_partition_positions (streaming scatter, rows of up to Context.SCATTER_MAX_WIDTH bytes) or ("order", order) from
-    uqb_partition_rows (gather)."""
-    kind, arr = router
-    if kind == "pos" and 0 < table.width <= ctx.SCATTER_MAX_WIDTH:
-        return ctx.scatter_rows_segmented(table, arr, seg_counts, align)
-    if kind == "pos":                                    # a wide payload behind a narrow sorted-on table: order = pos^-1
-        if len(router) < 3:
-            iota = ctx.upload(np.arange(arr.n, dtype=np.uint32))
-            router.append(ctx.scatter_u32(iota, arr))
-            iota.free()
-        return ctx.gather_rows_segmented(table, router[2], seg_counts, align)
-    return ctx.gather_rows_segmented(table, arr, seg_counts, align)
+    """the rows of `table` grouped by destination in a byte buffer with aligned segments.  router = [pos] from
+    uqb_partition_positions: rows of 1 .. Context.SCATTER_MAX_WIDTH bytes are scattered by pos (streaming), other widths
+    are gathered through order = pos^-1, which is computed on first use and kept as router[1]."""
+    pos = router[0]
+    if 0 < table.width <= ctx.SCATTER_MAX_WIDTH:
+        return ctx.scatter_rows_segmented(table, pos, seg_counts, align)
+    if len(router) < 2:
+        iota = ctx.upload(np.arange(pos.n, dtype=np.uint32))
+        router.append(ctx.scatter_u32(iota, pos))
+        iota.free()
+    return ctx.gather_rows_segmented(table, router[1], seg_counts, align)
 
 
 def _router_free(router):
-    for a in router[1:]:
+    for a in router:
         a.free()
 
 
@@ -237,10 +235,9 @@ def open_peer_window(dist, device, stream, nbytes, slots=3):
     buf = symm_mem.empty(int(nbytes), dtype=torch.uint8, device=device)
     hdl = symm_mem.rendezvous(buf, dist.group.WORLD)
 
-    def barrier(on=None):
-        s = on if on is not None else stream
-        if s is not None:
-            with torch.cuda.stream(s):
+    def barrier():
+        if stream is not None:
+            with torch.cuda.stream(stream):
                 hdl.barrier(channel=0)
         else:
             hdl.barrier(channel=0)
@@ -253,7 +250,7 @@ def _p2p_plan(comm, ctx, table, router, count_table):
     peer window, else None.  Decided from the count table alone, so every rank decides alike."""
     win = getattr(comm, "window", None)
     w = table.width
-    if win is None or count_table is None or router[0] != "pos" or not (0 < w <= ctx.SCATTER_MAX_WIDTH):
+    if win is None or count_table is None or not (0 < w <= ctx.SCATTER_MAX_WIDTH):
         return None
     world = comm.world
     if max(sum(count_table[s][d] for s in range(world)) for d in range(world)) * w > win.slot_bytes:
@@ -265,43 +262,9 @@ def _p2p_plan(comm, ctx, table, router, count_table):
 def _p2p_exchange(comm, ctx, table, router, send_counts, recv_counts, plan):
     base, addrs = plan
     recv = ctx.wrap(comm.window.ptrs[comm.rank] + base, sum(recv_counts), table.width)
-    side = getattr(comm, "side", None)
-    if side is None or comm.stream is None or _TRACE["on"]:
-        comm.window.barrier()                            # nobody reads what the slot held before
-        ctx.scatter_rows_to(table, router[1], send_counts, addrs)
-        return dict(p2p=True, recv=recv)
-    # The stores into the peers' memory are NVLink bound and need few SMs: they run on a side stream (high priority, a
-    # capped grid) next to whatever the context's stream does meanwhile - the partition of the next table, the sort of
-    # the previous one.  Both barriers of the exchange sit on the side stream; it starts after everything queued so far
-    # on the context's stream (rows and positions written, the slot's previous contents consumed), and
-    # exchange_rows_wait joins it back.  `keep`: what the side-stream kernel reads stays alive until then.
-    if comm.exchange_mode == "dma":
-        # Copy-engine form: one streaming pass groups the rows by destination in local HBM (context stream, HBM bound);
-        # the per-destination segments then leave as device-to-device copies on the side stream - no SM is involved, so
-        # the transfer runs under the sort of the previous table at full speed.
-        w = table.width
-        send_pad, soffs = ctx.scatter_rows_segmented(table, router[1], send_counts, 128)
-        src0 = send_pad.device_ptr.value or 0
-        side.wait_stream(comm.stream)
-        comm.window.barrier(side)
-        with ctx.on_stream(side.cuda_stream):
-            for k in range(comm.world):
-                d = (comm.rank + 1 + k) % comm.world         # every rank starts with another destination
-                nb = int(send_counts[d]) * w
-                if nb:
-                    view = ctx.wrap(addrs[d], nb, 1)
-                    ctx.copy_in(view, 0, src0 + int(soffs[d]), nb)
-                    view.free()
-        comm.window.barrier(side)                        # every rank's rows have landed ...
-        return dict(p2p=True, side=True, recv=recv, landed=side.record_event(), keep=(send_pad,), free_after=(send_pad,))
-    side.wait_stream(comm.stream)
-    comm.window.barrier(side)
-    with ctx.on_stream(side.cuda_stream, comm.side_ctas):
-        ctx.scatter_rows_to(table, router[1], send_counts, addrs)
-    comm.window.barrier(side)
-    # ... and the event marks that point of the side stream: the context's stream will wait for THIS exchange only, not
-    # for the next table's exchange that is queued behind it
-    return dict(p2p=True, side=True, recv=recv, landed=side.record_event(), keep=(table, router[1]))
+    comm.window.barrier()                                # nobody reads what the slot held before
+    ctx.scatter_rows_to(table, router[0], send_counts, addrs)
+    return dict(p2p=True, recv=recv)
 
 
 class ShmBoard:
@@ -382,9 +345,6 @@ class Comm:
         never blocks around them; without it every exchange is bracketed by host synchronisations."""
         self.dist, self.device, self.stream = dist, device, stream
         self.window = None                               # PeerWindow: row exchanges as direct stores into the peers' memory
-        self.side = None                                 # torch.cuda.Stream for the peer-window stores (see _p2p_exchange)
-        self.side_ctas = 1                               # CTAs per SM of the exchange kernels on the side stream
-        self.exchange_mode = "stores"                    # "stores": uqb_scatter_rows_to; "dma": local grouping + copy engines
         self.rank = dist.get_rank() if dist else 0
         self.world = dist.get_world_size() if dist else 1
         # the small object collectives run over gloo next to NCCL: queued on the NCCL communicator they would wait
@@ -528,12 +488,6 @@ class Comm:
         return dict(work=work, send=send_pad, recv=recv_pad, roffs=roffs, recv_counts=list(recv_counts), width=w)
 
     def exchange_rows_wait(self, ctx, ex):
-        if ex.get("side"):
-            self.stream.wait_event(ex["landed"])
-            ex.pop("keep", None)
-            for a in ex.pop("free_after", ()):           # stream ordered: reused only after the join above
-                a.free()
-            return ex["recv"]
         if ex.get("p2p"):
             self.window.barrier()                        # every rank's rows have landed
             return ex["recv"]
@@ -566,8 +520,8 @@ class _Repeated:
 # ------------------------------------------------------------------------------------------------
 # W ranks on ONE device (SURVEY section 4d): every rank is a host thread with its own context (stream, arena); the
 # collectives are barriers over shared Python slots and device->device copies out of the peers' buffers.  Everything
-# else - uqb_partition_rows, uqb_gather_rows_segmented, uqb_compact_segments, uqb_scatter_u32, the merges, global_order
-# - is the code the NCCL ranks run, so the single-GPU test box exercises the whole sharded path.
+# else - uqb_partition_positions, the segmented exchange buffers, uqb_compact_segments, the merges, global_order - is the
+# code the NCCL ranks run, so the single-GPU test box exercises the whole sharded path.
 # ------------------------------------------------------------------------------------------------
 class LocalGroup:
     def __init__(self, world):
@@ -763,12 +717,8 @@ def global_unique_begin(ctx, comm, table, want_perm=False, gathered=None):
         gathered = comm.all_gather_object((samples, table.n))
     _mark(ctx, comm, "gu.sample")
     splitters = pick_splitters(np.concatenate([g[0] for g in gathered]), comm.world)
-    if 0 < table.width <= ctx.SCATTER_MAX_WIDTH and os.environ.get("UQB_MG_GATHER") != "1":
-        pos, send_counts = ctx.partition_positions(table, np.sort(row_key64(splitters)))      # one sequential sweep
-        router = ["pos", pos]
-    else:
-        order, send_counts = ctx.partition_rows(table, np.sort(row_key64(splitters)))
-        router = ["order", order]
+    pos, send_counts = ctx.partition_positions(table, np.sort(row_key64(splitters)))      # one sequential sweep
+    router = [pos]
     send_counts += [0] * (comm.world - len(send_counts))
     count_table = comm.all_gather_object(list(map(int, send_counts)))            # one collective: who sends how much to whom
     recv_counts = [count_table[src][comm.rank] for src in range(comm.world)]
@@ -793,7 +743,7 @@ def global_unique_end(ctx, comm, st):
     recv = st["recv"] if st["recv"] is not None else comm.exchange_rows_wait(ctx, st["ex"])
     _mark(ctx, comm, "gu.exchange_wait")
     router, send_counts, recv_counts, want_perm = st["router"], st["send_counts"], st["recv_counts"], st["want_perm"]
-    if want_perm and os.environ.get("UQB_MG_KEY_ROUNDTRIP") != "1":
+    if want_perm:
         # The sorted-on table: the records are going to follow their rows to this rank anyway (global_order), so the key of
         # this rank's slice of the global order is the group id in SORTED order - no trip back to the record's rank and
         # forth again.
@@ -804,23 +754,19 @@ def global_unique_end(ctx, comm, st):
         ctx.add_scalar_u32(key_sorted, sum(counts[:comm.rank]))
         route = ("partition", router, send_counts, recv_counts, perm_r, st["count_table"])
         return dict(key=None, key_sorted=key_sorted, uniq=uniq_range, n_unique=sum(counts), counts=counts, route=route)
-    perm_r, key_r, uniq_range, nr = ctx.sort_rows(recv, want_perm=want_perm, want_key=True, want_uniq=True)
+    _, key_r, uniq_range, nr = ctx.sort_rows(recv, want_key=True, want_uniq=True)
     recv.free()
     _mark(ctx, comm, "gu.sort")
     counts = comm.all_gather_object(nr)
     ctx.add_scalar_u32(key_r, sum(counts[:comm.rank]))       # global id of every received row
     ids_back = comm.all_to_all_rows(ctx, key_r, recv_counts, send_counts)        # in the order the rows were sent
     key_r.free()
-    # ids_back is in the order the rows were sent: row i was sent at position pos[i] (= order^-1)
-    key_global = ctx.gather_rows(ids_back, router[1]) if router[0] == "pos" else ctx.scatter_u32(ids_back, router[1])
+    # ids_back is in the order the rows were sent: row i was sent at position pos[i]
+    key_global = ctx.gather_rows(ids_back, router[0])
     ids_back.free()
     _mark(ctx, comm, "gu.ids_back")
-    if want_perm:
-        route = ("partition", router, send_counts, recv_counts, perm_r, st["count_table"])
-    else:
-        _router_free(router)
-        route = None
-    return dict(key=key_global, uniq=uniq_range, n_unique=sum(counts), counts=counts, route=route)
+    _router_free(router)
+    return dict(key=key_global, uniq=uniq_range, n_unique=sum(counts), counts=counts, route=None)
 
 
 def global_unique_merge(ctx, comm, table, want_perm=False):
