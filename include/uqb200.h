@@ -274,8 +274,10 @@ int uqb_decode(uqb_ctx* ctx, const uqb_array* dna, const uqb_array* qual, uqb_ar
 
 /* ---- synthetic inputs for bench/tests (same generator as oracle/synth.py, oracle/synth_umi.py) - */
 typedef struct {
-    uint32_t kind;        /* 0 illumina, 1 genome, 2 casava, 3 ont, 4 umi (illumina header + '_' + 6-12 of ACGTN) */
-    uint32_t length;      /* read length (kinds 0-2, 4) */
+    uint32_t kind;        /* 0 illumina, 1 genome, 2 casava, 3 ont, 4 umi (illumina header + '_' + 6-12 of ACGTN),
+                             5 renamed (@SRR0000001.<record+1>), 6 mixed (blocks of 1024 records alternate between the
+                             casava header and the pre-1.8 @HWI-D00123:<lane>:<tile>:<x>:<y>#0/1) */
+    uint32_t length;      /* read length (kinds 0-2, 4-6) */
     uint32_t len_lo, len_hi; /* kind 3 */
     uint64_t seed, first, n; /* records first .. first+n-1 */
     uint64_t genome, pool;   /* kind 1 */

@@ -1,5 +1,5 @@
 // Synthetic FASTQ generator on the device (bench / tests only): the same counter-based generator as
-// oracle/synth.py (kind 4 'umi': oracle/synth_umi.py), so bench.py can create the 100 M-read inputs of BASELINE.json directly in HBM.
+// oracle/synth.py (kind 4 'umi': oracle/synth_umi.py; kinds 5 'renamed' and 6 'mixed': oracle/synth_names.py), so bench.py can create the 100 M-read inputs of BASELINE.json directly in HBM.
 #include "common.cuh"
 
 #define SY 256
@@ -57,7 +57,9 @@ __device__ unsigned synth_header(uint8_t* w, const uqb_synth_params& p, unsigned
                 n++;
             }
         }
-    } else if (p.kind == 2) {
+    } else if (p.kind == 5) {      // renamed reads: a run accession and the read number, no separator with a constant count
+        n += put_str(W, "@SRR0000001."); n += put_uint(W, r + 1);
+    } else if (p.kind == 2 || (p.kind == 6 && !((r >> 10) & 1))) {
         const bool flag = rnd(p.seed, ST_FLAG, r) % 8 == 0;
         const unsigned long long even = 2 * (rnd(p.seed, ST_EVEN, r) % 20), bc = rnd(p.seed, ST_BARCODE, r) % 4;
         n += put_str(W, "@EAS139:136:FC706VJ:");
@@ -65,6 +67,10 @@ __device__ unsigned synth_header(uint8_t* w, const uqb_synth_params& p, unsigned
         n += put_uint(W, x); n += put_str(W, ":"); n += put_uint(W, y);
         n += put_str(W, " 1:"); n += put_str(W, flag ? "Y" : "N"); n += put_str(W, ":");
         n += put_uint(W, even); n += put_str(W, ":"); n += put_str(W, c_barcodes[bc]);
+    } else if (p.kind == 6) {      // odd blocks of 1024 records: the pre-1.8 Illumina header
+        n += put_str(W, "@HWI-D00123:");
+        n += put_uint(W, lane); n += put_str(W, ":"); n += put_uint(W, tile); n += put_str(W, ":");
+        n += put_uint(W, x); n += put_str(W, ":"); n += put_uint(W, y); n += put_str(W, "#0/1");
     } else {
         const unsigned long long run = 1 + rnd(p.seed, ST_RUN, r) % 4, ch = 1 + rnd(p.seed, ST_CH, r) % 512;
         n += put_str(W, "@ONT7:");
@@ -132,7 +138,7 @@ __global__ void __launch_bounds__(SY) k_synth_write(uqb_synth_params p, const lo
 }
 
 extern "C" int uqb_synth(uqb_ctx* ctx, const uqb_synth_params* p, const int64_t* ont_len_table, uqb_array** bytes) {
-    if (p->kind > 4) return uqb_fail(ctx, "synth: kind %u", p->kind);
+    if (p->kind > 6) return uqb_fail(ctx, "synth: kind %u", p->kind);
     if (p->kind == 3 && !ont_len_table) return uqb_fail(ctx, "synth: ont needs a length table");
     if (p->kind == 1 && (p->genome <= p->length || p->pool == 0)) return uqb_fail(ctx, "synth: genome/pool too small");
     if (p->n >= (1ull << 32)) return uqb_fail(ctx, "synth: too many records");

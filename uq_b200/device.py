@@ -232,7 +232,7 @@ class Context:
         return fq
 
     def synth(self, kind, n, length, seed, first=0, genome=0, pool=0, len_table=None):
-        kinds = {"illumina": 0, "genome": 1, "casava": 2, "ont": 3, "umi": 4}
+        kinds = {"illumina": 0, "genome": 1, "casava": 2, "ont": 3, "umi": 4, "renamed": 5, "mixed": 6}
         p = L.SynthParams()
         p.kind = kinds[kind]
         if kind == "ont":

@@ -235,12 +235,17 @@ def pack_params(dec):
 # ------------------------------------------------------------------------------------------------
 # Pass-2 decisions (uq.py:586-602, 641-676)
 # ------------------------------------------------------------------------------------------------
-def decide_columns(colstats, n_reads, fetch_dict):
+def decide_columns(colstats, n_reads, fetch_dict, exact_ints=False):
+    """exact_ints (the single QNAME column of E2): a column counts as all-integer only when every token is the
+    canonical text of an int64 (str(int(t)) == t), so that integers decode to exactly the names they came from."""
     columns = []
     last = n_reads - 1
     for i, cs in enumerate(colstats):
         col = {'name': 'QNAME_%d' % (i + 1)}
-        if cs.overflow:
+        all_int = cs.all_int
+        if exact_ints:
+            all_int = cs.all_int and cs.all_canonical and not cs.overflow
+        elif cs.overflow:
             raise UQError('ERROR: QNAME column %d holds an integer outside the int64 range' % (i + 1))
         demoted = False
         t = 10000
@@ -252,7 +257,7 @@ def decide_columns(colstats, n_reads, fetch_dict):
         if not demoted and cs.n_distinct > last // 10:       # uq.py:638
             demoted = True
         if demoted:
-            if not cs.all_int:                     # 'strings' (uq.py:598-601, 624-630); the reference stops at uq.py:672-673
+            if not all_int:                        # 'strings' (uq.py:598-601, 624-630); the reference stops at uq.py:672-673
                 # declared extension E1: the tokens themselves, zero padded to the longest one over ALL records (the
                 # reference's own `longest` undercounts after an integers -> strings switch).  An all-empty column still
                 # gets one byte: numpy has no zero-width S dtype.
@@ -273,7 +278,7 @@ def decide_columns(colstats, n_reads, fetch_dict):
         else:
             n = int(cs.n_distinct)
             cap, col['dtype'], _ = next(d for d in _DT if n <= d[0])
-            if cs.all_int and int(cs.max_val) - int(cs.min_val) <= cap:     # uq.py:649-658
+            if all_int and int(cs.max_val) - int(cs.min_val) <= cap:        # uq.py:649-658
                 col['format'] = 'integers'
                 col['max'], col['min'] = int(cs.max_val), int(cs.min_val)
                 col['offset'] = bool(col['min'] < 0 or col['max'] > cap)
@@ -284,6 +289,36 @@ def decide_columns(colstats, n_reads, fetch_dict):
             raise UQError('ERROR: negative integers in QNAME column %d' % (i + 1))
         columns.append(col)
     return columns
+
+
+def decide_qname_columns(st, n_reads, scan, shortest_remainder, fetch_dict):
+    """QNAME layout and column typing -> (prefix, suffix, separators, columns).
+
+    scan(prefix, suffix, separators) -> (column statistics, bad_record) tokenises every record;
+    shortest_remainder(prefix_len) -> min over all records of len(name) - prefix_len.
+
+    A file whose names the reference cuts into columns (derive_qname_layout accepts it and every record holds the
+    separators in their order) gets exactly the reference's layout.  Every other file takes declared extension E2
+    (DESIGN section 4): no separators and one column QNAME_1, the part of each name between the longest common prefix
+    of all names and the longest common suffix of what that prefix leaves of them.  That suffix is the common suffix
+    of the names clamped to the shortest remainder: unclamped, it could overlap the prefix inside a short name
+    ('@ab' / '@abab'), whose middle the tokeniser would then cut empty."""
+    try:
+        prefix, suffix, separators = derive_qname_layout(st, n_reads)
+    except UQError:
+        pass
+    else:
+        colstats, bad = scan(prefix, suffix, separators)
+        if bad < 0:
+            return prefix, suffix, separators, decide_columns(colstats, n_reads, fetch_dict)
+    first = bytes(st.first_name[:st.first_len]).decode('latin-1')
+    plen = int(st.prefix_len)
+    slen = min(int(st.suffix_len), shortest_remainder(plen))
+    prefix, suffix = first[:plen], first[len(first) - slen:] if slen else ''
+    colstats, bad = scan(prefix, suffix, '')
+    if bad >= 0:                                   # with no separator every record is one column
+        raise UQError('ERROR: record %d does not split into one QNAME column' % bad)
+    return prefix, suffix, '', decide_columns(colstats, n_reads, fetch_dict, exact_ints=True)
 
 
 def column_specs(columns):
@@ -582,13 +617,11 @@ def prepare(ctx, fq, pad=False, notricks=False):
         if w == 'plus':                                                            # uq.py:360, 382
             raise UQError('ERROR: For entry %d the third line does not start with +' % r)
         raise UQError('ERROR: Length of DNA does not match the length of the quality scores for entry %d' % (r + 1))   # uq.py:366, 388
-    prefix, suffix, separators = derive_qname_layout(st, n)
+    prefix, suffix, separators, columns = decide_qname_columns(
+        st, n, lambda p, s, seps: _timed(ctx, 'qname_scan', fq.qname_scan, len(p), len(s), seps),
+        lambda plen: int(_timed(ctx, 'qname_remainder', fq.qname_scan, plen, 0, '', col_mode=[1])[0][0].min_len),
+        fq.qname_dict)
     dec = decide_alphabets(st, notricks=notricks, pad=pad)
-    colstats, bad_rec = _timed(ctx, 'qname_scan', fq.qname_scan, len(prefix), len(suffix), separators)
-    if bad_rec >= 0:                                                               # uq.py:609-613, 637
-        raise UQError('Encoding QNAMEs as strings has not been implimented yet. (record %d does not split into %d columns)'
-                      % (bad_rec, len(separators) + 1))
-    columns = decide_columns(colstats, n, fq.qname_dict)
     dna, qual = _timed(ctx, 'pack', fq.pack, pack_params(dec))
     cols = _timed(ctx, 'qname_encode', fq.qname_encode, column_specs(columns))
     return dict(stats=st, dec=dec, columns=columns, dna=dna, qual=qual, cols=cols, prefix=prefix, suffix=suffix,

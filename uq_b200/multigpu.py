@@ -973,39 +973,50 @@ def encode_sharded(ctx, comm, fq, sort=None, raw=None, pattern=None, pad=False, 
     if bad:
         r, w = min(bad, key=lambda t: (t[0], t[1] != 'plus'))
         raise host.UQError('ERROR: malformed FASTQ record %d (%s)' % (r, w))
-    prefix, suffix, separators = host.derive_qname_layout(st, n_total)
     dec = host.decide_alphabets(st, notricks=notricks, pad=pad)
     _mark(ctx, comm, "split+pass1")
     # ---- Pass 2: rank 0 decides which columns leave 'mapping' at checkpoint 0, the others skip those dictionaries ----
-    ncols = len(separators) + 1
-    # which columns leave 'mapping' at checkpoint 0 is a property of the first 10001 records of the file: rank 0 scans
-    # just that head (a few megabytes) and tells the others, then every rank scans its own range at the same time
-    early = None
-    if comm.rank == 0:
-        early = [False] * ncols
-        if n_total > 10000:
-            head_bytes = int(fq.line_offsets(4 * 10001, 1)[0])
-            hfq = ctx.load_fastq(fq.download(0, head_bytes))
-            hfq.split()
-            hcols, hbad = hfq.qname_scan(len(prefix), len(suffix), separators)
-            if hbad < 0:
-                early = [bool(hcols[c].n_distinct == L.U64_MAX) for c in range(ncols)]
-            hfq.free()
-    early = comm.all_gather_object(early)[0]
-    cols0, bad0 = fq.qname_scan(len(prefix), len(suffix), separators, col_mode=[1 if e else 2 for e in early])
-    my_dicts = {}
-    if bad0 < 0:
-        for c in range(ncols):
-            if not early[c]:
-                toks = fq.qname_dict(c)
-                my_dicts[c] = (toks, (fq.qname_dict_first(c).astype(np.int64) + base).tolist())
-    pass2 = comm.all_gather_object((bad0, colstats_to_plain(cols0, ncols) if bad0 < 0 else None, my_dicts))
-    if any(p[0] >= 0 for p in pass2):
-        raise host.UQError('Encoding QNAMEs as strings has not been implimented yet.')
-    all_plain = [p[1] for p in pass2]
-    all_dicts = [p[2] for p in pass2]
-    colstats, gdicts = merge_colstats(all_plain, n_total, early, all_dicts)
-    columns = host.decide_columns(colstats, n_total, lambda i: gdicts[i])
+    pass2_of = {}                                   # this rank's and the merged dictionaries of the final layout
+
+    def scan(prefix, suffix, separators):
+        """column statistics of the whole file; a record that does not split on ANY rank switches every rank to E2"""
+        ncols = len(separators) + 1
+        # which columns leave 'mapping' at checkpoint 0 is a property of the first 10001 records of the file: rank 0
+        # scans just that head (a few megabytes) and tells the others, then every rank scans its own range at the same time
+        early = None
+        if comm.rank == 0:
+            early = [False] * ncols
+            if n_total > 10000:
+                head_bytes = int(fq.line_offsets(4 * 10001, 1)[0])
+                hfq = ctx.load_fastq(fq.download(0, head_bytes))
+                hfq.split()
+                hcols, hbad = hfq.qname_scan(len(prefix), len(suffix), separators)
+                if hbad < 0:
+                    early = [bool(hcols[c].n_distinct == L.U64_MAX) for c in range(ncols)]
+                hfq.free()
+        early = comm.all_gather_object(early)[0]
+        cols0, bad0 = fq.qname_scan(len(prefix), len(suffix), separators, col_mode=[1 if e else 2 for e in early])
+        my_dicts = {}
+        if bad0 < 0:
+            for c in range(ncols):
+                if not early[c]:
+                    toks = fq.qname_dict(c)
+                    my_dicts[c] = (toks, (fq.qname_dict_first(c).astype(np.int64) + base).tolist())
+        pass2 = comm.all_gather_object((bad0, colstats_to_plain(cols0, ncols) if bad0 < 0 else None, my_dicts))
+        bad = [base_r + p[0] for p, (_, base_r, _) in zip(pass2, parts) if p[0] >= 0]
+        if bad:
+            return None, min(bad)
+        colstats, merged = merge_colstats([p[1] for p in pass2], n_total, early, [p[2] for p in pass2])
+        pass2_of.update(local=my_dicts, merged=merged)
+        return colstats, -1
+
+    def shortest_remainder(plen):
+        cols, _ = fq.qname_scan(plen, 0, '', col_mode=[1])
+        return min(comm.all_gather_object(int(cols[0].min_len)))
+
+    prefix, suffix, separators, columns = host.decide_qname_columns(st, n_total, scan, shortest_remainder,
+                                                                    lambda i: pass2_of['merged'][i])
+    my_dicts, gdicts = pass2_of['local'], pass2_of['merged']
     _mark(ctx, comm, "pass2")
     # ---- pack + column encode (per read) ----
     dna, qual = fq.pack(host.pack_params(dec))
