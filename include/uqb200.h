@@ -241,6 +241,16 @@ int uqb_rows_to_columns(uqb_ctx* ctx, const uqb_array* rows, uint32_t ncols, con
 int uqb_columns_to_rows_ex(uqb_ctx* ctx, uint32_t ncols, uqb_array* const* cols, const uint8_t* kinds, uqb_array** rows);
 int uqb_rows_to_columns_ex(uqb_ctx* ctx, const uqb_array* rows, uint32_t ncols, const uint32_t* itemsizes, const uint8_t* kinds,
                            uqb_array** cols);
+/* integer columns (itemsize 1/2/4/8) whose value ranges fit 64 bits together -> one packed sort key per row:
+ * key = sum over c of (cols[c][i] - bases[c]) << shifts[c], field c `bits[c]` wide (0: a constant column), the first column
+ * in the highest bits.  Its numeric order is the memcmp order of the rows of uqb_columns_to_rows.  `table` is a table of
+ * 8-byte rows for uqb_sort_rows only, which sorts it by the key alone: its row bytes are the key itself (little-endian),
+ * not memcmp rows.  The unique table uqb_sort_rows returns for it holds the distinct keys as 8 big-endian bytes;
+ * uqb_key_to_columns unpacks such rows into columns of itemsizes[c] bytes: (field c) + bases[c]. */
+int uqb_columns_to_key(uqb_ctx* ctx, uint32_t ncols, uqb_array* const* cols, const uint32_t* shifts, const uint32_t* bits,
+                       const uint64_t* bases, uqb_array** table);
+int uqb_key_to_columns(uqb_ctx* ctx, const uqb_array* keys, uint32_t ncols, const uint32_t* itemsizes, const uint32_t* shifts,
+                       const uint32_t* bits, const uint64_t* bases, uqb_array** cols);
 
 /* ---- stage 4: physical layouts (replaces write_pattern uq.py:257-270) ------------------------ */
 /* pattern ids: 0='0.1' 1='1.1' 2='2.1' 3='3.1' 4='0.2' 5='1.2' 6='2.2' 7='3.2'.  Produces the exact

@@ -1133,6 +1133,104 @@ __global__ void __launch_bounds__(ST) k_rows_to_cols_staged(col_desc_out cd, uin
     }
 }
 
+// ---- QNAME columns <-> one packed 64-bit key ------------------------------------------------------------------
+// Integer / mapping columns whose value ranges fit 64 bits together: field c holds (value - base) in `bits` bits at
+// `shift`, the first column highest.  The key's numeric order is the memcmp order of the big-endian rows above, so the
+// key alone sorts the table (no refinement, no row reads) and the unique keys unpack straight into typed columns.
+struct key_desc {
+    const uint8_t* p[UQB_MAX_COLS]; uint64_t base[UQB_MAX_COLS]; uint64_t mask[UQB_MAX_COLS];
+    uint32_t size[UQB_MAX_COLS]; uint32_t shift[UQB_MAX_COLS]; uint32_t ncols;
+};
+
+__global__ void __launch_bounds__(ST) k_cols_to_key(key_desc kd, uint64_t n, uint64_t* __restrict__ key) {
+    for (uint64_t r = (uint64_t)blockIdx.x * ST + threadIdx.x; r < n; r += (uint64_t)gridDim.x * ST) {
+        uint64_t k = 0;
+        for (uint32_t c = 0; c < kd.ncols; c++) {
+            const uint32_t sz = kd.size[c];
+            const uint64_t v = sz == 1 ? cr_load<uint8_t>(kd.p[c], r) : sz == 2 ? cr_load<uint16_t>(kd.p[c], r)
+                             : sz == 4 ? cr_load<uint32_t>(kd.p[c], r) : cr_load<uint64_t>(kd.p[c], r);
+            k |= ((v - kd.base[c]) & kd.mask[c]) << kd.shift[c];
+        }
+        key[r] = k;
+    }
+}
+
+// unique rows of such a table (8 big-endian key bytes, k_uniq_from_keys) -> typed columns; p[] are the outputs
+__global__ void __launch_bounds__(ST) k_key_to_cols(key_desc kd, uint64_t n, const uint64_t* __restrict__ rows) {
+    for (uint64_t r = (uint64_t)blockIdx.x * ST + threadIdx.x; r < n; r += (uint64_t)gridDim.x * ST) {
+        const uint64_t be = rows[r];
+        const uint64_t k = ((uint64_t)__byte_perm((uint32_t)be, 0u, 0x0123u) << 32) | __byte_perm((uint32_t)(be >> 32), 0u, 0x0123u);
+        for (uint32_t c = 0; c < kd.ncols; c++) {
+            const uint64_t v = ((k >> kd.shift[c]) & kd.mask[c]) + kd.base[c];
+            uint8_t* o = const_cast<uint8_t*>(kd.p[c]);
+            const uint32_t sz = kd.size[c];
+            if (sz == 1) reinterpret_cast<uint8_t*>(o)[r] = (uint8_t)v;
+            else if (sz == 2) reinterpret_cast<uint16_t*>(o)[r] = (uint16_t)v;
+            else if (sz == 4) reinterpret_cast<uint32_t*>(o)[r] = (uint32_t)v;
+            else reinterpret_cast<uint64_t*>(o)[r] = v;
+        }
+    }
+}
+
+static int key_desc_fill(uqb_ctx* ctx, key_desc* kd, uint32_t ncols, const uint32_t* shifts, const uint32_t* bits, const uint64_t* bases) {
+    if (ncols == 0 || ncols > UQB_MAX_COLS) return uqb_fail(ctx, "packed key: bad column count %u", ncols);
+    uint32_t total = 0;
+    kd->ncols = ncols;
+    for (uint32_t c = 0; c < ncols; c++) {
+        if (bits[c] > 64 || (bits[c] && shifts[c] + bits[c] > 64))
+            return uqb_fail(ctx, "packed key: column %u has %u bits at shift %u", c, bits[c], shifts[c]);
+        total += bits[c];
+        kd->shift[c] = bits[c] ? shifts[c] : 0;
+        kd->mask[c] = bits[c] == 64 ? ~0ull : (1ull << bits[c]) - 1;
+        kd->base[c] = bases[c];
+    }
+    if (total > 64) return uqb_fail(ctx, "packed key: %u bits exceed 64", total);
+    return 0;
+}
+
+extern "C" int uqb_columns_to_key(uqb_ctx* ctx, uint32_t ncols, uqb_array* const* cols, const uint32_t* shifts, const uint32_t* bits,
+                                  const uint64_t* bases, uqb_array** table) {
+    key_desc kd;
+    UQB_TRY(key_desc_fill(ctx, &kd, ncols, shifts, bits, bases));
+    const uint64_t n = cols[0]->n;
+    uint64_t ab = 8 * n;
+    for (uint32_t c = 0; c < ncols; c++) {
+        const uint32_t sz = cols[c]->width;
+        if (cols[c]->n != n) return uqb_fail(ctx, "columns_to_key: ragged columns");
+        if (sz != 1 && sz != 2 && sz != 4 && sz != 8) return uqb_fail(ctx, "columns_to_key: column %u has itemsize %u", c, sz);
+        kd.p[c] = (const uint8_t*)cols[c]->d; kd.size[c] = sz;
+        ab += n * sz;
+    }
+    uint64_t* key;
+    UQB_TRY(uqb_dalloc_t(ctx, &key, n));
+    // the key is the table's key0, which is all uqb_sort_rows reads of a table of 8-byte rows; the row bytes are the same
+    // buffer (little-endian keys, not memcmp rows), owned through key0
+    uqb_array* a = new (std::nothrow) uqb_array();
+    if (!a) { uqb_dfree(ctx, key, n * 8); return uqb_fail(ctx, "out of host memory"); }
+    a->d = key; a->n = n; a->width = 8; a->owned = false; a->key0 = key;
+    *table = a;
+    if (n) UQB_LAUNCH_B(ab, k_cols_to_key, uqb_grid(ctx, n, ST, 16), ST, 0, kd, n, key);
+    return 0;
+}
+
+extern "C" int uqb_key_to_columns(uqb_ctx* ctx, const uqb_array* keys, uint32_t ncols, const uint32_t* itemsizes, const uint32_t* shifts,
+                                  const uint32_t* bits, const uint64_t* bases, uqb_array** cols) {
+    key_desc kd;
+    UQB_TRY(key_desc_fill(ctx, &kd, ncols, shifts, bits, bases));
+    if (keys->width != 8) return uqb_fail(ctx, "key_to_columns: rows are %u bytes wide, not 8", keys->width);
+    const uint64_t n = keys->n;
+    uint64_t ab = 8 * n;
+    for (uint32_t c = 0; c < ncols; c++) {
+        const uint32_t sz = itemsizes[c];
+        if (sz != 1 && sz != 2 && sz != 4 && sz != 8) return uqb_fail(ctx, "key_to_columns: column %u has itemsize %u", c, sz);
+        UQB_TRY(uqb_new_array(ctx, n, sz, &cols[c]));
+        kd.p[c] = (const uint8_t*)cols[c]->d; kd.size[c] = sz;
+        ab += n * sz;
+    }
+    if (n) UQB_LAUNCH_B(ab, k_key_to_cols, uqb_grid(ctx, n, ST, 16), ST, 0, kd, n, (const uint64_t*)keys->d);
+    return 0;
+}
+
 // ---- the same transforms with byte columns (kind 1: 'strings' QNAME columns, E1) -------------------------------
 // A byte column enters the row as it is: memcmp of its zero-padded bytes is numpy's order of S values.  Bit c of
 // `bytes_mask` marks column c as such a column.  These kernels are separate from the ones above so that tables of

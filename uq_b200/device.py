@@ -17,6 +17,12 @@ def _ptr(a):
     return a.ctypes.data_as(C.c_void_p)
 
 
+def _plan_arrays(plan):
+    n = len(plan)
+    return ((C.c_uint32 * n)(*[int(s) for s, _, _ in plan]), (C.c_uint32 * n)(*[int(b) for _, b, _ in plan]),
+            (C.c_uint64 * n)(*[int(a) for _, _, a in plan]))
+
+
 class Context:
     """One per host thread.  `stream` may be a raw cudaStream_t (e.g. torch.cuda.current_stream().cuda_stream)."""
 
@@ -292,6 +298,23 @@ class Context:
         else:
             k = np.ascontiguousarray(kinds, dtype=np.uint8)
             self.check(self.lib.uqb_rows_to_columns_ex(self.h, rows.h, n, sizes, _ptr(k), outs))
+        return [DeviceArray(self, C.c_void_p(outs[i])) for i in range(n)]
+
+    def columns_to_key(self, cols, plan):
+        """integer columns -> table of packed 64-bit sort keys; plan = [(shift, bits, base)] per column"""
+        arr = (C.c_void_p * len(cols))(*[c.h for c in cols])
+        shifts, bits, bases = _plan_arrays(plan)
+        h = C.c_void_p()
+        self.check(self.lib.uqb_columns_to_key(self.h, len(cols), arr, shifts, bits, bases, C.byref(h)))
+        return DeviceArray(self, h)
+
+    def key_to_columns(self, keys, itemsizes, plan):
+        """unique rows of a packed-key table (8 big-endian bytes) -> columns of the given itemsizes"""
+        n = len(itemsizes)
+        sizes = (C.c_uint32 * n)(*[int(s) for s in itemsizes])
+        shifts, bits, bases = _plan_arrays(plan)
+        outs = (C.c_void_p * n)()
+        self.check(self.lib.uqb_key_to_columns(self.h, keys.h, n, sizes, shifts, bits, bases, outs))
         return [DeviceArray(self, C.c_void_p(outs[i])) for i in range(n)]
 
     def layout(self, table, pattern):

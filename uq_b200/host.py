@@ -487,16 +487,10 @@ def _mix_dna_qual(ctx, out, table, name, order, raw, pattern, prepared=None):
             k2 = ctx.gather_rows(key, order)                                       # key[sort_order], uq.py:798
             key.free()
             key = k2
-        size = key_itemsize(nu)
-        narrow = ctx.narrow_u32(key, size)                                         # uq.py:790
-        key.free()
-        out.add_vector(name + '.key', narrow, 'uint%d' % (8 * size))
+        out.add_vector(name + '.key', *_narrow_key(ctx, key, nu))                  # uq.py:790
     else:
         key, uniq, nu, order = _keyed(ctx, table, order)                           # uq.py:786, 796
-        size = key_itemsize(nu)
-        narrow = ctx.narrow_u32(key, size)                                         # uq.py:790
-        key.free()
-        out.add_vector(name + '.key', narrow, 'uint%d' % (8 * size))
+        out.add_vector(name + '.key', *_narrow_key(ctx, key, nu))                  # uq.py:790
         stream, aliased = _layout(ctx, uniq, pattern)
         out.add_table(name, stream, uniq.n, uniq.width, pattern)
         if not aliased:
@@ -517,32 +511,74 @@ def qname_rows(ctx, cols, columns):
     return ctx.columns_to_rows(cols, qname_kinds(columns))
 
 
-def qname_columns(ctx, rows, columns):
-    """sort rows (e.g. the unique ones) -> typed QNAME columns again (uq.py:842-847)"""
-    return ctx.rows_to_columns(rows, [np.dtype(m['dtype']).itemsize for m in columns], qname_kinds(columns))
+def qname_key_plan(columns):
+    """One packed 64-bit sort key for QNAME columns -> [(shift, bits, base)] per column, or None (a 'strings' column, or
+    more than 64 bits).  Field c holds the column's encoded value minus `base` in `bits` bits at `shift`, the first
+    column in the highest bits, so the key's numeric order is the memcmp order of qname_rows: sorting the key alone
+    sorts the table, and the unique keys unpack straight into the columns."""
+    fields = []
+    for c in columns:
+        if c['format'] == 'strings':
+            return None
+        if c['format'] == 'mapping':                       # rank in the sorted dictionary
+            fields.append(((len(c['map']) - 1).bit_length(), 0))
+        else:                                              # an offset column already holds value - min
+            fields.append(((c['max'] - c['min']).bit_length(), 0 if c['offset'] else c['min']))
+    if sum(b for b, _ in fields) > 64:
+        return None
+    plan, shift = [], 0
+    for bits, base in reversed(fields):
+        plan.append((shift, bits, base))
+        shift += bits
+    return plan[::-1]
+
+
+def qname_sort_table(ctx, cols, columns):
+    """QNAME columns -> (table that uqb_sort_rows sorts into the row order of E1, plan): the packed-key table when
+    qname_key_plan gives one (plan), else the sort rows (None)"""
+    plan = qname_key_plan(columns)
+    if plan is None:
+        return qname_rows(ctx, cols, columns), None
+    return ctx.columns_to_key(cols, plan), plan
+
+
+def qname_columns(ctx, uniq, columns, plan):
+    """unique rows of the qname_sort_table table -> typed QNAME columns again (uq.py:842-847)"""
+    sizes = [np.dtype(m['dtype']).itemsize for m in columns]
+    if plan is None:
+        return ctx.rows_to_columns(uniq, sizes, qname_kinds(columns))
+    return ctx.key_to_columns(uniq, sizes, plan)
+
+
+def _narrow_key(ctx, key, nu):
+    """key.astype(min_scalar_type(max(key))) (uq.py:790, 832) -> (array, dtype).  Takes over `key`: a key of four-byte
+    items is that array already."""
+    size = key_itemsize(nu)
+    if size != 4:
+        narrow = ctx.narrow_u32(key, size)
+        key.free()
+        key = narrow
+    return key, 'uint%d' % (8 * size)
 
 
 def _mix_qname(ctx, out, cols, columns, order, raw):
     """encode_qname (uq.py:808-851)."""
     if raw:
         if order is False:
-            rows = qname_rows(ctx, cols, columns)
-            order, _, _, _ = ctx.sort_rows(rows, want_perm=True)                   # uq.py:816
-            rows.free()
+            table, _ = qname_sort_table(ctx, cols, columns)
+            order, _, _, _ = ctx.sort_rows(table, want_perm=True)                  # uq.py:816
+            table.free()
         for c, meta in zip(cols, columns):
             if order is not None:
                 out.add_vector(meta['name'] + '.raw', ctx.gather_rows(c, order), meta['dtype'])
             else:
                 out.add_vector(meta['name'] + '.raw', c, meta['dtype'])
     else:
-        rows = qname_rows(ctx, cols, columns)
-        key, uniq, nu, order = _keyed(ctx, rows, order)                            # uq.py:830, 833
-        rows.free()
-        size = key_itemsize(nu)
-        narrow = ctx.narrow_u32(key, size)
-        key.free()
-        out.add_vector('QNAME.key', narrow, 'uint%d' % (8 * size))
-        ucols = qname_columns(ctx, uniq, columns)                                  # uq.py:842-847
+        table, plan = qname_sort_table(ctx, cols, columns)
+        key, uniq, nu, order = _keyed(ctx, table, order)                           # uq.py:830, 833
+        table.free()
+        out.add_vector('QNAME.key', *_narrow_key(ctx, key, nu))
+        ucols = qname_columns(ctx, uniq, columns, plan)                            # uq.py:842-847
         uniq.free()
         for c, meta in zip(ucols, columns):
             out.add_vector(meta['name'], c, meta['dtype'])
@@ -658,6 +694,7 @@ class MixFeed:
         self.ctx = ctx
         self.p = prepare(ctx, fq, pad=pad, notricks=notricks)
         self.tables = {'DNA': self.p['dna'], 'QUAL': self.p['qual'], 'QNAME': None}
+        self.qname_plan = None
         self.sorted = {}            # table -> dict(perm, key, key_sorted, uniq, nu)
         self.cache = {}             # derived device arrays: ('rows', T, S) / ('key', T, S) / ('stream', ...) ...
         self.kernel_launches_after_prepare = ctx.launches
@@ -669,7 +706,7 @@ class MixFeed:
 
     def _table(self, t):
         if self.tables[t] is None:                       # QNAME sort rows (uq.py:814-816)
-            self.tables[t] = qname_rows(self.ctx, self.p['cols'], self.p['columns'])
+            self.tables[t], self.qname_plan = qname_sort_table(self.ctx, self.p['cols'], self.p['columns'])
         return self.tables[t]
 
     def _sorted(self, t):
@@ -726,7 +763,7 @@ class MixFeed:
             out['QNAME.key'] = self._key('QNAME', s_on, order)
 
             def make_cols():
-                ucols = qname_columns(ctx, srt['uniq'], columns)
+                ucols = qname_columns(ctx, srt['uniq'], columns, self.qname_plan)
                 host = [u.download(dtype=np.dtype(m['dtype'])).reshape(-1) for u, m in zip(ucols, columns)]
                 for u in ucols:
                     u.free()
@@ -746,9 +783,10 @@ class MixFeed:
                 k32, tmp = srt['key'], None
             else:
                 k32 = tmp = self.ctx.gather_rows(srt['key'], order)                  # key[sort_order], uq.py:798
-            narrow = self.ctx.narrow_u32(k32, size)
+            narrow = k32 if size == 4 else self.ctx.narrow_u32(k32, size)
             h = narrow.download(dtype=np.dtype('uint%d' % (8 * size))).reshape(-1)
-            narrow.free()
+            if narrow is not k32:
+                narrow.free()
             if tmp is not None:
                 tmp.free()
             return h

@@ -1046,6 +1046,8 @@ def encode_sharded(ctx, comm, fq, sort=None, raw=None, pattern=None, pad=False, 
         res.add(name, stream, 'table', dict(width=rows_arr.width, pattern=pat, rows=rows_arr.n))
 
     sorted_on = sort if sort in ('DNA', 'QUAL', 'QNAME') else None
+    # QNAME keeps its sort rows here, not the packed key of host.qname_sort_table: the sample-sort partition and the
+    # splitter search read row bytes
     tables = {'DNA': dna, 'QUAL': qual, 'QNAME': host.qname_rows(ctx, cols, columns)}
     keyed = {t: (t not in raw) for t in tables}
     uniq = {}
@@ -1072,7 +1074,7 @@ def encode_sharded(ctx, comm, fq, sort=None, raw=None, pattern=None, pad=False, 
             else:
                 payload[t + '.key'] = g['key']
             if t == 'QNAME':                        # unique rows back to typed columns (uq.py:842-847)
-                ucols = host.qname_columns(ctx, g['uniq'], columns)
+                ucols = host.qname_columns(ctx, g['uniq'], columns, None)
                 for c, meta in zip(ucols, columns):
                     res.add(meta['name'], c, 'vector', meta['dtype'])
                 g['uniq'].free()
