@@ -56,3 +56,33 @@ def sort_unique(table):
     perm = np.argsort(v, kind='stable')
     uniq, key = np.unique(v, return_inverse=True)
     return perm, key.reshape(-1), uniq.view(np.uint8).reshape(len(uniq), table.shape[1])
+
+
+def be_words(table):
+    """uint8 rows -> list of big-endian 64-bit words, most significant first (the last one zero padded): comparing the
+    word lists in order is memcmp order of the rows"""
+    n, w = table.shape
+    pad = np.zeros((n, -(-w // 8) * 8), dtype=np.uint8)
+    pad[:, :w] = table
+    return [pad[:, i:i + 8].copy().view('>u8').reshape(-1) for i in range(0, pad.shape[1], 8)]
+
+
+def sort_unique_rows(table):
+    """sort_unique through np.lexsort over big-endian words, an order of magnitude faster on millions of wide rows.
+    -> (perm: stable argsort of the rows, key: unique index of every row, key_sorted = key[perm], uniq: the unique
+    rows in ascending order)"""
+    n, w = table.shape
+    if n == 0:
+        e = np.zeros(0, dtype=np.int64)
+        return e, e, e, np.zeros((0, w), dtype=np.uint8)
+    words = be_words(table)
+    perm = np.lexsort(words[::-1])                  # stable, the first word is the primary key
+    head = np.zeros(n, dtype=bool)
+    head[0] = True
+    for c in words:
+        s = c[perm]
+        head[1:] |= s[1:] != s[:-1]
+    key_sorted = np.cumsum(head, dtype=np.int64) - 1
+    key = np.empty(n, dtype=np.int64)
+    key[perm] = key_sorted
+    return perm, key, key_sorted, table[perm[head]]

@@ -5,6 +5,7 @@ import numpy as np
 import pytest
 
 from oracle.synth import rnd, _skew, ST_GENOME, ST_NPOS, ST_OFF, ST_POOL, ST_QA, ST_QB, ST_SUB, ST_SUBV
+from oracle.uq_vec import sort_unique_rows
 
 pytestmark = pytest.mark.gpu
 
@@ -20,31 +21,9 @@ def ctx():
     c.close()
 
 
-def _be_words(t):
-    n, w = t.shape
-    pad = np.zeros((n, -(-w // 8) * 8), dtype=np.uint8)
-    pad[:, :w] = t
-    return [pad[:, i:i + 8].copy().view(">u8").reshape(-1) for i in range(0, pad.shape[1], 8)]
-
-
-def _np_sort_unique(t):
-    """numpy argsort(kind='stable') + unique(return_inverse) of the rows, through big-endian words and lexsort."""
-    words = _be_words(t)
-    perm = np.lexsort(words[::-1])                  # stable, first word major
-    head = np.zeros(len(perm), dtype=bool)
-    head[0] = True
-    for c in words:
-        s = c[perm]
-        head[1:] |= s[1:] != s[:-1]
-    gid = np.cumsum(head, dtype=np.int64) - 1
-    key = np.empty(len(perm), dtype=np.int64)
-    key[perm] = gid
-    return perm, key, gid, t[perm[head]]
-
-
 def _check(ctx, t):
     assert len(t) >= MSD_MIN_N
-    perm_w, key_w, ks_w, uniq_w = _np_sort_unique(t)
+    perm_w, key_w, ks_w, uniq_w = sort_unique_rows(t)
     d = ctx.upload(np.ascontiguousarray(t))
     perm, key, uniq, nu, ks = ctx.sort_rows(d, want_perm=True, want_key=True, want_uniq=True, want_key_sorted=True)
     assert nu == len(uniq_w)
