@@ -22,7 +22,7 @@
 extern "C" {
 #endif
 
-#define UQB_VERSION 100
+#define UQB_VERSION 101
 #define UQB_HDR_MAX 1024          /* longest first/last QNAME line the analysis reports on */
 #define UQB_MAX_COLS 64           /* QNAME columns (separators + 1) */
 #define UQB_MAX_CHECKPOINTS 40    /* Pass-2 checkpoints 10000*2^k (uq.py:572, 634-636) */
@@ -93,11 +93,11 @@ int uqb_fastq_load(uqb_ctx* ctx, const uint8_t* host, uint64_t nbytes, uqb_fastq
 int uqb_fastq_adopt(uqb_ctx* ctx, const uint8_t* dev, uint64_t nbytes, uqb_fastq** out);
 /* H2D in chunks on a second stream while the compute stream splits and analyses every chunk that has
  * landed: when the call returns, uqb_split / uqb_analyze on the handle only return the cached results.
- * `host` should be pinned (uqb_host_alloc) for the copies to overlap; chunk_bytes 0 = 256 MiB. */
-int uqb_fastq_load_streamed(uqb_ctx* ctx, const uint8_t* host, uint64_t nbytes, uint64_t chunk_bytes, uqb_fastq** out);
-/* the same for a multi-GPU shard (see uqb_fastq_set_reference): rbase > 0 = this shard does not start the file */
-int uqb_fastq_load_streamed_ref(uqb_ctx* ctx, const uint8_t* host, uint64_t nbytes, uint64_t chunk_bytes,
-                                const uint8_t* ref, uint32_t ref_len, uint64_t rbase, uqb_fastq** out);
+ * `host` should be pinned (uqb_host_alloc) for the copies to overlap; chunk_bytes 0 = 256 MiB.
+ * ref / ref_len / rbase: a multi-GPU shard, as uqb_fastq_set_reference (rbase > 0 = this shard does not start the
+ * file); ref NULL, ref_len 0, rbase 0 = the handle is the whole file. */
+int uqb_fastq_load_streamed(uqb_ctx* ctx, const uint8_t* host, uint64_t nbytes, uint64_t chunk_bytes,
+                            const uint8_t* ref, uint32_t ref_len, uint64_t rbase, uqb_fastq** out);
 int uqb_fastq_free(uqb_ctx* ctx, uqb_fastq* fq);
 int uqb_fastq_download(uqb_ctx* ctx, const uqb_fastq* fq, uint64_t offset, uint8_t* host, uint64_t nbytes);
 int uqb_split(uqb_ctx* ctx, uqb_fastq* fq, uqb_split_info* info);
@@ -151,13 +151,11 @@ typedef struct {
 } uqb_colstats;
 
 /* seps: the ordered separator string (uq.py:438-439).  bad_record: first record whose separator
- * sequence differs (the reference falls back / exits at uq.py:609-613, 637), -1 if none. */
+ * sequence differs (the reference falls back / exits at uq.py:609-613, 637), -1 if none.
+ * col_mode: one mode per column (NULL = all 0): 0 automatic, 1 no dictionary wanted (the column is known to
+ * leave 'mapping'), 2 dictionary forced (skip the checkpoint-0 shortcut) - used by multi-GPU merges */
 int uqb_qname_scan(uqb_ctx* ctx, uqb_fastq* fq, uint32_t prefix_len, uint32_t suffix_len,
-                   const uint8_t* seps, uint32_t nseps, uqb_colstats* cols, int64_t* bad_record);
-/* as uqb_qname_scan with a per-column mode (NULL = all 0): 0 automatic, 1 no dictionary wanted (the column
- * is known to leave 'mapping'), 2 dictionary forced (skip the checkpoint-0 shortcut) - used by multi-GPU merges */
-int uqb_qname_scan_ex(uqb_ctx* ctx, uqb_fastq* fq, uint32_t prefix_len, uint32_t suffix_len,
-                      const uint8_t* seps, uint32_t nseps, const uint8_t* col_mode, uqb_colstats* cols, int64_t* bad_record);
+                   const uint8_t* seps, uint32_t nseps, const uint8_t* col_mode, uqb_colstats* cols, int64_t* bad_record);
 /* first record (local index) holding each dictionary entry, uint32[count] */
 int uqb_qname_dict_first(uqb_ctx* ctx, uqb_fastq* fq, uint32_t col, uint32_t* host, uint64_t count);
 /* sorted dictionary of a column (uq.py:659-661): count rows x width bytes, zero padded */
@@ -232,15 +230,13 @@ int uqb_scatter_u32(uqb_ctx* ctx, const uqb_array* src, const uqb_array* idx, uq
 int uqb_index_u32(uqb_ctx* ctx, const uqb_array* a, uint64_t bound, uqb_array** out, int64_t* first_bad);
 /* uint32 -> little-endian integer of itemsize bytes (key.astype(min_scalar_type(max)), uq.py:790) */
 int uqb_narrow_u32(uqb_ctx* ctx, const uqb_array* a, uint32_t itemsize, uqb_array** out);
-/* QNAME columns <-> rows in sort-key form: columns concatenated big-endian at their own widths,
- * which makes memcmp order equal numpy's field-by-field unsigned comparison (uq.py:814-816, 828-830) */
-int uqb_columns_to_rows(uqb_ctx* ctx, uint32_t ncols, uqb_array* const* cols, uqb_array** rows);
-int uqb_rows_to_columns(uqb_ctx* ctx, const uqb_array* rows, uint32_t ncols, const uint32_t* itemsizes, uqb_array** cols);
-/* the same with a kind per column (kinds NULL = all 0): 0 little-endian integer (stored big-endian in the row), 1 bytes
- * copied in order ('strings' columns, E1: memcmp of zero-padded bytes is numpy's order of S values) */
-int uqb_columns_to_rows_ex(uqb_ctx* ctx, uint32_t ncols, uqb_array* const* cols, const uint8_t* kinds, uqb_array** rows);
-int uqb_rows_to_columns_ex(uqb_ctx* ctx, const uqb_array* rows, uint32_t ncols, const uint32_t* itemsizes, const uint8_t* kinds,
-                           uqb_array** cols);
+/* QNAME columns <-> rows in sort-key form: columns concatenated at their own widths, which makes memcmp order equal
+ * numpy's field-by-field comparison (uq.py:814-816, 828-830).  kinds: one kind per column (NULL = all 0): 0 little-endian
+ * integer (stored big-endian in the row: unsigned comparison), 1 bytes copied in order ('strings' columns, E1: memcmp of
+ * zero-padded bytes is numpy's order of S values) */
+int uqb_columns_to_rows(uqb_ctx* ctx, uint32_t ncols, uqb_array* const* cols, const uint8_t* kinds, uqb_array** rows);
+int uqb_rows_to_columns(uqb_ctx* ctx, const uqb_array* rows, uint32_t ncols, const uint32_t* itemsizes, const uint8_t* kinds,
+                        uqb_array** cols);
 /* integer columns (itemsize 1/2/4/8) whose value ranges fit 64 bits together -> one packed sort key per row:
  * key = sum over c of (cols[c][i] - bases[c]) << shifts[c], field c `bits[c]` wide (0: a constant column), the first column
  * in the highest bits.  Its numeric order is the memcmp order of the rows of uqb_columns_to_rows.  `table` is a table of

@@ -26,8 +26,10 @@ def _line_offsets_ref(fq):
     return np.concatenate([np.zeros(1, np.uint64), nl])
 
 
-def test_context_and_version(ctx):
-    assert ctx.lib.uqb_version() == 100
+def test_context_and_abi_version(ctx):
+    """ABI 101: uqb_qname_scan, uqb_fastq_load_streamed, uqb_columns_to_rows and uqb_rows_to_columns take their
+    optional arguments (col_mode; ref, ref_len, rbase; kinds) directly"""
+    assert ctx.lib.uqb_version() == 101
     used, free, total = ctx.mem_info()
     assert total > 100 << 30, "expected a B200 with ~180 GB of HBM"
 

@@ -12,6 +12,7 @@ import numpy as np
 import pytest
 
 from conftest import ROOT, assert_config_equal, assert_members_equal, records_multiset
+from test_symbol_paths import assert_kernels
 
 MIXES = [dict(sort=s, raw=r) for s in ("None", "DNA", "QNAME") for r in (None, ["QNAME"])]
 
@@ -298,6 +299,39 @@ def _np_rows(cols, kinds):
     return np.ascontiguousarray(np.concatenate(parts, axis=1))
 
 
+# the kernel pair each direction takes: staged through shared memory for rows of up to 64 bytes (its own pair when a
+# column holds bytes), generic above
+CR_KERNELS = {"staged": ("k_cols_to_rows_staged", "k_rows_to_cols_staged"),
+              "staged_mixed": ("k_cols_to_rows_staged_mixed", "k_rows_to_cols_staged_mixed"),
+              "generic": ("k_cols_to_rows", "k_rows_to_cols")}
+
+
+def _columns_rows_round_trip(ctx, cols, kinds):
+    """columns -> rows against _np_rows, rows -> columns against the columns (kinds None: integer columns); the launch
+    timers must show the kernel pair of CR_KERNELS that the table takes, in both directions, and no other"""
+    n = len(cols[0])
+    widths = [c.dtype.itemsize for c in cols]
+    want = _np_rows(cols, [0] * len(cols) if kinds is None else kinds)
+    dcols = [ctx.upload(c.view(np.uint8).reshape(n, -1)) for c in cols]
+    ctx.timing(True)
+    ctx.timing_reset()
+    try:
+        rows = ctx.columns_to_rows(dcols, kinds)
+        back = ctx.rows_to_columns(rows, widths, kinds)
+        rep = ctx.timing_report()
+    finally:
+        ctx.timing(False)
+    assert rows.width == sum(widths)
+    assert np.array_equal(rows.download().reshape(n, -1), want)
+    for c, b in zip(cols, back):
+        assert np.array_equal(b.download().reshape(-1), c.view(np.uint8).reshape(-1))
+    for a in dcols + back + [rows]:
+        a.free()
+    path = "generic" if sum(widths) > 64 else "staged_mixed" if kinds and any(kinds) else "staged"
+    assert_kernels(rep, ran=CR_KERNELS[path], absent=[k for p, ks in CR_KERNELS.items() if p != path for k in ks],
+                   what="widths %s kinds %s" % (widths, kinds))
+
+
 @pytest.mark.gpu
 @pytest.mark.parametrize("widths", [(4, 3, 1, 2), (1, 8, 5, 2, 8), (2, 60, 4), (8, 100, 1), (4, 255)])
 def test_columns_rows_ex_against_numpy(ctx, widths):
@@ -312,33 +346,18 @@ def test_columns_rows_ex_against_numpy(ctx, widths):
         else:
             cols.append(rng.integers(0, 256, size=(n, w), dtype=np.uint8).reshape(-1).view("S%d" % w))
             kinds.append(1)
-    dcols = [ctx.upload(c.view(np.uint8).reshape(n, -1)) for c in cols]
-    rows = ctx.columns_to_rows(dcols, kinds)
-    want = _np_rows(cols, kinds)
-    assert rows.width == sum(widths)
-    assert np.array_equal(rows.download().reshape(n, -1), want)
-    back = ctx.rows_to_columns(rows, list(widths), kinds)
-    for c, b in zip(cols, back):
-        assert np.array_equal(b.download().reshape(-1), c.view(np.uint8).reshape(-1))
-    for a in dcols + back + [rows]:
-        a.free()
+    _columns_rows_round_trip(ctx, cols, kinds)
 
 
 @pytest.mark.gpu
 @pytest.mark.parametrize("widths", [(1, 2, 4), (8, 8, 8, 8, 8, 8, 8, 8, 8), (2, 2)])
-def test_columns_rows_ex_all_integer_equals_old_entry_points(ctx, widths):
+def test_columns_rows_all_integer_against_numpy(ctx, widths):
+    """integer columns only, with no kinds and with kinds all 0: staged (rows <= 64 B) and generic path (72-byte rows)"""
     rng = np.random.default_rng(3)
     n = 50000
-    cols = [ctx.upload(rng.integers(0, 2 ** (8 * w) - 1, size=n, dtype=np.uint64).astype("u%d" % w)) for w in widths]
-    old = ctx.columns_to_rows(cols)
-    new = ctx.columns_to_rows(cols, [0] * len(cols))
-    assert old.first_difference(new) == -1
-    b_old = ctx.rows_to_columns(old, list(widths))
-    b_new = ctx.rows_to_columns(old, list(widths), [0] * len(cols))
-    for a, b, c in zip(b_old, b_new, cols):
-        assert a.first_difference(b) == -1 and a.first_difference(c) == -1
-    for a in cols + b_old + b_new + [old, new]:
-        a.free()
+    cols = [rng.integers(0, 2 ** (8 * w) - 1, size=n, dtype=np.uint64).astype("u%d" % w) for w in widths]
+    for kinds in (None, [0] * len(cols)):
+        _columns_rows_round_trip(ctx, cols, kinds)
 
 
 @pytest.mark.gpu

@@ -18,7 +18,7 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
 
 # report rows kept: the string-column writer, the integer / rank column writers and tokeniser next to it, and every
-# columns <-> rows kernel (the *_mixed ones run when a string column is present)
+# columns <-> rows kernel (the staged *_mixed pair runs when a string column is present)
 KERNELS = ("k_encode_str", "k_encode_int", "k_encode_rank", "k_qname_tokens", "k_cols_to_rows", "k_rows_to_cols")
 
 

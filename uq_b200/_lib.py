@@ -99,8 +99,7 @@ SIGNATURES = {
     "uqb_index_u32": (C.c_int, [P, P, C.c_uint64, PP, C.POINTER(C.c_int64)]),
     "uqb_fastq_load": (C.c_int, [P, P, C.c_uint64, PP]),
     "uqb_fastq_adopt": (C.c_int, [P, P, C.c_uint64, PP]),
-    "uqb_fastq_load_streamed": (C.c_int, [P, P, C.c_uint64, C.c_uint64, PP]),
-    "uqb_fastq_load_streamed_ref": (C.c_int, [P, P, C.c_uint64, C.c_uint64, P, C.c_uint32, C.c_uint64, PP]),
+    "uqb_fastq_load_streamed": (C.c_int, [P, P, C.c_uint64, C.c_uint64, P, C.c_uint32, C.c_uint64, PP]),
     "uqb_array_download_async": (C.c_int, [P, P, P, C.c_uint64]),
     "uqb_ctx_copy_sync": (C.c_int, [P]),
     "uqb_fastq_free": (C.c_int, [P, P]),
@@ -109,7 +108,6 @@ SIGNATURES = {
     "uqb_fastq_line_offsets": (C.c_int, [P, P, C.c_uint64, C.c_uint64, P]),
     "uqb_analyze": (C.c_int, [P, P, C.POINTER(Stats)]),
     "uqb_fastq_set_reference": (C.c_int, [P, P, P, C.c_uint32, C.c_uint64]),
-    "uqb_qname_scan_ex": (C.c_int, [P, P, C.c_uint32, C.c_uint32, P, C.c_uint32, P, C.POINTER(ColStats), C.POINTER(C.c_int64)]),
     "uqb_qname_dict_first": (C.c_int, [P, P, C.c_uint32, P, C.c_uint64]),
     "uqb_rows_lower_bound": (C.c_int, [P, P, P, C.c_uint32, P]),
     "uqb_add_scalar_u32": (C.c_int, [P, P, C.c_uint32]),
@@ -119,7 +117,7 @@ SIGNATURES = {
     "uqb_partition_positions": (C.c_int, [P, P, P, C.c_uint32, PP, P]),
     "uqb_scatter_rows_segmented": (C.c_int, [P, P, P, C.c_uint32, P, C.c_uint32, PP, P]),
     "uqb_scatter_rows_to": (C.c_int, [P, P, P, C.c_uint32, P, P]),
-    "uqb_qname_scan": (C.c_int, [P, P, C.c_uint32, C.c_uint32, P, C.c_uint32, C.POINTER(ColStats), C.POINTER(C.c_int64)]),
+    "uqb_qname_scan": (C.c_int, [P, P, C.c_uint32, C.c_uint32, P, C.c_uint32, P, C.POINTER(ColStats), C.POINTER(C.c_int64)]),
     "uqb_qname_dict_info": (C.c_int, [P, P, C.c_uint32, C.POINTER(C.c_uint64), C.POINTER(C.c_uint32)]),
     "uqb_qname_dict": (C.c_int, [P, P, C.c_uint32, P, C.c_uint64]),
     "uqb_qname_encode": (C.c_int, [P, P, C.c_uint32, C.POINTER(ColSpec), PP]),
@@ -127,10 +125,8 @@ SIGNATURES = {
     "uqb_sort_rows": (C.c_int, [P, P, PP, PP, PP, PP, C.POINTER(C.c_uint64)]),
     "uqb_gather_rows": (C.c_int, [P, P, P, PP]),
     "uqb_narrow_u32": (C.c_int, [P, P, C.c_uint32, PP]),
-    "uqb_columns_to_rows": (C.c_int, [P, C.c_uint32, PP, PP]),
-    "uqb_rows_to_columns": (C.c_int, [P, P, C.c_uint32, C.POINTER(C.c_uint32), PP]),
-    "uqb_columns_to_rows_ex": (C.c_int, [P, C.c_uint32, PP, P, PP]),
-    "uqb_rows_to_columns_ex": (C.c_int, [P, P, C.c_uint32, C.POINTER(C.c_uint32), P, PP]),
+    "uqb_columns_to_rows": (C.c_int, [P, C.c_uint32, PP, P, PP]),
+    "uqb_rows_to_columns": (C.c_int, [P, P, C.c_uint32, C.POINTER(C.c_uint32), P, PP]),
     "uqb_columns_to_key": (C.c_int, [P, C.c_uint32, PP, C.POINTER(C.c_uint32), C.POINTER(C.c_uint32), C.POINTER(C.c_uint64), PP]),
     "uqb_key_to_columns": (C.c_int, [P, P, C.c_uint32, C.POINTER(C.c_uint32), C.POINTER(C.c_uint32), C.POINTER(C.c_uint32),
                                      C.POINTER(C.c_uint64), PP]),
@@ -156,7 +152,7 @@ def load():
         fn = getattr(lib, name)          # AttributeError if the export is missing
         fn.restype = res
         fn.argtypes = args
-    if lib.uqb_version() != 100:
+    if lib.uqb_version() != 101:
         raise RuntimeError("uq_b200: libuqb200.so version %d does not match the binding" % lib.uqb_version())
     _lib = lib
     return lib

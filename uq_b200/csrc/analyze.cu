@@ -860,14 +860,11 @@ extern "C" int uqb_analyze(uqb_ctx* ctx, uqb_fastq* fq, uqb_stats* out) {
 // records completed so far).  When the last chunk arrives the split and the Pass-1 statistics are
 // done; uqb_split / uqb_analyze on the returned handle return them without touching the data again.
 // ================================================================================================
-extern "C" int uqb_fastq_load_streamed(uqb_ctx* ctx, const uint8_t* host, uint64_t nbytes, uint64_t chunk_bytes, uqb_fastq** out_fq) {
-    return uqb_fastq_load_streamed_ref(ctx, host, nbytes, chunk_bytes, nullptr, 0, 0, out_fq);
-}
-
-// as above for a multi-GPU shard: statistics are measured against the global first QNAME line `ref`; rbase > 0
-// says that this shard does not start the file (its first record takes part in the prefix/suffix statistics)
-extern "C" int uqb_fastq_load_streamed_ref(uqb_ctx* ctx, const uint8_t* host, uint64_t nbytes, uint64_t chunk_bytes,
-                                           const uint8_t* ref, uint32_t ref_len, uint64_t rbase, uqb_fastq** out_fq) {
+// `ref`: the global first QNAME line that a multi-GPU shard's statistics are measured against (NULL: the handle is the
+// whole file); rbase > 0 says that the shard does not start the file (its first record takes part in the prefix/suffix
+// statistics).
+extern "C" int uqb_fastq_load_streamed(uqb_ctx* ctx, const uint8_t* host, uint64_t nbytes, uint64_t chunk_bytes,
+                                       const uint8_t* ref, uint32_t ref_len, uint64_t rbase, uqb_fastq** out_fq) {
     if (chunk_bytes == 0) chunk_bytes = 256ull << 20;
     chunk_bytes = (chunk_bytes + UQB_SPLIT_TILE - 1) / UQB_SPLIT_TILE * UQB_SPLIT_TILE;
     cudaStream_t cs;

@@ -212,13 +212,8 @@ static int distinct_of_prefix(uqb_ctx* ctx, uqb_fastq* fq, const uqb_qcol& qc, u
 }
 
 extern "C" int uqb_qname_scan(uqb_ctx* ctx, uqb_fastq* fq, uint32_t prefix_len, uint32_t suffix_len,
-                              const uint8_t* seps, uint32_t nseps, uqb_colstats* cols, int64_t* bad_record) {
-    return uqb_qname_scan_ex(ctx, fq, prefix_len, suffix_len, seps, nseps, nullptr, cols, bad_record);
-}
-
-extern "C" int uqb_qname_scan_ex(uqb_ctx* ctx, uqb_fastq* fq, uint32_t prefix_len, uint32_t suffix_len,
-                                 const uint8_t* seps, uint32_t nseps, const uint8_t* col_mode,
-                                 uqb_colstats* cols, int64_t* bad_record) {
+                              const uint8_t* seps, uint32_t nseps, const uint8_t* col_mode,
+                              uqb_colstats* cols, int64_t* bad_record) {
     if (!fq->line_off) return uqb_fail(ctx, "uqb_qname_scan: call uqb_split first");
     if (nseps + 1 > UQB_MAX_COLS) return uqb_fail(ctx, "uqb_qname_scan: more than %d QNAME columns", UQB_MAX_COLS);
     const uint64_t N = fq->n_reads;

@@ -211,12 +211,9 @@ class Context:
         ref / rbase: multi-GPU shard measured against the global first QNAME line (rbase > 0: not the first shard)."""
         arr = data.array if isinstance(data, PinnedBuffer) else np.ascontiguousarray(data, dtype=np.uint8)
         h = C.c_void_p()
-        if ref is None:
-            rc = self.lib.uqb_fastq_load_streamed(self.h, _ptr(arr) if arr.size else None, int(arr.size), int(chunk_bytes), C.byref(h))
-        else:
-            rb = np.frombuffer(ref, dtype=np.uint8)
-            rc = self.lib.uqb_fastq_load_streamed_ref(self.h, _ptr(arr) if arr.size else None, int(arr.size), int(chunk_bytes),
-                                                      _ptr(rb) if rb.size else None, int(rb.size), int(rbase), C.byref(h))
+        rb = np.frombuffer(b"" if ref is None else ref, dtype=np.uint8)
+        rc = self.lib.uqb_fastq_load_streamed(self.h, _ptr(arr) if arr.size else None, int(arr.size), int(chunk_bytes),
+                                              _ptr(rb) if rb.size else None, int(rb.size), int(rbase), C.byref(h))
         if rc:
             msg = self.lib.uqb_last_error(self.h).decode()
             if h:
@@ -282,22 +279,16 @@ class Context:
         """columns -> sort rows; kinds[c]: 0 little-endian integer (big-endian in the row), 1 bytes as they are"""
         arr = (C.c_void_p * len(cols))(*[c.h for c in cols])
         h = C.c_void_p()
-        if kinds is None:
-            self.check(self.lib.uqb_columns_to_rows(self.h, len(cols), arr, C.byref(h)))
-        else:
-            k = np.ascontiguousarray(kinds, dtype=np.uint8)
-            self.check(self.lib.uqb_columns_to_rows_ex(self.h, len(cols), arr, _ptr(k), C.byref(h)))
+        k = None if kinds is None else np.ascontiguousarray(kinds, dtype=np.uint8)
+        self.check(self.lib.uqb_columns_to_rows(self.h, len(cols), arr, _ptr(k) if k is not None else None, C.byref(h)))
         return DeviceArray(self, h)
 
     def rows_to_columns(self, rows, itemsizes, kinds=None):
         n = len(itemsizes)
         sizes = (C.c_uint32 * n)(*[int(s) for s in itemsizes])
         outs = (C.c_void_p * n)()
-        if kinds is None:
-            self.check(self.lib.uqb_rows_to_columns(self.h, rows.h, n, sizes, outs))
-        else:
-            k = np.ascontiguousarray(kinds, dtype=np.uint8)
-            self.check(self.lib.uqb_rows_to_columns_ex(self.h, rows.h, n, sizes, _ptr(k), outs))
+        k = None if kinds is None else np.ascontiguousarray(kinds, dtype=np.uint8)
+        self.check(self.lib.uqb_rows_to_columns(self.h, rows.h, n, sizes, _ptr(k) if k is not None else None, outs))
         return [DeviceArray(self, C.c_void_p(outs[i])) for i in range(n)]
 
     def columns_to_key(self, cols, plan):
@@ -472,9 +463,9 @@ class Fastq:
         cols = (L.ColStats * ncols)()
         bad = C.c_int64()
         mode = None if col_mode is None else np.ascontiguousarray(col_mode, dtype=np.uint8)
-        self.ctx.check(self.ctx.lib.uqb_qname_scan_ex(self.ctx.h, self.h, int(prefix_len), int(suffix_len),
-                                                      _ptr(seps) if len(seps) else None, len(seps),
-                                                      _ptr(mode) if mode is not None else None, cols, C.byref(bad)))
+        self.ctx.check(self.ctx.lib.uqb_qname_scan(self.ctx.h, self.h, int(prefix_len), int(suffix_len),
+                                                   _ptr(seps) if len(seps) else None, len(seps),
+                                                   _ptr(mode) if mode is not None else None, cols, C.byref(bad)))
         return cols, int(bad.value)
 
     def qname_dict_first(self, col):
