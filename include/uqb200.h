@@ -278,6 +278,23 @@ typedef struct {
 int uqb_decode(uqb_ctx* ctx, const uqb_array* dna, const uqb_array* qual, uqb_array* const* cols,
                const uqb_decode_params* p, uqb_array** fastq);
 
+/* ---- verification of an encode (no reference counterpart: uq.py never reads back what it wrote) ----------- */
+typedef struct {
+    uint64_t records;        /* container rows compared */
+    uint64_t differ[4];      /* rows whose line k differs: 0 name, 1 sequence, 2 '+' line, 3 quality */
+    int64_t  first_row[4];   /* smallest such container row, -1 none */
+    int64_t  first_src[4];   /* its input record number */
+} uqb_verify_report;
+/* src: the encoded FASTQ; text: decoded rows [first_row, first_row + k) as a uqb_fastq (adopted + split, k = its records);
+ * order: uint32[n] container row -> input record, NULL = identity.  Compares the four lines of decoded record i - first_row
+ * with those of input record order[i], lengths first, then bytes; an order value >= the input's record count is a
+ * difference in all four fields and is not dereferenced.  Accumulates into *report, whose first_row entries the caller
+ * starts at -1. */
+int uqb_verify_records(uqb_ctx* ctx, const uqb_fastq* src, const uqb_fastq* text, uint64_t first_row,
+                       const uqb_array* order, uqb_verify_report* report);
+/* missing = smallest value in [0, n) that order does not hold, -1 if order (of length n) is a permutation of [0, n) */
+int uqb_check_permutation(uqb_ctx* ctx, const uqb_array* order, uint64_t n, int64_t* missing);
+
 /* ---- synthetic inputs for bench/tests (same generator as oracle/synth.py, oracle/synth_umi.py) - */
 typedef struct {
     uint32_t kind;        /* 0 illumina, 1 genome, 2 casava, 3 ont, 4 umi (illumina header + '_' + 6-12 of ACGTN),

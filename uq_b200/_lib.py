@@ -64,6 +64,10 @@ class DecodeParams(C.Structure):
                 ("cols", C.POINTER(DecodeCol))]
 
 
+class VerifyReport(C.Structure):
+    _fields_ = [("records", C.c_uint64), ("differ", C.c_uint64 * 4), ("first_row", C.c_int64 * 4), ("first_src", C.c_int64 * 4)]
+
+
 class SynthParams(C.Structure):
     _fields_ = [("kind", C.c_uint32), ("length", C.c_uint32), ("len_lo", C.c_uint32), ("len_hi", C.c_uint32),
                 ("seed", C.c_uint64), ("first", C.c_uint64), ("n", C.c_uint64), ("genome", C.c_uint64), ("pool", C.c_uint64)]
@@ -133,6 +137,8 @@ SIGNATURES = {
     "uqb_layout": (C.c_int, [P, P, C.c_int, PP]),
     "uqb_unlayout": (C.c_int, [P, P, C.c_uint64, C.c_uint32, C.c_int, PP]),
     "uqb_decode": (C.c_int, [P, P, P, PP, C.POINTER(DecodeParams), PP]),
+    "uqb_verify_records": (C.c_int, [P, P, P, C.c_uint64, P, C.POINTER(VerifyReport)]),
+    "uqb_check_permutation": (C.c_int, [P, P, C.c_uint64, C.POINTER(C.c_int64)]),
     "uqb_synth": (C.c_int, [P, C.POINTER(SynthParams), P, PP]),
 }
 

@@ -308,6 +308,18 @@ class Context:
         self.check(self.lib.uqb_key_to_columns(self.h, keys.h, n, sizes, shifts, bits, bases, outs))
         return [DeviceArray(self, C.c_void_p(outs[i])) for i in range(n)]
 
+    def verify_records(self, src, text, first_row, order, report):
+        """decoded records (text: split Fastq of container rows first_row..) against the encoded FASTQ src, under order
+        (uint32 DeviceArray, container row -> input record; None = identity); accumulates into report (L.VerifyReport)"""
+        self.check(self.lib.uqb_verify_records(self.h, src.h, text.h, int(first_row), order.h if order is not None else None,
+                                               C.byref(report)))
+
+    def check_permutation(self, order, n):
+        """-> smallest value in [0, n) that order does not hold, -1 if it is a permutation of [0, n)"""
+        m = C.c_int64()
+        self.check(self.lib.uqb_check_permutation(self.h, order.h, int(n), C.byref(m)))
+        return int(m.value)
+
     def layout(self, table, pattern):
         h = C.c_void_p()
         self.check(self.lib.uqb_layout(self.h, table.h, PATTERN_ID[pattern], C.byref(h)))

@@ -354,6 +354,7 @@ class DeviceMembers:
     def __init__(self, ctx=None, sink=None):
         self.items = {}
         self.ctx, self.sink, self.host = ctx, sink, {}
+        self.order = None       # run_mix: uint32 DeviceArray, container row -> input record (None: rows in input order)
 
     def _queue(self, name, arr):
         if self.sink is not None:
@@ -395,6 +396,9 @@ class DeviceMembers:
         for a, _, _ in self.items.values():
             a.free()
         self.items = {}
+        if self.order is not None:
+            self.order.free()
+            self.order = None
 
     def __del__(self):
         # members dropped without free() (an exception in the middle of run_mix): the queued device->host copies must
@@ -588,7 +592,8 @@ def _mix_qname(ctx, out, cols, columns, order, raw):
 def run_mix(ctx, dna, qual, cols, columns, sorted_on, raw_tables, pattern, sink=None):
     """uq.py:739-753.  The reference runs the sorted-on table first; here the order-independent half of the
     other keyed table (its unique table - the largest output) is produced before that, so that its
-    device->host copy overlaps the remaining sorts.  The results are identical."""
+    device->host copy overlaps the remaining sorts.  The results are identical.  The sort order (the stable argsort that
+    links container row i to input record order[i]) stays on the members as `order` for verify_device."""
     out = DeviceMembers(ctx, sink)
     pd, pq = pattern
     if sorted_on in ('DNA', 'QUAL'):
@@ -597,13 +602,13 @@ def run_mix(ctx, dna, qual, cols, columns, sorted_on, raw_tables, pattern, sink=
         prepared = None
         if second[1] not in raw_tables:
             prepared = _timed(ctx, 'mix_' + second[1], _prepare_keyed, ctx, out, second[0], second[1], second[2])
-        order = _timed(ctx, 'mix_' + first[1], _mix_dna_qual, ctx, out, first[0], first[1], False, first[1] in raw_tables, first[2])
-        _timed(ctx, 'mix_' + second[1], _mix_dna_qual, ctx, out, second[0], second[1], order, second[1] in raw_tables, second[2], prepared)
-        _timed(ctx, 'mix_QNAME', _mix_qname, ctx, out, cols, columns, order, 'QNAME' in raw_tables)
+        out.order = _timed(ctx, 'mix_' + first[1], _mix_dna_qual, ctx, out, first[0], first[1], False, first[1] in raw_tables, first[2])
+        _timed(ctx, 'mix_' + second[1], _mix_dna_qual, ctx, out, second[0], second[1], out.order, second[1] in raw_tables, second[2], prepared)
+        _timed(ctx, 'mix_QNAME', _mix_qname, ctx, out, cols, columns, out.order, 'QNAME' in raw_tables)
     elif sorted_on == 'QNAME':
-        order = _timed(ctx, 'mix_QNAME', _mix_qname, ctx, out, cols, columns, False, 'QNAME' in raw_tables)
-        _timed(ctx, 'mix_QUAL', _mix_dna_qual, ctx, out, qual, 'QUAL', order, 'QUAL' in raw_tables, pq)
-        _timed(ctx, 'mix_DNA', _mix_dna_qual, ctx, out, dna, 'DNA', order, 'DNA' in raw_tables, pd)
+        out.order = _timed(ctx, 'mix_QNAME', _mix_qname, ctx, out, cols, columns, False, 'QNAME' in raw_tables)
+        _timed(ctx, 'mix_QUAL', _mix_dna_qual, ctx, out, qual, 'QUAL', out.order, 'QUAL' in raw_tables, pq)
+        _timed(ctx, 'mix_DNA', _mix_dna_qual, ctx, out, dna, 'DNA', out.order, 'DNA' in raw_tables, pd)
     else:
         _timed(ctx, 'mix_QUAL', _mix_dna_qual, ctx, out, qual, 'QUAL', None, 'QUAL' in raw_tables, pq)
         _timed(ctx, 'mix_DNA', _mix_dna_qual, ctx, out, dna, 'DNA', None, 'DNA' in raw_tables, pd)
@@ -933,57 +938,184 @@ def decode_device(ctx, dna, qual, dcols, config):
     return DeviceArray(ctx, h)
 
 
-def decode_members_device(ctx, dm, config):
-    """The decoder's front (load_from_tar + key expansion, uq.py:943-973) and decode_device on members that are already
-    in HBM (a DeviceMembers as encode_device returns it): streams are un-laid-out, keys widened and bound-checked, rows
-    gathered, text produced - all on the device.  -> DeviceArray with the FASTQ text."""
-    it = dm.items
-    pat = config['pattern']
-    tmp = []
+class MemberRows:
+    """The decoder's front (load_from_tar + key expansion, uq.py:943-973) on members that are already in HBM (a
+    DeviceMembers as encode_device returns it), for any range of container rows [a, b): rows(a, b) -> (dna, qual, dcols),
+    the logical tables and the QNAME columns of those rows, ready for decode_device.  Streams are un-laid-out, keys widened
+    and bound-checked, rows gathered - all on the device.
 
-    def key_of(name, n_rows):
-        arr = it[name][0]
-        k32, bad = ctx.index_u32(arr, n_rows)
-        tmp.append(k32)
-        if bad >= 0:
-            raise UQError('ERROR: %s[%d] points outside its table of %d rows (malformed uQ file)' % (name, bad, n_rows))
-        return k32
+    A raw pattern-0.1 stream and a raw QNAME column are views of their rows.  A keyed table or QNAME column is gathered
+    through a view of its key's rows, so a batch needs memory for its own rows only.  A unique table, and a raw table in
+    another pattern, are un-laid-out once for the whole file (here, in the constructor).  The arrays of one rows() call
+    are released by release() (or close())."""
 
-    def table(name, pattern):
-        def logical(entry):
+    def __init__(self, ctx, dm, config):
+        self.ctx, self.it, self.config = ctx, dm.items, config
+        self.n = int(config['reads'])
+        self.whole, self.batch = [], []
+        try:
+            self.src = {name: self._logical(name) for name in ('DNA', 'QUAL')}
+        except Exception:
+            self.close()
+            raise
+
+    def _logical(self, name):
+        """DNA / QUAL -> (logical table of the raw rows or of the unique rows, key member name or None)"""
+        def unlaid(entry):
             stream, _, (n, width, p) = entry
             if p == '0.1':
-                return ctx.wrap(stream.device_ptr.value, n, width), True
-            t = ctx.unlayout(stream, n, width, p)
-            return t, True
-        if name + '.raw' in it:
-            t, own = logical(it[name + '.raw'])
-            tmp.append(t)
-            return t
-        uniq, _ = logical(it[name])
-        tmp.append(uniq)
-        t = ctx.gather_rows(uniq, key_of(name + '.key', uniq.n))                   # uq.py:953, 957
-        tmp.append(t)
-        return t
+                return self._hold(self.ctx.wrap(stream.device_ptr.value, n, width), self.whole)
+            return self._hold(self.ctx.unlayout(stream, n, width, p), self.whole)
+        if name + '.raw' in self.it:
+            return unlaid(self.it[name + '.raw']), None
+        return unlaid(self.it[name]), name + '.key'
 
-    try:
-        dna, qual = table('DNA', pat[0]), table('QUAL', pat[1])
-        dcols = []
-        keyed = 'QNAME.key' in it
-        key = None
-        for meta in config['QNAME_columns']:
-            nm = meta['name'] + ('' if keyed else '.raw')
-            c = it[nm][0]
+    @staticmethod
+    def _hold(a, into):
+        into.append(a)
+        return a
+
+    def _view(self, arr, a, b):
+        """rows [a, b) of a device array: a view when it starts 16-byte aligned (the decode kernels load packed rows as
+        aligned 16-byte words), else a copy of the rows"""
+        w = arr.width
+        ptr = arr.device_ptr.value + a * w
+        if a == 0 or ptr % 16 == 0:
+            return self._hold(self.ctx.wrap(ptr, b - a, w), self.batch)
+        out = self._hold(self.ctx.alloc(b - a, w), self.batch)
+        self.ctx.copy_in(out, 0, ptr, (b - a) * w)
+        return out
+
+    def _key(self, name, n_rows, a, b):
+        k32, bad = self.ctx.index_u32(self._view(self.it[name][0], a, b), n_rows)
+        self._hold(k32, self.batch)
+        if bad >= 0:
+            raise UQError('ERROR: %s[%d] points outside its table of %d rows (malformed uQ file)' % (name, a + bad, n_rows))
+        return k32
+
+    def _rows(self, table, key, a, b):
+        if key is None:
+            return self._view(table, a, b)
+        return self._hold(self.ctx.gather_rows(table, self._key(key, table.n, a, b)), self.batch)      # uq.py:953, 957
+
+    def rows(self, a, b):
+        self.release()
+        dna, qual = (self._rows(t, k, a, b) for t, k in (self.src['DNA'], self.src['QUAL']))
+        keyed = 'QNAME.key' in self.it
+        dcols, key = [], None
+        for meta in self.config['QNAME_columns']:
+            c = self.it[meta['name'] + ('' if keyed else '.raw')][0]
             if keyed:
                 if key is None:
-                    key = key_of('QNAME.key', c.n)
-                c = ctx.gather_rows(c, key)                                        # uq.py:973
-                tmp.append(c)
-            dcols.append(c)
-        return decode_device(ctx, dna, qual, dcols, config)
+                    key = self._key('QNAME.key', c.n, a, b)
+                dcols.append(self._hold(self.ctx.gather_rows(c, key), self.batch))                     # uq.py:973
+            else:
+                dcols.append(self._view(c, a, b))
+        return dna, qual, dcols
+
+    def release(self):
+        for x in self.batch:
+            x.free()
+        self.batch = []
+
+    def close(self):
+        self.release()
+        for x in self.whole:
+            x.free()
+        self.whole = []
+
+
+def decode_members_device(ctx, dm, config):
+    """decode_device on members that are already in HBM (a DeviceMembers as encode_device returns it), all rows at once.
+    -> DeviceArray with the FASTQ text."""
+    rows = MemberRows(ctx, dm, config)
+    try:
+        return decode_device(ctx, *rows.rows(0, rows.n), config)
     finally:
-        for a in tmp:
-            a.free()
+        rows.close()
+
+
+# ------------------------------------------------------------------------------------------------
+# verify: the encode decoded on the device and compared with its input, record by record
+# ------------------------------------------------------------------------------------------------
+FIELDS = ('name', 'sequence', '+ line', 'quality')
+
+
+def verify_batch_rows(ctx, fq, members, config, want=1 << 24):
+    """Rows per verify batch that fit next to what is already allocated: the largest multiple of 2^20 up to `want` whose
+    decoded text, line offsets and gathered rows take at most 3/4 of the device memory the context does not hold;
+    0 when not even 2^20 rows fit.  (Device memory is counted as total - held: the context's arena keeps what it has
+    mapped, so that is the room it can grow into.)"""
+    n = int(config['reads'])
+    in_use, _, total = ctx.mem_info()
+    widths = 0
+    once = (n + 31) // 32 * 4                                         # permutation bits
+    for name, (arr, kind, meta) in members.items.items():
+        if kind == 'table':
+            m, width, pattern = meta
+            widths += width
+            if pattern != '0.1':
+                once += m * width                                     # un-laid-out once for the whole file
+        else:
+            widths += arr.width + (4 if name.endswith('.key') else 0)
+    per_row = 2 * (fq.nbytes // max(n, 1) + 1) + 4 * 8 + 12 + 2 * widths     # text (+ its copy in flight), line offsets, decode scratch
+    room = (total - in_use - once) * 3 // 4
+    if n <= (1 << 20):
+        return n if room >= n * per_row else 0
+    fit = room // per_row // (1 << 20) * (1 << 20)
+    return int(min(want, fit, n)) if fit >= (1 << 20) else 0
+
+
+def verify_device(ctx, fq, members, config, batch_rows=1 << 24):
+    """Decode the members of an encode (a DeviceMembers from encode_device, still in HBM) batch by batch and compare
+    every record with its input record in fq (the split FASTQ they were encoded from), under members.order.  Nothing is
+    copied to the host but the report.
+    -> dict(records, differ[4], first_row[4], first_src[4], missing, lines): per field (0 name, 1 sequence, 2 '+' line,
+    3 quality) the rows whose line differs and the first such container row with its input record; `missing` the
+    smallest input record that members.order does not hold (-1: a permutation, or no order); `lines[f]` = (input line,
+    decoded line) of the first difference of field f, as bytes without the newline."""
+    n = int(config['reads'])
+    if fq.n_reads is None:
+        fq.split()
+    rep = L.VerifyReport()
+    for f in range(4):
+        rep.first_row[f] = rep.first_src[f] = -1
+    order = members.order
+    missing = _timed(ctx, 'verify_perm', ctx.check_permutation, order, n) if order is not None else -1
+    batch_rows = max(1, int(batch_rows))
+    lines = {}
+
+    def line(h, k):
+        o = h.line_offsets(k, 2)
+        return h.download(int(o[0]), int(o[1] - o[0]) - 1).tobytes()
+
+    rows = MemberRows(ctx, members, config)
+    try:
+        for a in range(0, n, batch_rows):
+            b = min(n, a + batch_rows)
+            tables = _timed(ctx, 'verify_rows', rows.rows, a, b)
+            text = _timed(ctx, 'verify_decode', decode_device, ctx, *tables, config)
+            rows.release()
+            tfq = ctx.adopt_fastq(text)
+            try:
+                _timed(ctx, 'verify_split', tfq.split)
+                before = list(rep.first_row)
+                _timed(ctx, 'verify_compare', ctx.verify_records, fq, tfq, a, order, rep)
+                for f in range(4):
+                    if rep.first_row[f] >= 0 and before[f] < 0:     # the first difference of field f is in this batch
+                        r, s = int(rep.first_row[f]), int(rep.first_src[f])
+                        lines[f] = (line(fq, 4 * s + f) if s < fq.n_reads else None, line(tfq, 4 * (r - a) + f))
+            finally:
+                tfq.free()
+                text.free()
+    finally:
+        rows.close()
+    return dict(records=int(rep.records), differ=[int(x) for x in rep.differ], first_row=[int(x) for x in rep.first_row],
+                first_src=[int(x) for x in rep.first_src], missing=missing, lines=lines)
+
+
+def verify_clean(report):
+    return not any(report['differ']) and report['missing'] < 0
 
 
 def decode(members, config, ctx=None, out=None):

@@ -4,7 +4,7 @@ format, with the FASTQ -> uQ encode and uQ -> FASTQ decode hot path running on t
 libuqb200.so.  Host logic only; there is no CPU implementation of the path in this package.
 
     python -m uq_b200.uq -i reads.fastq [--sort DNA|QUAL|QNAME|None] [--raw DNA QUAL QNAME] \\
-                         [--pattern 0.1 0.1] [--pad] [--notricks] [--peek] [--test] [--compressor CMD]
+                         [--pattern 0.1 0.1] [--pad] [--notricks] [--peek] [--test] [--compressor CMD] [--verify]
     python -m uq_b200.uq -i reads.fastq.uQ --decode > reads.fastq
 """
 import argparse
@@ -38,7 +38,40 @@ def build_parser():
     p.add_argument("--peek", action='store_true', default=False, help='Optional. No output files are created, the input is just scanned and report printed to terminal.')
     p.add_argument("--decode", action='store_true', default=False, help='Requred if you want to convert a .uQ back to .fastq')
     p.add_argument("--device", type=int, default=0, help='CUDA device ordinal (this implementation only).')
+    p.add_argument("--verify", action='store_true', default=False,
+                   help='Optional. FASTQ->uQ only. Decode the container on the GPU and compare every record with its input '
+                        'record before writing it; on any difference nothing is written and the exit status is 1.')
     return p
+
+
+def check_options(args):
+    if args.verify and (args.decode or args.peek):
+        raise host.UQError('ERROR: --verify checks a FASTQ -> uQ encode; it cannot be combined with --%s'
+                           % ('decode' if args.decode else 'peek'))
+
+
+HINTS = {0: 'integer QNAME columns lose leading zeros and "+" signs in the reference format (Q9)',
+         2: 'the reference format keeps no text after the "+" of the third line (Q13)'}
+
+
+def verify_failure(report):
+    """the report of a verify that found differences -> the lines to print"""
+    out = ['ERROR: --verify: the container does not reproduce the input; nothing was written.']
+    for f, field in enumerate(host.FIELDS):
+        if not report['differ'][f]:
+            continue
+        out.append('  %s: %d records differ; first at container row %d, input record %d' % (
+            field, report['differ'][f], report['first_row'][f], report['first_src'][f]))
+        want, got = report['lines'].get(f, (None, None))
+        if want is not None:
+            out.append('    input:   %r' % want)
+        if got is not None:
+            out.append('    decoded: %r' % got)
+        if f in HINTS:
+            out.append('    hint: ' + HINTS[f])
+    if report['missing'] >= 0:
+        out.append('  order: input record %d is missing from the container' % report['missing'])
+    return out
 
 
 def compressed_size(arr, compressor):
@@ -94,6 +127,7 @@ def main(argv=None):
         print('ERROR: Sorry, the input path you have specified is not a file!')
         return 0
     try:
+        check_options(args)
         ctx = Context(args.device)
         if args.decode:
             members, config = container.read_container(args.input)
@@ -139,6 +173,19 @@ def main(argv=None):
 
         fq = ctx.load_fastq_streamed(data) if got >= (1 << 20) else ctx.load_fastq(data)
         dmembers, config = host.encode_device(ctx, fq, sort=sort, raw=raw, pattern=pattern, pad=args.pad, notricks=args.notricks, sink=sink)
+        if args.verify:                                                                 # while the members' D2H copies run
+            tv = time.time()
+            batch = host.verify_batch_rows(ctx, fq, dmembers, config)
+            if batch == 0:
+                raise host.UQError('ERROR: --verify: not enough free device memory to decode even 2^20 records next to the encoded members')
+            report = host.verify_device(ctx, fq, dmembers, config, batch_rows=batch)
+            if not host.verify_clean(report):
+                dmembers.free(); fq.free()
+                for p in pins:
+                    p.free()
+                print('\n'.join(verify_failure(report)))
+                return 1
+            print('Verified: all %d records decode to their input records (%.3f s)' % (report['records'], time.time() - tv))
         members = dmembers.download()
         print('\nWriting final config...')
         print('Archiving results...')
@@ -147,7 +194,7 @@ def main(argv=None):
         for p in pins:
             p.free()
         print('All Done! :)  (%d reads, %.2f s, %d kernel launches on cuda:%d)' % (config['reads'], time.time() - t0, ctx.launches, args.device))
-    except host.UQError as e:                                                           # uq.py:48-50: print, exit status 0
+    except host.UQError as e:                                                           # uq.py:48-50: print, exit status 0 (a failed --verify: 1)
         print(e)
     return 0
 
